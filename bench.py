@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- vertex-moves/sec of the Metropolis-Hastings sweep on synthetic planted bipartite SBMs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[2], SURVEY.md 8(d) row C3): 1M nodes (5e5+5e5) / 10M edges,
@@ -15,8 +15,13 @@ e2e     = the same through the C ABI with HOST buffers: every step uploads the c
 roofline= algorithmic HBM bytes per move (16 + 8*(2E/N) + 4*acceptance, SURVEY.md 8(d)) x moves
           / CUDA-event time of the sweep launches, against MEASURED_PEAKS.json hbm_gbs.
 cpu_baseline / --impl reference = the UNMODIFIED reference (oracle/_ref/libref.so, built from
-          /root/reference/src) or, if that build is absent, the oracle port, one chain per host
-          core, anneal() only, on a bounded sample of the same workload.
+          the reference's sources by `make -C oracle ref`) or, if that build is absent, the oracle port,
+          one chain per host core, anneal() only, on a bounded sample of the same workload.
+--dump-outputs DIR (C3 workload, one process) = after the timed steps, what the last one computed, as DIR/<name>.npy
+          (see dump_outputs); the inputs depend only on the arguments, so two builds can be compared output for output.
+          The staged parallel sweep evaluates and commits in fixed rounds, so two runs of one build write identical
+          files -- unless a block of some chain gets small enough to empty within one launch, where the order of the
+          "would empty the block" veto's atomics decides (no block of the C3 workload comes near that).
 """
 import argparse
 import ctypes
@@ -72,6 +77,27 @@ def planted_chunked(na, nb, ka, kb, n_edges, seed, chunk=50_000_000):
 
 def planted_labels(na, nb, ka, kb):
     return np.concatenate([np.arange(na) * ka // na, ka + np.arange(nb) * kb // nb]).astype(np.uint32)
+
+
+DUMP_CHAINS = 256       # --dump-outputs keeps every chain up to this many, else a seeded sample of this many
+DUMP_NODES = 16384      # ... and the labels of a seeded sample of this many nodes: at most 16 MB of labels
+
+
+def dump_outputs(out_dir, pool, acc, sweeps):
+    """Write what one anneal() call handed back (per-chain acceptance ratio and sweeps done) and the state it left behind
+    (per-chain description length, labels) as float64 / float32 .npy files.  The chains and nodes kept are a fixed sample
+    (the same for every run with the same arguments), whose indices are written beside the labels."""
+    rng = np.random.default_rng(0)
+    C, n = pool.n_chains, pool.g.n
+    chains = np.arange(C) if C <= DUMP_CHAINS else np.sort(rng.choice(C, DUMP_CHAINS, replace=False))
+    nodes = np.arange(n) if n <= DUMP_NODES else np.sort(rng.choice(n, DUMP_NODES, replace=False))
+    labels = pool.labels(out=np.empty((C, n), dtype=np.uint8 if pool.K(0) <= 256 else np.uint32))
+    out = {"acceptance": acc[chains], "sweeps": sweeps[chains].astype(np.float64), "entropy": pool.entropy()[chains],
+           "labels": labels[np.ix_(chains, nodes)].astype(np.float32), "labels_chains": chains.astype(np.float64),
+           "labels_nodes": nodes.astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class stdout_to_stderr:
@@ -533,11 +559,19 @@ def main():
     ap.add_argument("--warps", type=int, default=0, help="experiment builds only: warps per CTA (20, 24)")
     ap.add_argument("--no-spare-sms", action="store_true", help="A/B: leave the SMs that groups x CTAs do not fill idle")
     ap.add_argument("--no-fp32-extra", action="store_true", help="skip the short fp32 run reported under 'extra'")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="C3 workload: write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, < 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "c3"):
+        ap.error("--dump-outputs is implemented for the C3 workload of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:     # several ranks time one more sweep after the steps (the marginal all-reduce)
+        ap.error("--dump-outputs is implemented for one process")
     na = nb = args.nodes // 2
     n = na + nb
     ka = kb = args.k
@@ -644,7 +678,7 @@ def main():
     t0 = time.perf_counter()
     ev_ms, launches, moves, accs, sweep_launches = 0.0, 0, 0, [], 0
     for _ in range(args.steps):
-        acc, _sw = pool.anneal("constant", 1.0, 0.0, duration, 10 ** 18, seeds)
+        acc, sw = pool.anneal("constant", 1.0, 0.0, duration, 10 ** 18, seeds)
         ms_, la_, mv_ = pool.last_timing()
         ev_ms += ms_; launches += la_; moves += mv_; accs.append(float(acc.mean()))
         sweep_launches += pool.sweep_launches()
@@ -659,6 +693,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs:       # before the e2e arm below restarts the chains from snap_host
+        dump_outputs(args.dump_outputs, pool, acc, sw)
     t = torch.tensor([wall, ev_ms], dtype=torch.float64, device="cuda")
     tot = torch.tensor([float(moves)], dtype=torch.float64, device="cuda")
     if world > 1:

@@ -105,6 +105,7 @@ struct bisbm_handle {
             *d_eta = nullptr;
     int32_t *d_m2 = nullptr, *d_e2 = nullptr, *d_nr2 = nullptr;  // "next" count buffers of the sliced shared-memory sweep
     int32_t* d_nr_live = nullptr;              // exact n_r counters of the blocks that could empty within one sliced launch
+    int32_t* d_eta_snap = nullptr;             // eta as a sliced shared-memory launch reads it (taken before the launch)
     double* d_kat_out = nullptr;               // {dS, log accu_r} of bisbm_parallel_transition
     ncclComm_t comm = nullptr;                 // bisbm_nccl_init: communicator of the marginal-histogram all-reduce
     uint8_t* d_lab8 = nullptr;                 // u8 shadow of the labels for the shared-memory sweep
@@ -156,7 +157,7 @@ void dfree(T*& p) {
 
 void free_chains(bisbm_handle* h) {
     dfree(h->d_ka); dfree(h->d_kb); dfree(h->d_labels); dfree(h->d_labels_tmp);
-    dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_nr_live); dfree(h->d_kat_out); dfree(h->d_lab8);
+    dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_nr_live); dfree(h->d_eta_snap); dfree(h->d_kat_out); dfree(h->d_lab8);
     dfree(h->d_seeds); dfree(h->d_active); dfree(h->d_accepted); dfree(h->d_u); dfree(h->d_sweeps);
     dfree(h->d_dS); dfree(h->d_entmin); dfree(h->d_ent_out); dfree(h->d_nactive); dfree(h->d_hist);
     for (auto& kv : h->replay) { dfree(kv.second.d_rs); dfree(kv.second.d_vlist); dfree(kv.second.d_kh); }
@@ -781,6 +782,7 @@ SweepParams base_params(bisbm_handle* h, uint32_t type) {
     memset(&P, 0, sizeof P);
     P.g = gview(h); P.s = sview(h); P.tb = tview(h, false);
     P.lab8 = h->d_lab8; P.m_next = h->d_m2; P.e_next = h->d_e2; P.nr_next = h->d_nr2; P.nr_live = h->d_nr_live;
+    P.eta_read = h->d_eta;
     P.seeds = h->d_seeds; P.active = h->d_active; P.accepted = h->d_accepted; P.dS_accum = h->d_dS;
     P.lq = h->d_lq;
     P.n_chains = h->n_chains; P.type = type; P.n_groups = h->C / 32;
@@ -837,17 +839,21 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
             }
             if (sliced && s2) {
                 // next := -(publishers - 1) * base: every CTA adds its whole staged copy (sweep2.cuh)
-                const uint32_t nmax = std::max(n_m, n_e);
+                // and the moving type's eta into the snapshot the launch reads (its commits go to d_eta)
+                const uint32_t nmax = std::max(std::max(n_m, n_e), G * kmax * h->W * 32u);
                 sweep2_preinit_kernel<<<(nmax + 255) / 256, 256, 0, h->stream>>>(h->d_m, h->d_e, h->d_nr, h->d_m2, h->d_e2, h->d_nr2,
                                                                                  h->d_nr_live, n_m, n_e, h->KA, h->KB, type, lp.ctas_per_group - 1,
                                                                                  lp.cluster ? lp.ctas_per_group / lp.cluster - 1 : lp.ctas_per_group - 1,
-                                                                                 G, extras, l);
+                                                                                 G, extras, l, h->d_eta, h->d_eta_snap, h->W);
                 h->last_launches += 1;
             } else if (sliced) {  // next := base; the launch adds each CTA's (staged - base) into next
                 CU(cudaMemcpyAsync(h->d_m2, h->d_m, (size_t)n_m * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
                 CU(cudaMemcpyAsync(h->d_e2, h->d_e, (size_t)n_e * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
             }
             SweepParams P = base_params(h, type);
+            // sliced staged launches read eta as it was before the launch: what other CTAs commit meanwhile is not seen,
+            // so the result does not depend on their timing (the cluster form's counts are shared live anyway)
+            if (sliced && s2 && !lp.cluster) P.eta_read = h->d_eta_snap;
             P.ctas_per_group = lp.ctas_per_group; P.warps_used = lp.warps_used;
             P.pos_begin = (uint32_t)pos; P.pos_end = (uint32_t)std::min<uint64_t>(nv, pos + lp.slice);
             P.exclusive = sliced ? 0 : 1;
@@ -1158,6 +1164,7 @@ static int alloc_chains(bisbm_handle* h, uint32_t n_chains, const uint32_t* ka, 
         CU(cudaMalloc(&h->d_nr_live, (size_t)C * KK * sizeof(int32_t)));
         CU(cudaMalloc(&h->d_kat_out, 2 * sizeof(double)));
         CU(cudaMalloc(&h->d_eta, (size_t)C * KK * h->W * sizeof(int32_t)));
+        CU(cudaMalloc(&h->d_eta_snap, (size_t)C * KK * h->W * sizeof(int32_t)));
         CU(cudaMalloc(&h->d_lq, (size_t)C * KK * sizeof(LogqExp)));
         CU(cudaMalloc(&h->d_seeds, C * sizeof(uint64_t)));
         CU(cudaMalloc(&h->d_active, C));

@@ -77,6 +77,7 @@ struct SweepParams {
     // sweep2_kernel (sweep2.cuh)
     int32_t* nr_next;                // sliced launches: where the n_r view is added
     int32_t* nr_live;                // exact n_r counters for blocks small enough to empty within a launch
+    const int32_t* eta_read;         // sweep2: where eta is READ (a snapshot taken before a sliced launch; commits go to s.eta)
     uint32_t group_offset;           // first chain group of this launch (0 except for single-group launches)
     uint32_t kat_mode;               // 1: evaluate ONE forced proposal (kat_v -> own-type block kat_s of chain kat_chain) and write
     uint32_t kat_chain, kat_v, kat_s;   //    {dS, log accu_r} to kat_out instead of accepting / committing (bisbm_parallel_transition)

@@ -437,13 +437,22 @@ __device__ __noinline__ static double slow2_beta(int schedule, float p0, float p
 
 // next base of a sliced launch: every CTA of a group adds its whole staged copy (base + its deltas) into
 // `next`, so next starts at -(ctas_per_group - 1) * base for the arrays the CTAs publish (m_rs, and e_r / n_r of
-// the moving type) and at base for the frozen type's e_r / n_r.  nr_live := n_r (exact veto counters).
+// the moving type) and at base for the frozen type's e_r / n_r.  nr_live := n_r (exact veto counters).  eta_snap := eta of the moving type.
 __global__ void sweep2_preinit_kernel(const int32_t* __restrict__ m, const int32_t* __restrict__ e, const int32_t* __restrict__ nr,
                                       int32_t* __restrict__ m2, int32_t* __restrict__ e2, int32_t* __restrict__ nr2,
                                       int32_t* __restrict__ nr_live, uint32_t n_m, uint32_t n_e, uint32_t KA, uint32_t KB,
                                       uint32_t type, uint32_t mult, uint32_t mult_m,    // mult_m: publishers of m per group - 1 (clusters, or CTAs)
-                                      uint32_t n_groups, uint32_t extras, uint32_t launch_idx) {   // spare-SM CTAs: one more publisher in the groups that have one
+                                      uint32_t n_groups, uint32_t extras, uint32_t launch_idx,   // spare-SM CTAs: one more publisher in the groups that have one
+                                      const int32_t* __restrict__ eta, int32_t* __restrict__ eta_snap, uint32_t W) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    {   // eta_snap := eta for the moving type's blocks: the launch reads the snapshot and commits into eta
+        const uint32_t kown = type ? KB : KA, per = kown * W * 32u;
+        if (i < n_groups * per) {
+            const uint32_t g = i / per;
+            const size_t j = ((size_t)g * (KA + KB) + (type ? KA : 0u)) * W * 32u + (i - g * per);
+            eta_snap[j] = eta[j];
+        }
+    }
     auto extra_of = [&](uint32_t grp) -> uint32_t {
         if (extras == 0u) return 0u;
         const uint32_t slot0 = (uint32_t)(((uint64_t)launch_idx * extras) % n_groups);
@@ -475,6 +484,12 @@ __global__ void sweep2_preinit_kernel(const int32_t* __restrict__ m, const int32
 template <typename R, int KF, int TYPE, bool STAGED = true, int NT = 512, bool CLUSTER = false>
 __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ SweepParams P) {
     typedef Ar<R> AR;
+    // staged counts: the warps of a CTA take the vertices of a batch in fixed rounds (warp w: w, w + warps_used, ..), every
+    // warp of a round evaluates its move against the counts left by the rounds before, then all commit: the counts a move
+    // sees do not depend on timing, so a call's result is a function of its inputs -- except where a block of a chain is
+    // small enough to empty within the launch: the "would empty block r" veto below is an atomic decrement-and-check whose
+    // order among the moves out of r (other warps' in the commit phase, other CTAs' on nr_live) is not fixed
+    constexpr bool LOCKSTEP = STAGED && !CLUSTER;
     extern __shared__ __align__(128) unsigned char s2_smem[];
     unsigned char* const smem_raw = s2_smem;
     constexpr uint32_t FULL = 0xffffffffu;
@@ -505,6 +520,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     int32_t* const gNR = P.s.nr + (size_t)group * KK * GROUP;
     int32_t* const gLIVE = P.nr_live + (size_t)group * KK * GROUP + (size_t)own_off * 32;
     int32_t* const gETA = P.s.eta + (size_t)group * KK * W * GROUP + (size_t)own_off * W * 32;
+    const int32_t* const gETAr = P.eta_read + (size_t)group * KK * W * GROUP + (size_t)own_off * W * 32;
     const LogqExp* const gLQ = P.lq + ((size_t)group * KK + own_off) * GROUP;
 
     const uint32_t c = group * 32 + lane;
@@ -730,14 +746,22 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     auto lab_st = [&](uint32_t vtx, uint32_t x) {
         asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %0, %1, %2;\n\tst.global.u8 [a], %3;\n\t}" :: "r"(vtx), "r"(C), "l"(LAB8 + (uint64_t)lane), "r"(x) : "memory");
     };
+    uint32_t ticket = warp;                               // LOCKSTEP: this warp's next vertex of the batch
     auto pop = [&]() -> uint32_t {
+        if constexpr (LOCKSTEP) { const uint32_t i = ticket; ticket += P.warps_used; return i; }
         uint32_t i = 0;
         if (lane == 0) i = atomicAdd(sCtr, 1u);
         return __shfl_sync(FULL, i, 0);
     };
+    const uint32_t round_threads = P.warps_used * 32u;
+    auto round_barrier = [&]() {                          // LOCKSTEP: the warps that take vertices
+        if constexpr (LOCKSTEP) asm volatile("bar.sync 1, %0;" :: "r"(round_threads) : "memory");
+    };
 
     for (uint32_t j0 = 0;;) {
         if (warp < P.warps_used) {
+            ticket = warp;
+            uint32_t rounds = 0;
             // pipeline: while vertex k is evaluated, the rows and the own label of vertex k+1 are in flight
             uint32_t nxt = pop();
             uint4 ninfo = make_uint4(0, 0, 0, 0);
@@ -749,6 +773,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 r_nxt = lab_ld(ninfo.x);
             }
             while (nxt < nb) {
+                ++rounds;
                 const uint4 cur = ninfo;
                 uint32_t v = cur.x;
                 const uint32_t d = cur.z, didx = cur.w, r = r_nxt;
@@ -840,6 +865,8 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     // (src/metropolis_hasting.cc:47-52)
                     if (live && !cross && !T_zero && n_r != 1 && !P.kat_mode) ++n_acc;
                     issue_next();
+                    round_barrier();
+                    round_barrier();
                     continue;
                 }
 
@@ -915,8 +942,8 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 R dS;
                 // what stays in global memory -- eta (L2, updated by atomics) and the two log q expansions (read only) -- is
                 // requested first; the e_r terms below only need shared memory and cover part of the latency
-                const int eta_r = ldc(&gETA[(r * W + didx) * 32 + lane]);
-                const int eta_s = ldc(&gETA[(s * W + didx) * 32 + lane]);
+                const int eta_r = ldc(&gETAr[(r * W + didx) * 32 + lane]);
+                const int eta_s = ldc(&gETAr[(s * W + didx) * 32 + lane]);
                 const int n_s = no_ld(s);
                 {
                     const int e_r = eo_ld(r), e_s = eo_ld(s);
@@ -959,6 +986,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     }
                     // s == r: see above
                     if (live && !cross && s == r && !T_zero && n_r != 1 && !P.kat_mode) ++n_acc;
+                    round_barrier();                         // every warp of the round has read its counts
                     if (go && P.vary_k) {
                         no_red(r, -1);                       // estimate mode: a block may empty
                         occ_own += ((n_s == 0) ? 1 : 0) - ((n_r == 1) ? 1 : 0);
@@ -1041,7 +1069,10 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     ++n_acc;
                     ds_sum += (double)dS;
                 }
+                round_barrier();                             // every warp of the round has committed
             }
+            if constexpr (LOCKSTEP)                          // rounds of the batch in which this warp has no vertex
+                for (const uint32_t all = (nb + P.warps_used - 1u) / P.warps_used; rounds < all; ++rounds) { round_barrier(); round_barrier(); }
         }
         j0 += (uint32_t)S2_VB;
         if (j0 >= cnt) break;

@@ -39,3 +39,16 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
 def test_reference_arm_other_ranks_exit_without_work():
     r = _run({"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert r.returncode == 0 and r.stdout.strip() == ""
+
+
+def test_steps_and_dump_outputs_are_checked(tmp_path):
+    """No timed step, or --dump-outputs where it is not implemented (other workloads, several ranks): a usage error before
+    any work, nothing written."""
+    out = str(tmp_path / "out")
+    two_ranks = {"RANK": "0", "LOCAL_RANK": "0", "WORLD_SIZE": "2"}
+    for args, env in ((["--steps", "0"], {}), (["--impl", "reference", "--dump-outputs", out], {}),
+                      (["--workload", "c4", "--dump-outputs", out], {}), (["--dump-outputs", out], two_ranks)):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True, timeout=60,
+                           cwd=ROOT, env=dict(os.environ, **env))
+        assert r.returncode == 2 and r.stdout == "" and "error:" in r.stderr, (args, r.stderr)
+    assert not os.path.exists(out)
