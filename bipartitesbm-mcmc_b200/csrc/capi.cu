@@ -31,6 +31,7 @@
 #include "gltable.h"
 #include "sweep_aux.cuh"
 #include "sweep2.cuh"
+#include "tempering.cuh"
 
 using namespace bisbm;
 
@@ -145,6 +146,14 @@ struct bisbm_handle {
     // import / export) and the u8 shadow (sweep2 kernels, 8-bit import / export, marginals).  At most one is stale.
     bool lab32_stale = false;
     bool lab8_stale = true;
+    // parallel tempering (bisbm_tempering_set): a ladder of tp_rungs temperatures over the pool, device-resident (LadderView)
+    uint32_t tp_rungs = 0;
+    uint64_t tp_round = 0;                     // swap rounds since bisbm_tempering_set: the parity and the draw of the next one
+    double* d_tp_rung_beta = nullptr;
+    double* d_tp_beta = nullptr;
+    uint32_t *d_tp_rung_of = nullptr, *d_tp_chain_at = nullptr;
+    uint8_t* d_tp_trip = nullptr;
+    unsigned long long *d_tp_acc_prev = nullptr, *d_tp_stats = nullptr;
 };
 
 namespace {
@@ -155,7 +164,15 @@ void dfree(T*& p) {
     p = nullptr;
 }
 
+void free_ladder(bisbm_handle* h) {
+    dfree(h->d_tp_rung_beta); dfree(h->d_tp_beta); dfree(h->d_tp_rung_of); dfree(h->d_tp_chain_at); dfree(h->d_tp_trip);
+    dfree(h->d_tp_acc_prev); dfree(h->d_tp_stats);
+    h->tp_rungs = 0;
+    h->tp_round = 0;
+}
+
 void free_chains(bisbm_handle* h) {
+    free_ladder(h);
     dfree(h->d_ka); dfree(h->d_kb); dfree(h->d_labels); dfree(h->d_labels_tmp);
     dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_nr_live); dfree(h->d_eta_snap); dfree(h->d_kat_out); dfree(h->d_lab8);
     dfree(h->d_seeds); dfree(h->d_active); dfree(h->d_accepted); dfree(h->d_u); dfree(h->d_sweeps);
@@ -795,7 +812,9 @@ SweepParams base_params(bisbm_handle* h, uint32_t type) {
 
 // one full sweep = type-a half sweep + type-b half sweep (each preceded by the log q refresh
 // of the blocks that half sweep changes)
-int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_t sweep_in_call, uint32_t max_inflight) {
+// beta_chain (device, [C], may be null): per-chain 1/T of parallel tempering, which replaces the schedule
+int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_t sweep_in_call, uint32_t max_inflight,
+                      const double* beta_chain = nullptr) {
     uint32_t wpc = 32, cluster = 0;
     const int kernel = plan_kernel(h, &wpc, &cluster);
     if (!kern_is_s2(kernel)) {   // the round-1 kernels read the canonical labels (counts in L2) or the shadow (staged) and write the canonical ones
@@ -867,6 +886,7 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
                 if ((float)(hi - 1) < p0) { P.schedule = BISBM_CONSTANT; P.p0 = 1.0f; P.beta0 = 1.0; }
                 else if (!((float)lo < p0)) { P.schedule = BISBM_CONSTANT; P.p0 = 0.0f; P.beta0 = -1.0; }
             }
+            P.beta_chain = beta_chain;
             P.cluster_size = lp.cluster; P.rows_per_cta = lp.rows_per_cta; P.work_ctas = lp.work_ctas;
             P.extras = extras; P.launch_idx = l; P.per_cta = per_cta;
             const unsigned grid = P.n_groups * lp.ctas_per_group + extras;
@@ -1134,6 +1154,7 @@ static int alloc_chains(bisbm_handle* h, uint32_t n_chains, const uint32_t* ka, 
     if (n_chains == 0) return fail(BISBM_ERR_ARG, "n_chains must be > 0");
     if (!(eps > 0.0)) return fail(BISBM_ERR_ARG, "epsilon must be > 0");
     CU(cudaSetDevice(h->device));
+    free_ladder(h);      // a new pool has no ladder
     uint32_t KA = 0, KB = 0;
     for (uint32_t c = 0; c < n_chains; ++c) {
         if (ka[c] == 0 || kb[c] == 0) return fail(BISBM_ERR_ARG, "chain %u: ka and kb must be >= 1", c);
@@ -1781,14 +1802,14 @@ int bisbm_anneal(bisbm_handle* h, int schedule, float p0, float p1, uint64_t dur
 }
 
 // one sample of every chain's current labels into the histogram, straight from the array the sweep kernel keeps
-// current: the u8 shadow (sweep2 kernels) or the i32 labels
-static int launch_marginal(bisbm_handle* h) {
+// current: the u8 shadow (sweep2 kernels) or the i32 labels.  rung (device, may be null): only the chains at rung 0
+static int launch_marginal(bisbm_handle* h, const uint32_t* rung = nullptr) {
     const uint64_t mw = (uint64_t)h->n * (h->C / 32);
     const unsigned mgrid = (unsigned)((mw * 32 + 255) / 256);
     if (h->lab32_stale)
-        marginal_kernel<uint8_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_lab8, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width);
+        marginal_kernel<uint8_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_lab8, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width, rung);
     else
-        marginal_kernel<int32_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_labels, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width);
+        marginal_kernel<int32_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_labels, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width, rung);
     CU(cudaGetLastError());
     return BISBM_OK;
 }
@@ -1851,6 +1872,150 @@ int bisbm_marginalize(bisbm_handle* h, uint64_t burn_in, uint64_t sweeps, uint64
     float ms = 0.f;
     CU(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
     h->last_ms = ms;
+    return BISBM_OK;
+}
+
+// ---------------------------------------------------------------- parallel tempering
+static LadderView ladder_view(bisbm_handle* h) {
+    LadderView L;
+    L.R = h->tp_rungs; L.n_ladders = h->n_chains / h->tp_rungs;
+    L.rung_beta = h->d_tp_rung_beta; L.rung_of = h->d_tp_rung_of; L.chain_at = h->d_tp_chain_at; L.beta = h->d_tp_beta;
+    L.trip = h->d_tp_trip; L.acc_prev = h->d_tp_acc_prev; L.stats = h->d_tp_stats;
+    return L;
+}
+
+static size_t ladder_stats_len(uint32_t R, uint32_t n_ladders) { return 2 * (size_t)(R - 1) + 2 * (size_t)R + n_ladders; }
+
+int bisbm_tempering_set(bisbm_handle* h, uint32_t n_rungs, const double* temps, const uint32_t* rung_of_chain) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (n_rungs == 0) { free_ladder(h); return BISBM_OK; }
+    if (!temps) return fail(BISBM_ERR_ARG, "null temperatures");
+    const uint32_t n_chains = h->n_chains, R = n_rungs;
+    if (n_chains % R) return fail(BISBM_ERR_ARG, "%u rungs do not divide %u chains", R, n_chains);
+    for (uint32_t i = 0; i < R; ++i) {
+        if (!(temps[i] > 0.0) || !std::isfinite(temps[i])) return fail(BISBM_ERR_ARG, "temperature %u (%g) must be finite and > 0", i, temps[i]);
+        if (i && temps[i] < temps[i - 1]) return fail(BISBM_ERR_ARG, "temperatures must be non-decreasing (T%u = %g < T%u = %g)", i, temps[i], i - 1, temps[i - 1]);
+    }
+    const uint32_t n_ladders = n_chains / R, C = h->C;
+    std::vector<uint32_t> rung(C, 0), at(n_chains);
+    std::vector<double> rbeta(R), beta(C, 1.0);
+    std::vector<uint8_t> trip(n_chains);
+    for (uint32_t i = 0; i < R; ++i) rbeta[i] = 1.0 / temps[i];
+    for (uint32_t l = 0; l < n_ladders; ++l) {
+        std::vector<bool> seen(R, false);
+        for (uint32_t i = 0; i < R; ++i) {
+            const uint32_t c = l * R + i, r = rung_of_chain ? rung_of_chain[c] : i;
+            if (r >= R || seen[r]) return fail(BISBM_ERR_ARG, "rung_of_chain of ladder %u is not a permutation of 0..%u", l, R - 1);
+            seen[r] = true;
+            rung[c] = r; at[l * R + r] = c; beta[c] = rbeta[r]; trip[c] = r == 0 ? 1 : 0;
+        }
+    }
+    free_ladder(h);
+    const size_t ns = ladder_stats_len(R, n_ladders);
+    CU(cudaMalloc(&h->d_tp_rung_beta, R * sizeof(double)));
+    CU(cudaMalloc(&h->d_tp_beta, C * sizeof(double)));
+    CU(cudaMalloc(&h->d_tp_rung_of, C * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_tp_chain_at, n_chains * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_tp_trip, n_chains));
+    CU(cudaMalloc(&h->d_tp_acc_prev, C * sizeof(unsigned long long)));
+    CU(cudaMalloc(&h->d_tp_stats, ns * sizeof(unsigned long long)));
+    CU(cudaMemcpyAsync(h->d_tp_rung_beta, rbeta.data(), R * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_tp_beta, beta.data(), C * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_tp_rung_of, rung.data(), C * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_tp_chain_at, at.data(), n_chains * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_tp_trip, trip.data(), n_chains, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemsetAsync(h->d_tp_stats, 0, ns * sizeof(unsigned long long), h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    h->tp_rungs = R;
+    h->tp_round = 0;
+    return BISBM_OK;
+}
+
+int bisbm_tempering_run(bisbm_handle* h, uint64_t sweeps, uint64_t swap_every, uint64_t sample_every, const uint64_t* seeds,
+                        uint64_t swap_seed, uint32_t max_inflight, double* accept_ratio) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!h->tp_rungs) return fail(BISBM_ERR_STATE, "no ladder: call bisbm_tempering_set first");
+    if (swap_every == 0) return fail(BISBM_ERR_ARG, "swap interval must be >= 1");
+    if (sample_every && !h->d_hist) { rc = bisbm_marginals_clear(h); if (rc) return rc; }
+    rc = upload_seeds(h, seeds);
+    if (rc) return rc;
+    rc = sync_labels8(h);
+    if (rc) return rc;
+    const uint32_t C = h->C;
+    const LadderView L = ladder_view(h);
+    const unsigned lgrid = (L.n_ladders + 127) / 128;
+    {
+        std::vector<uint8_t> act(C, 0);
+        std::fill(act.begin(), act.begin() + h->n_chains, 1);
+        CU(cudaMemcpyAsync(h->d_active, act.data(), C, cudaMemcpyHostToDevice, h->stream));
+        CU(cudaMemsetAsync(h->d_accepted, 0, C * sizeof(unsigned long long), h->stream));
+        CU(cudaMemsetAsync(h->d_tp_acc_prev, 0, C * sizeof(unsigned long long), h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+    }
+    h->last_launches = 0; h->last_sweep_launches = 0; h->last_moves = 0; h->last_ms = 0.0;
+    h->last_marginal_launches = 0;
+    CU(cudaEventRecord(h->ev0, h->stream));
+    uint64_t unattributed = 0;       // sweeps whose moves the swap kernel has not yet credited to a rung
+    for (uint64_t sw = 0; sw < sweeps; ++sw) {
+        rc = launch_full_sweep(h, BISBM_CONSTANT, 1.0f, 0.0f, sw, max_inflight, h->d_tp_beta);
+        if (rc) return rc;
+        ++unattributed;
+        if ((sw + 1) % swap_every == 0) {
+            entropy_kernel<<<h->n_chains, 256, 0, h->stream>>>(gview(h), sview(h), tview(h, false), h->ent_base, h->n_chains,
+                                                               h->d_ent_out, h->opt_vary_k, nullptr);
+            tempering_swap_kernel<<<lgrid, 128, 0, h->stream>>>(L, h->d_ent_out, h->d_accepted, unattributed * h->n, 1, h->tp_round++, swap_seed);
+            CU(cudaGetLastError());
+            h->last_launches += 2;
+            unattributed = 0;
+        }
+        if (sample_every && (sw + 1) % sample_every == 0) {
+            rc = launch_marginal(h, h->d_tp_rung_of);
+            if (rc) return rc;
+            h->last_marginal_launches += 1;
+            h->last_launches += 1;
+        }
+    }
+    if (unattributed) {      // the sweeps after the last round: credited to the rungs the chains hold now
+        tempering_swap_kernel<<<lgrid, 128, 0, h->stream>>>(L, h->d_ent_out, h->d_accepted, unattributed * h->n, 0, 0, 0);
+        CU(cudaGetLastError());
+        h->last_launches += 1;
+    }
+    CU(cudaEventRecord(h->ev1, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaGetLastError());
+    float ms = 0.f;
+    CU(cudaEventElapsedTime(&ms, h->ev0, h->ev1));
+    h->last_ms = ms;
+    if (accept_ratio) {
+        std::vector<unsigned long long> acc(C);
+        CU(cudaMemcpy(acc.data(), h->d_accepted, C * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        for (uint32_t c = 0; c < h->n_chains; ++c) accept_ratio[c] = sweeps ? (double)acc[c] / ((double)sweeps * (double)h->n) : 0.0;
+    }
+    return BISBM_OK;
+}
+
+int bisbm_tempering_stats(bisbm_handle* h, uint32_t* rung_of_chain, uint64_t* swaps_tried, uint64_t* swaps_accepted,
+                          uint64_t* moves_tried, uint64_t* moves_accepted, uint64_t* round_trips) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!h->tp_rungs) return fail(BISBM_ERR_STATE, "no ladder: call bisbm_tempering_set first");
+    const uint32_t R = h->tp_rungs, n_ladders = h->n_chains / R;
+    std::vector<unsigned long long> st(ladder_stats_len(R, n_ladders));
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaMemcpy(st.data(), h->d_tp_stats, st.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+    if (rung_of_chain) CU(cudaMemcpy(rung_of_chain, h->d_tp_rung_of, h->n_chains * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    const unsigned long long* p = st.data();
+    if (swaps_tried) std::copy(p, p + (R - 1), swaps_tried);
+    p += R - 1;
+    if (swaps_accepted) std::copy(p, p + (R - 1), swaps_accepted);
+    p += R - 1;
+    if (moves_tried) std::copy(p, p + R, moves_tried);
+    p += R;
+    if (moves_accepted) std::copy(p, p + R, moves_accepted);
+    p += R;
+    if (round_trips) std::copy(p, p + n_ladders, round_trips);
     return BISBM_OK;
 }
 

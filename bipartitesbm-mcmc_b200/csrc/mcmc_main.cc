@@ -9,7 +9,9 @@
 //                          second engine) the label line is identical to the reference's
 //   --chains N             N parallel chains (restarts with randomised starts); prints the best
 //   --marginalize          README "marginalization": -b burn-in sweeps, -t sampling sweeps, one sample
-//                          every -f sweeps over --chains chains; prints the arg-max label per node
+//                          every -f sweeps over --chains chains; prints the arg-max label per node.  With
+//                          --tempering T0 T1 .. the chains form ladders of those temperatures (parallel tempering,
+//                          swaps every --swap_every sweeps) and only the chains at T0 are sampled
 //   --estimate             README "estimation" output format for fixed (Ka, Kb): CSV lines
 //                          sweep,Ka,Kb,loglik,labels... of the last 1000 samples
 //   -g / --merge, -u / --nature, or initial labels whose block counts differ from -z: the agglomerative
@@ -56,7 +58,7 @@ const Spec kSpecs[] = {
     {"help", 'h', 0},
     // README-only modes and the extensions of this build
     {"maximize", 0, 0}, {"estimate", 0, 0}, {"marginalize", 0, 0}, {"chains", 0, 1}, {"gen_seed", 0, 1},
-    {"device", 0, 1}, {"max_inflight", 0, 1}, {"gpus", 0, 1},
+    {"device", 0, 1}, {"max_inflight", 0, 1}, {"gpus", 0, 1}, {"tempering", 0, 2}, {"swap_every", 0, 1},
 };
 
 const Spec* find_spec(const std::string& tok) {
@@ -134,7 +136,12 @@ void usage(const char* argv0) {
                  "  --device arg (=0), --max_inflight arg (=0)\n"
                  "  --gpus arg (=1)                       GPUs of this node: the chains are dealt round-robin to devices\n"
                  "                                        device .. device+gpus-1 (graph replicated); --marginalize sums the\n"
-                 "                                        per-node histograms with one NCCL all-reduce\n";
+                 "                                        per-node histograms with one NCCL all-reduce\n"
+                 "  --tempering T0 T1 ...                 --marginalize with parallel tempering: the chains form ladders of\n"
+                 "                                        these temperatures (non-decreasing, T0 the cold one; --chains a\n"
+                 "                                        multiple of their count); -b burn-in and -t sampling sweeps, the\n"
+                 "                                        marginals sample only the chains at T0\n"
+                 "  --swap_every arg (=1)                 sweeps between two swap rounds of --tempering\n";
 }
 
 // the ladder of block counts between (start_a, start_b) and (end_a, end_b) (reference src/support/util.hh:99-146): the type
@@ -238,6 +245,17 @@ int main(int argc, char const* argv[]) {
     if (o.has("max_inflight") && !to_num(o.vals["max_inflight"][0], max_inflight)) { std::cerr << "bad value for --max_inflight\n"; return 1; }
     size_t gpus = 1;
     if (o.has("gpus") && (!to_num(o.vals["gpus"][0], gpus) || gpus == 0)) { std::cerr << "bad value for --gpus\n"; return 1; }
+    std::vector<double> temps;
+    size_t swap_every = 1;
+    for (auto& s : o.get("tempering")) { double v; if (!to_num(s, v)) { std::cerr << "bad value for --tempering\n"; return 1; } temps.push_back(v); }
+    if (o.has("swap_every") && (!to_num(o.vals["swap_every"][0], swap_every) || swap_every == 0)) { std::cerr << "bad value for --swap_every\n"; return 1; }
+    if (!temps.empty()) {
+        if (o.has("estimate")) { std::cerr << "--tempering does not combine with --estimate\n"; return 1; }
+        if (merge || nature) { std::cerr << "--tempering does not combine with the agglomerative paths (-g / -u)\n"; return 1; }
+        if (gpus > 1) { std::cerr << "--tempering runs on one GPU (no --gpus > 1)\n"; return 1; }
+        if (!o.has("marginalize")) { std::cerr << "--tempering needs --marginalize\n"; return 1; }
+        if (chains % temps.size()) { std::cerr << "--chains must be a multiple of the number of --tempering temperatures\n"; return 1; }
+    }
     if (gpus > chains) gpus = chains;
     // stdout carries the label line and nothing else: whatever NCCL has to say (its version banner under NCCL_DEBUG)
     // goes to stderr unless the user chose a file
@@ -469,7 +487,15 @@ int main(int argc, char const* argv[]) {
     if (o.has("marginalize") || o.has("estimate")) {
         // README modes: burn-in, then sampling at T = 1
         if (randomize && !check(bisbm_randomize(h, seeds.data()))) return 1;
-        if (o.has("marginalize")) {
+        if (o.has("marginalize") && !temps.empty()) {
+            // parallel tempering: burn-in without samples, then -t sweeps sampling the cold rung every -f sweeps
+            const size_t f = std::max<size_t>(sampling_frequency, 1);
+            if (!check(bisbm_marginals_clear(h)) || !check(bisbm_tempering_set(h, (uint32_t)temps.size(), temps.data(), nullptr))) return 1;
+            if (burn_in && !check(bisbm_tempering_run(h, burn_in, swap_every, 0, seeds.data(), (uint64_t)seed, (uint32_t)max_inflight, nullptr))) return 1;
+            if (!check(bisbm_tempering_run(h, sampling_steps, swap_every, f, seeds.data(), (uint64_t)seed, (uint32_t)max_inflight, nullptr))) return 1;
+            if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
+            output_vec(out, std::cout);
+        } else if (o.has("marginalize")) {
             if (!check(bisbm_marginals_clear(h))) return 1;
             if (!check(bisbm_marginalize(h, burn_in, sampling_steps, std::max<size_t>(sampling_frequency, 1), seeds.data(), (uint32_t)max_inflight))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;

@@ -92,6 +92,8 @@ struct SweepParams {
     uint32_t extras, launch_idx, per_cta;
     uint32_t vary_k;                 // estimate mode (README "estimation"): blocks may empty and be re-populated; the K-dependent
                                      // prior terms of the description length enter dS with the OCCUPIED block counts
+    const double* beta_chain;        // [C] parallel tempering: 1/T of each chain's rung, loaded once per lane (the launch then runs
+                                     // at constant temperature and schedule / p0 / beta0 are ignored); null: one schedule for all
 };
 
 // temperature of global step t (same five schedules as src/metropolis_hasting.cc:10-37,
@@ -445,8 +447,9 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     const uint32_t nv = type ? G.nb : G.na, v0 = type ? G.na : 0;
     const uint64_t pkey = (P.sweep * 2 + type) * 0x9E3779B97F4A7C15ull + (uint64_t)group * 0xD1B54A32D192ED03ull;
     constexpr int SAFE_NR = 8192;   // > any number of concurrently evaluated moves of one chain (<= 148 SMs * 32 warps)
-    const bool const_T = (P.schedule == 3);
-    const double T_const = (double)P.p0, beta_const = 1.0 / (double)P.p0;
+    const bool const_T = (P.schedule == 3) || P.beta_chain;
+    double T_const = (double)P.p0, beta_const = 1.0 / (double)P.p0;
+    if (P.beta_chain) { beta_const = P.beta_chain[cc]; T_const = 1.0 / beta_const; }   // (a ladder never holds T = 0)
 
     unsigned long long n_acc = 0;
     double ds_sum = 0.0;

@@ -702,7 +702,8 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     uint64_t LAB8 = (uint64_t)__cvta_generic_to_global(P.lab8 + (size_t)(group * 32u < C ? group * 32u : 0u));
     asm volatile("" : "+l"(LAB8));
     const uint32_t key0 = (uint32_t)P.seeds[cc], key1 = (uint32_t)(P.seeds[cc] >> 32);
-    const bool const_T = (P.schedule == 3);
+    const bool const_T = (P.schedule == 3) || P.beta_chain;
+    const R beta_lane = P.beta_chain ? (R)P.beta_chain[cc] : (R)P.beta0;   // parallel tempering: this chain's rung
     const bool movable_chain = live && (kown != 1);
     const uint32_t kat_lane = P.kat_mode ? (P.kat_chain & 31u) : 32u;
 
@@ -815,7 +816,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     else tq = (e < 32u) ? sh_ld_u8(tile_lane + e * TE) : lab_ld(__ldcg(G.col + cur.y + e));
                 }
                 tq = min(tq, kopp_max - 1u);
-                R beta = (R)P.beta0;
+                R beta = beta_lane;
                 if (!const_T) {
                     const uint64_t step = P.step_base + pos_begin + cta_in_group + (uint64_t)pos_index * cpg;
                     // abrupt_cool in line (a launch that straddles the switch; whole launches on one side arrive as constant T)

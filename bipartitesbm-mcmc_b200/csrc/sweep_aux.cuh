@@ -325,17 +325,17 @@ __global__ void bookkeep_kernel(uint32_t n_chains, uint8_t* active, const double
 // marginal accumulation: hist[v][g] += #chains with global label g at v.  One warp per (vertex, chain group): the 32
 // chains' labels are ONE 128-byte line of the chain-minor i32 labels (or one 32-byte sector of the u8 shadow, LabT =
 // uint8_t); lanes holding the same label elect one of them, which adds their count -- a handful of atomics per warp
-// instead of 32.
+// instead of 32.  rung (may be null = every chain): parallel tempering samples only the chains with rung[c] == 0.
 template <typename LabT>
 __global__ void marginal_kernel(GraphView G, const LabT* __restrict__ labels, uint32_t C, const uint32_t* __restrict__ ka,
-                                uint32_t n_chains, uint32_t* hist, uint32_t width) {
+                                uint32_t n_chains, uint32_t* hist, uint32_t width, const uint32_t* __restrict__ rung) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t n_groups = C / 32;
     const uint64_t w = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (w >= (uint64_t)G.n * n_groups) return;
     const uint32_t v = (uint32_t)(w / n_groups), c = (uint32_t)(w % n_groups) * 32 + lane;
-    uint32_t g = 0xffffffffu;     // padding lanes: a key of their own, never added
-    if (c < n_chains) {
+    uint32_t g = 0xffffffffu;     // padding lanes and masked chains: a key of their own, never added
+    if (c < n_chains && (!rung || rung[c] == 0)) {
         const uint32_t l = (uint32_t)labels[(size_t)v * C + c];
         g = v < G.na ? l : ka[c] + l;
     }

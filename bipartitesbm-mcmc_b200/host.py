@@ -77,6 +77,9 @@ SIGNATURES = {
     "bisbm_marginalize": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, _u64p, C.c_uint32]),
     "bisbm_marginals_clear": (C.c_int, [C.c_void_p]),
     "bisbm_marginal_sample": (C.c_int, [C.c_void_p]),
+    "bisbm_tempering_set": (C.c_int, [C.c_void_p, C.c_uint32, _dp, _u32p]),
+    "bisbm_tempering_run": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, _u64p, C.c_uint64, C.c_uint32, _dp]),
+    "bisbm_tempering_stats": (C.c_int, [C.c_void_p, _u32p, _u64p, _u64p, _u64p, _u64p, _u64p]),
     "bisbm_set_precision": (C.c_int, [C.c_void_p, C.c_int]),
     "bisbm_set_option": (C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     "bisbm_parallel_transition": (C.c_int, [C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, _dp, _dp]),
@@ -276,6 +279,21 @@ def grid_partition(graph, points, restarts, world, l2_cost=4.5, classify=None):
     return [sorted(o) for o in out]
 
 
+def geometric_ladder(t_min, t_max, n):
+    """n temperatures from t_min to t_max in constant ratio (t_min first: rung 0 is the cold one), for
+    ChainPool.tempering_set; n = 1 gives [t_min]."""
+    n = int(n)
+    if n < 1:
+        raise ValueError("a ladder needs at least one rung")
+    if not (0 < t_min <= t_max < np.inf):
+        raise ValueError("need 0 < t_min <= t_max < inf")
+    if n == 1:
+        return np.array([float(t_min)])
+    out = t_min * (t_max / t_min) ** (np.arange(n) / (n - 1))
+    out[-1] = t_max
+    return np.maximum.accumulate(out)
+
+
 def edge_to_adj(edge_list, N, na=None, nb=None, device=0):
     """reference src/graph_utilities.cc:36-49.  The bipartition (na, nb) must be given since
     the device graph validates it; N = na + nb."""
@@ -330,6 +348,50 @@ class ChainPool:
     def marginalize(self, burn_in, sweeps, every, seeds, max_inflight=0):
         seeds = np.ascontiguousarray(seeds, dtype=np.uint64)
         _check(self.L.bisbm_marginalize(self.g.h, burn_in, sweeps, every, _p(seeds, C.c_uint64), max_inflight))
+
+    # -- parallel tempering (include/bisbm.h)
+    def tempering_set(self, temps, rung_of_chain=None):
+        """Ladder of len(temps) non-decreasing temperatures over the pool (rung 0 = temps[0], the cold one): chains l R .. l R + R - 1
+        form ladder l.  rung_of_chain [n_chains] (optional) resumes a saved rung assignment.  temps = [] clears the ladder."""
+        t = np.ascontiguousarray(temps, dtype=np.float64).ravel()
+        if len(t) and self.n_chains % len(t):
+            raise ValueError("%d rungs do not divide %d chains" % (len(t), self.n_chains))
+        if not np.all(np.isfinite(t) & (t > 0)) or np.any(np.diff(t) < 0):
+            raise ValueError("temperatures must be finite, > 0 and non-decreasing")
+        rp = None
+        if rung_of_chain is not None:
+            rung_of_chain = np.ascontiguousarray(rung_of_chain, dtype=np.uint32)
+            if rung_of_chain.shape != (self.n_chains,):
+                raise ValueError("rung_of_chain must have one entry per chain")
+            rp = _p(rung_of_chain, C.c_uint32)
+        _check(self.L.bisbm_tempering_set(self.g.h, len(t), _p(t, C.c_double) if len(t) else None, rp))
+
+    def tempering_run(self, sweeps, swap_every, seeds, swap_seed=1, sample_every=0, max_inflight=0):
+        """sweeps full sweeps at each chain's rung temperature, a swap round every swap_every sweeps, a marginal sample of the
+        rung-0 chains every sample_every sweeps (0: none).  Returns the per-chain acceptance of this run."""
+        if int(swap_every) < 1:
+            raise ValueError("swap_every must be >= 1")
+        seeds = np.ascontiguousarray(seeds, dtype=np.uint64)
+        assert seeds.size == self.n_chains
+        acc = np.zeros(self.n_chains, dtype=np.float64)
+        _check(self.L.bisbm_tempering_run(self.g.h, int(sweeps), int(swap_every), int(sample_every), _p(seeds, C.c_uint64),
+                                          int(swap_seed), int(max_inflight), _p(acc, C.c_double)))
+        return acc
+
+    def tempering_stats(self):
+        """dict of numpy arrays: rung_of_chain [n_chains], swaps_tried / swaps_accepted [R-1] per adjacent pair, moves_tried /
+        moves_accepted [R] per rung, round_trips [n_ladders]."""
+        rung = np.zeros(self.n_chains, dtype=np.uint32)
+        _check(self.L.bisbm_tempering_stats(self.g.h, _p(rung, C.c_uint32), None, None, None, None, None))
+        R = int(rung.max()) + 1     # the library holds the ladder (however it was set): every ladder is a permutation of 0..R-1
+        out = {"rung_of_chain": rung,
+               "swaps_tried": np.zeros(R - 1, dtype=np.uint64), "swaps_accepted": np.zeros(R - 1, dtype=np.uint64),
+               "moves_tried": np.zeros(R, dtype=np.uint64), "moves_accepted": np.zeros(R, dtype=np.uint64),
+               "round_trips": np.zeros(self.n_chains // R, dtype=np.uint64)}
+        u64 = lambda k: _p(out[k], C.c_uint64) if out[k].size else None
+        _check(self.L.bisbm_tempering_stats(self.g.h, None, u64("swaps_tried"), u64("swaps_accepted"),
+                                            u64("moves_tried"), u64("moves_accepted"), u64("round_trips")))
+        return out
 
     def set_precision(self, mode):
         """'fp64' (default: the move is evaluated in double like the reference) or 'fp32'."""

@@ -140,6 +140,32 @@ int bisbm_marginalize(bisbm_handle* h, uint64_t burn_in, uint64_t sweeps, uint64
 int bisbm_marginals_clear(bisbm_handle* h);
 /* adds ONE sample of every chain's current labels to the histogram (asynchronous on the handle's stream) */
 int bisbm_marginal_sample(bisbm_handle* h);
+/* ---- parallel tempering (replica exchange; no counterpart in the reference) ----------------------------------------
+ * Ladder: n_rungs = R temperatures temps[0..R-1], each finite and > 0, non-decreasing; rung 0 is the cold one.  n_chains
+ * must be a multiple of R: chains l R .. l R + R - 1 form ladder l, and chain l R + i starts at rung i unless rung_of_chain
+ * is given (e.g. resuming from a checkpoint).  A swap exchanges the RUNGS of two chains of one ladder -- never their labels
+ * or counts.  A swap round follows every swap_every full sweeps; round k of a ladder proposes the pairs (i, i+1) with
+ * i = k (mod 2) (deterministic even-odd scheme), each accepted with probability min(1, exp((beta_i - beta_{i+1})(S_i -
+ * S_{i+1}))), S = entropy() of the chain's current state (in estimate mode, "vary_k", with the occupied block counts, as
+ * bisbm_entropy* use).  The uniform draw is Philox keyed by (swap_seed, ladder, round), a stream of its own.  The round
+ * counter lives on the handle: consecutive runs neither repeat draws nor restart the parity.  Per sweep of a run: full
+ * sweep -> swap round if due -> marginal sample of the rung-0 chains if due.  S, the rung maps and 1/T stay on the device;
+ * a run makes no host synchronisation per round.
+ * bisbm_anneal, bisbm_marginalize, bisbm_grid_search and bisbm_parallel_transition ignore any ladder.  bisbm_set_chains*
+ * clears it; bisbm_randomize keeps it.  Errors: BISBM_ERR_ARG for R not dividing n_chains, a temperature <= 0, NaN,
+ * infinite or decreasing, a bad rung permutation, swap_every == 0; BISBM_ERR_STATE for a run or stats call without a ladder.
+ * The counters persist until the next bisbm_tempering_set; bisbm_last_timing and bisbm_sweep_launches report a run like any
+ * other parallel call. */
+/* n_rungs = 0 clears the ladder; rung_of_chain may be NULL (identity), else each ladder's entries are a permutation of 0..R-1 */
+int bisbm_tempering_set(bisbm_handle* h, uint32_t n_rungs, const double* temps, const uint32_t* rung_of_chain);
+/* sample_every = 0: no marginal samples; accept_ratio[c] = accepted moves / (sweeps x N) of this run (may be NULL) */
+int bisbm_tempering_run(bisbm_handle* h, uint64_t sweeps, uint64_t swap_every, uint64_t sample_every,
+                        const uint64_t* seeds, uint64_t swap_seed, uint32_t max_inflight, double* accept_ratio);
+/* any pointer may be NULL.  rung_of_chain[n_chains]; swaps_tried / swaps_accepted[R-1] per adjacent pair (summed over
+ * ladders); moves_tried / moves_accepted[R] per rung (a chain's moves are attributed to the rung it held while making them);
+ * round_trips[n_ladders] (rung 0 -> rung R-1 -> rung 0 journeys completed by any chain of the ladder) */
+int bisbm_tempering_stats(bisbm_handle* h, uint32_t* rung_of_chain, uint64_t* swaps_tried, uint64_t* swaps_accepted,
+                          uint64_t* moves_tried, uint64_t* moves_accepted, uint64_t* round_trips);
 /* Arithmetic of the parallel sweep's per-move evaluation (dS, Hastings factor, accept test).  The reference
  * computes transition_ratio in double (src/metropolis_hasting.cc:103-192) and so does parallel mode by default
  * (BISBM_PRECISION_FP64).  BISBM_PRECISION_FP32 evaluates the move in fp32 on the MUFU unit (|error of the log
