@@ -2268,6 +2268,18 @@ int bisbm_set_option(bisbm_handle* h, const char* name, int64_t value) {
     return BISBM_OK;
 }
 
+#ifdef BISBM_ROUND_CLOCKS
+// instrumented builds only (scripts/round_clocks.py): copy the 8 counters of sweep2.cuh's g_round_clocks to `out`, then zero them
+int bisbm_round_clocks(unsigned long long* out) {
+    if (!out) return fail(BISBM_ERR_ARG, "null argument");
+    CU(cudaDeviceSynchronize());
+    CU(cudaMemcpyFromSymbol(out, g_round_clocks, sizeof(unsigned long long) * 8));
+    const unsigned long long zero[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    CU(cudaMemcpyToSymbol(g_round_clocks, zero, sizeof zero));
+    return BISBM_OK;
+}
+#endif
+
 int bisbm_parallel_transition(bisbm_handle* h, uint32_t chain, uint32_t v, uint32_t s, double* dS, double* log_accu) {
     int rc = need_chains(h);
     if (rc) return rc;

@@ -411,6 +411,31 @@ __device__ __forceinline__ int gl_atom(uint64_t base, uint32_t off, int v) {
     int o; asm volatile("{\n\t.reg .u64 a;\n\tcvt.u64.u32 a, %2;\n\tadd.u64 a, a, %1;\n\tatom.global.add.s32 %0, [a], %3;\n\t}" : "=r"(o) : "l"(base), "r"(off), "r"(v) : "memory"); return o;
 }
 
+#ifdef BISBM_ROUND_CLOCKS
+// instrumented builds (scripts/round_clocks.py): clock64 cycles of the staged sweep's warps, summed over all launches --
+// [0] proposal + pass, [1] dS / accept, [2] commit, [3] waiting at the barrier after the round's reads, [4] waiting at the
+// barrier after its commits, [5] vertices, [6] the longest proposal + pass of one vertex, [7] warp-rounds
+__device__ unsigned long long g_round_clocks[8];
+#define RC_DECL() long long rc[5] = {0, 0, 0, 0, 0}, rc_t = 0, rc_v0 = 0, rc_pass_max = 0; unsigned long long rc_n = 0, rc_rounds = 0
+#define RC_START() (rc_t = clock64())
+#define RC_MARK(ph) do { const long long t_ = clock64(); rc[ph] += t_ - rc_t; rc_t = t_; } while (0)
+#define RC_VSTART() (rc_v0 = rc[0], ++rc_rounds)
+#define RC_PASS() do { RC_MARK(0); rc_pass_max = max(rc_pass_max, rc[0] - rc_v0); ++rc_n; } while (0)
+#define RC_ROUND() (++rc_rounds)
+#define RC_PUBLISH(on) do { if (on) {                                                                                  \
+        for (int k_ = 0; k_ < 5; ++k_) atomicAdd(&g_round_clocks[k_], (unsigned long long)rc[k_]);                    \
+        atomicAdd(&g_round_clocks[5], rc_n); atomicMax(&g_round_clocks[6], (unsigned long long)rc_pass_max);          \
+        atomicAdd(&g_round_clocks[7], rc_rounds); } } while (0)
+#else
+#define RC_DECL() do {} while (0)
+#define RC_START() ((void)0)
+#define RC_MARK(ph) ((void)0)
+#define RC_VSTART() ((void)0)
+#define RC_PASS() ((void)0)
+#define RC_ROUND() ((void)0)
+#define RC_PUBLISH(on) ((void)0)
+#endif
+
 // the rare double-precision completions, out of line (arguments by value)
 __device__ __noinline__ static double slow2_block_degree_delta(int e_r, int e_s, int d) { return block_degree_delta(e_r, e_s, d); }
 // log q(e + de, n + dn) - log q(e, n) for a block without a valid expansion (small, or drifted out of its range): the exact
@@ -747,6 +772,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     auto lab_st = [&](uint32_t vtx, uint32_t x) {
         asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %0, %1, %2;\n\tst.global.u8 [a], %3;\n\t}" :: "r"(vtx), "r"(C), "l"(LAB8 + (uint64_t)lane), "r"(x) : "memory");
     };
+    RC_DECL();
     uint32_t ticket = warp;                               // LOCKSTEP: this warp's next vertex of the batch
     auto pop = [&]() -> uint32_t {
         if constexpr (LOCKSTEP) { const uint32_t i = ticket; ticket += P.warps_used; return i; }
@@ -763,6 +789,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         if (warp < P.warps_used) {
             ticket = warp;
             uint32_t rounds = 0;
+            RC_START();
             // pipeline: while vertex k is evaluated, the rows and the own label of vertex k+1 are in flight
             uint32_t nxt = pop();
             uint4 ninfo = make_uint4(0, 0, 0, 0);
@@ -775,6 +802,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
             }
             while (nxt < nb) {
                 ++rounds;
+                RC_VSTART();
                 const uint4 cur = ninfo;
                 uint32_t v = cur.x;
                 const uint32_t d = cur.z, didx = cur.w, r = r_nxt;
@@ -866,9 +894,21 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     // (src/metropolis_hasting.cc:47-52)
                     if (live && !cross && !T_zero && n_r != 1 && !P.kat_mode) ++n_acc;
                     issue_next();
+                    RC_PASS();
                     round_barrier();
+                    RC_MARK(3);
                     round_barrier();
+                    RC_MARK(4);
                     continue;
+                }
+                // eta of the move is requested before the pass: the pass's shared-memory round trips cover its L2 latency, which
+                // dS would otherwise wait for (+5.6 % on the C3 bench, profiles/r05_eta_early_ab.txt).  The staged one-CTA form
+                // commits only between the round's barriers, so these are the values a read after the pass would see; the
+                // cluster and counts-in-L2 forms read eta live and keep the read after the pass
+                int eta_r = 0, eta_s = 0;
+                if constexpr (LOCKSTEP) {
+                    eta_r = ldc(&gETAr[(r * W + didx) * 32 + lane]);
+                    eta_s = ldc(&gETAr[(s * W + didx) * 32 + lane]);
                 }
 
                 // ---- one pass over v's neighbours: dS and the Hastings factor (transition_ratio).  Every lane
@@ -937,14 +977,18 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 }
                 issue_next();
                 __syncwarp();
+                RC_PASS();
 
                 // ---- dS, accept (step) ----
                 bool go;
                 R dS;
-                // what stays in global memory -- eta (L2, updated by atomics) and the two log q expansions (read only) -- is
-                // requested first; the e_r terms below only need shared memory and cover part of the latency
-                const int eta_r = ldc(&gETAr[(r * W + didx) * 32 + lane]);
-                const int eta_s = ldc(&gETAr[(s * W + didx) * 32 + lane]);
+                // what stays in global memory -- the two log q expansions (read only) and, where it was not requested before the
+                // pass, eta (L2, updated by atomics) -- is requested first; the e_r terms below only need shared memory and cover
+                // part of the latency
+                if constexpr (!LOCKSTEP) {
+                    eta_r = ldc(&gETAr[(r * W + didx) * 32 + lane]);
+                    eta_s = ldc(&gETAr[(s * W + didx) * 32 + lane]);
+                }
                 const int n_s = no_ld(s);
                 {
                     const int e_r = eo_ld(r), e_s = eo_ld(s);
@@ -987,7 +1031,9 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     }
                     // s == r: see above
                     if (live && !cross && s == r && !T_zero && n_r != 1 && !P.kat_mode) ++n_acc;
+                    RC_MARK(1);
                     round_barrier();                         // every warp of the round has read its counts
+                    RC_MARK(3);
                     if (go && P.vary_k) {
                         no_red(r, -1);                       // estimate mode: a block may empty
                         occ_own += ((n_s == 0) ? 1 : 0) - ((n_r == 1) ? 1 : 0);
@@ -1070,10 +1116,14 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     ++n_acc;
                     ds_sum += (double)dS;
                 }
+                RC_MARK(2);
                 round_barrier();                             // every warp of the round has committed
+                RC_MARK(4);
             }
             if constexpr (LOCKSTEP)                          // rounds of the batch in which this warp has no vertex
-                for (const uint32_t all = (nb + P.warps_used - 1u) / P.warps_used; rounds < all; ++rounds) { round_barrier(); round_barrier(); }
+                for (const uint32_t all = (nb + P.warps_used - 1u) / P.warps_used; rounds < all; ++rounds) {
+                    RC_ROUND(); round_barrier(); RC_MARK(3); round_barrier(); RC_MARK(4);
+                }
         }
         j0 += (uint32_t)S2_VB;
         if (j0 >= cnt) break;
@@ -1081,6 +1131,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         nb = prepare(j0);
         __syncthreads();
     }
+    RC_PUBLISH(LOCKSTEP && warp < P.warps_used && lane == 0);
     if (warp < P.warps_used && live) {
         if (n_acc) atomicAdd(&P.accepted[c], (unsigned long long)n_acc);
         if (ds_sum != 0.0) atomicAdd(&P.dS_accum[c], ds_sum);
