@@ -128,7 +128,7 @@ struct bisbm_handle {
     // move arithmetic of the parallel sweep: double like the reference (default) or fp32 (sweep2.cuh)
     int precision = BISBM_PRECISION_FP64;
     // bisbm_set_option
-    int opt_kernel = -1;               // -1: automatic; KERN_L2 / KERN_STAGED_OLD force the round-1 double kernels
+    int opt_kernel = -1;               // -1: automatic; KERN_L2 forces the round-1 kernel, KERN_S2L_F64 sweep2 with counts in L2
     uint32_t opt_inflight_div = 64;    // default in-flight bound = half sweep / this
     int opt_generic = 0;               // 1: never take the Ka = Kb = 32 specialisation
     int opt_vary_k = 0;                // estimate mode: blocks may empty, K-dependent prior terms in dS
@@ -142,7 +142,7 @@ struct bisbm_handle {
     uint64_t last_sweep_launches = 0, last_marginal_launches = 0;
     uint32_t last_wpc = 0, last_cpg = 0, last_slice = 0;   // launch plan of the last half sweep
     int last_kernel = -1;                                   // KERN_* of the last parallel call
-    // two label arrays, refreshed from each other on demand: the canonical i32 labels (replay, round-1 kernels, 32-bit
+    // two label arrays, refreshed from each other on demand: the canonical i32 labels (replay, round-1 kernel, 32-bit
     // import / export) and the u8 shadow (sweep2 kernels, 8-bit import / export, marginals).  At most one is stale.
     bool lab32_stale = false;
     bool lab8_stale = true;
@@ -583,62 +583,39 @@ int validate_schedule(int schedule, float p0, float p1, uint64_t duration) {
     return BISBM_OK;
 }
 
-// kernels of the parallel sweep (bisbm_sweep_info reports which one ran)
-enum { KERN_L2 = 0, KERN_STAGED_OLD = 1, KERN_S2_F32 = 2, KERN_S2_F64 = 3, KERN_S2L_F32 = 4, KERN_S2L_F64 = 5, KERN_S2C_F32 = 6, KERN_S2C_F64 = 7 };
+// kernels of the parallel sweep (bisbm_sweep_info reports which one ran; ids 1, 6 and 7 are retired and not reused)
+enum { KERN_L2 = 0, KERN_S2_F32 = 2, KERN_S2_F64 = 3, KERN_S2L_F32 = 4, KERN_S2L_F64 = 5 };
 static inline bool kern_is_s2(int k) { return k >= KERN_S2_F32; }
-static inline bool kern_is_cluster(int k) { return k == KERN_S2C_F32 || k == KERN_S2C_F64; }   // m_rs distributed over a thread-block cluster
-static inline bool kern_is_s2_staged(int k) { return k == KERN_S2_F32 || k == KERN_S2_F64 || kern_is_cluster(k); }
-static inline bool kern_is_f32(int k) { return k == KERN_S2_F32 || k == KERN_S2L_F32 || k == KERN_S2C_F32; }
+static inline bool kern_is_s2_staged(int k) { return k == KERN_S2_F32 || k == KERN_S2_F64; }
+static inline bool kern_is_f32(int k) { return k == KERN_S2_F32 || k == KERN_S2L_F32; }
 
 struct LaunchPlan {
     int kernel;               // KERN_*
-    bool smem;                // counts staged in shared memory (every kernel except KERN_L2)
+    bool smem;                // counts staged in shared memory (KERN_S2_F32 / KERN_S2_F64)
     int hist_bytes;           // 1, 2 or 4
     uint32_t wpc;             // warps per CTA (blockDim / 32)
     uint32_t warps_used;      // of which take vertices
     uint32_t ctas_per_group;
     uint32_t slice;           // positions of the visiting order per launch
     size_t smem_bytes;
-    uint32_t work_ctas;       // CTAs per group that take vertices (cluster kernels may carry idle CTAs that only hold rows of m)
-    uint32_t cluster;         // CTAs per cluster (cluster kernels), else 0
-    uint32_t rows_per_cta;    // own-type rows of m per CTA of the cluster
 };
 
 const size_t kSmemMax = 227 * 1024;
 
 // Which kernel a parallel call uses -- decided ONCE for both half sweeps (the kernels keep different label
 // arrays current: the staged ones the u8 shadow, the L2 one the i32 labels), so asymmetric K can never mix them.
-int plan_kernel(const bisbm_handle* h, uint32_t* wpc_out, uint32_t* cluster_out = nullptr) {
+int plan_kernel(const bisbm_handle* h, uint32_t* wpc_out) {
     const uint32_t hb = h->max_degree <= 255u ? 1 : (h->max_degree <= 65535u ? 2 : 4);
     *wpc_out = 32;
-    if (cluster_out) *cluster_out = 0;
     if (h->opt_kernel == KERN_L2 && !h->opt_vary_k) return KERN_L2;
     const bool k8 = h->KA <= 256 && h->KB <= 256;
-    if (h->opt_kernel == KERN_STAGED_OLD) {
-        for (uint32_t w : {32u, 16u})
-            if (k8 && sweep_smem_bytes(true, h->KA, h->KB, 0, w, hb) <= 220 * 1024 &&
-                sweep_smem_bytes(true, h->KA, h->KB, 1, w, hb) <= 220 * 1024) { *wpc_out = w; return KERN_STAGED_OLD; }
-        return KERN_L2;
-    }
     if (hb == 1 && k8) {
         const uint32_t rs = h->precision == BISBM_PRECISION_FP32 ? 4u : 8u;
-        if (h->opt_kernel != KERN_S2L_F64 && h->opt_kernel != KERN_S2C_F64)
+        if (h->opt_kernel != KERN_S2L_F64)
             for (uint32_t w : {h->opt_warps, 16u, 8u, 4u})
                 if (sweep2_layout(h->KA, h->KB, 0, w, rs).total <= kSmemMax && sweep2_layout(h->KA, h->KB, 1, w, rs).total <= kSmemMax) {
                     *wpc_out = w;
                     return rs == 4 ? KERN_S2_F32 : KERN_S2_F64;
-                }
-        // on request (option "kernel" = 7): m_rs distributed over the shared memories of a thread-block cluster (portable sizes
-        // 2, 4, 8).  Measured slower than counts in L2 at K = 64 (distributed shared memory moves ~20 bytes per clock per SM:
-        // profiles/r02_experiments.txt), so it is not a default
-        if (h->opt_kernel == KERN_S2C_F64 && cluster_out)
-            for (uint32_t cs : {2u, 4u, 8u})
-                for (uint32_t w : {16u, 8u}) {
-                    const uint32_t ra = (h->KA + cs - 1) / cs, rb = (h->KB + cs - 1) / cs;
-                    if (sweep2_layout(h->KA, h->KB, 0, w, rs, true, ra).total <= kSmemMax && sweep2_layout(h->KA, h->KB, 1, w, rs, true, rb).total <= kSmemMax) {
-                        *wpc_out = w; *cluster_out = cs;
-                        return rs == 4 ? KERN_S2C_F32 : KERN_S2C_F64;
-                    }
                 }
         // larger still: the same kernel with m_rs / e_r / n_r in L2
         for (uint32_t w : {16u, 8u, 4u})
@@ -655,17 +632,17 @@ int plan_kernel(const bisbm_handle* h, uint32_t* wpc_out, uint32_t* cluster_out 
 //   one CTA per chain group  -> warps_used concurrent moves (shared-memory counts are exact)
 //   several CTAs per group   -> one slice of the visiting order per launch (a CTA sees the other
 //                               CTAs' moves of the same slice only in the next launch)
-int plan_sweep(bisbm_handle* h, uint32_t type, uint32_t max_inflight, int kernel, uint32_t wpc, LaunchPlan* lp, uint32_t cluster = 0) {
+int plan_sweep(bisbm_handle* h, uint32_t type, uint32_t max_inflight, int kernel, uint32_t wpc, LaunchPlan* lp) {
     const uint32_t nv = type ? h->nb : h->na;
     const uint32_t n_groups = h->C / 32;
     const uint32_t hb = h->max_degree <= 255u ? 1 : (h->max_degree <= 65535u ? 2 : 4);
     lp->hist_bytes = (int)hb;
     lp->kernel = kernel;
-    lp->smem = kernel != KERN_L2 && kernel != KERN_S2L_F32 && kernel != KERN_S2L_F64;
+    lp->smem = kern_is_s2_staged(kernel);
     if (kernel == KERN_L2) {
         wpc = 32;
-        if (sweep_smem_bytes(false, h->KA, h->KB, type, wpc, hb) > 220 * 1024) wpc = 16;
-        if (sweep_smem_bytes(false, h->KA, h->KB, type, wpc, hb) > 220 * 1024)
+        if (sweep_smem_bytes(h->KA, h->KB, type, wpc, hb) > 220 * 1024) wpc = 16;
+        if (sweep_smem_bytes(h->KA, h->KB, type, wpc, hb) > 220 * 1024)
             return fail(BISBM_ERR_ARG, "K too large for the shared-memory histogram");
     }
     // default bound: 1/inflight_div of the half sweep (DESIGN.md 4) -- also on small graphs, where it means
@@ -675,40 +652,29 @@ int plan_sweep(bisbm_handle* h, uint32_t type, uint32_t max_inflight, int kernel
     uint32_t cpg = std::max<uint32_t>(1, (uint32_t)h->sm_count / n_groups);
     cpg = std::min<uint32_t>(cpg, std::max<uint32_t>(1, inflight / wpc));
     cpg = std::min<uint32_t>(cpg, std::max<uint32_t>(1, nv / (wpc * 4)));
-    lp->cluster = kern_is_cluster(kernel) ? cluster : 0;
-    lp->rows_per_cta = 0;
-    if (lp->cluster) {      // whole clusters per group; a cluster of 4 only places on 132 of the 148 SMs (GPC granularity)
-        const uint32_t usable = cluster >= 4 ? (uint32_t)h->sm_count * 132u / 148u : (uint32_t)h->sm_count;
-        cpg = std::min<uint32_t>(cpg, std::max<uint32_t>(1, usable / n_groups));
-        lp->work_ctas = cpg;       // CTAs that take vertices (what the in-flight bound and the work allow) ...
-        cpg = std::max<uint32_t>(cluster, (cpg + cluster - 1) / cluster * cluster);   // ... inside whole clusters: the others only hold their rows of m
-        if (cpg * n_groups > usable) { cpg = std::max<uint32_t>(cluster, usable / n_groups / cluster * cluster); lp->work_ctas = std::min(lp->work_ctas, cpg); }
-        lp->rows_per_cta = ((type ? h->KB : h->KA) + cluster - 1) / cluster;
-    } else lp->work_ctas = cpg;
     lp->ctas_per_group = cpg;
     lp->wpc = wpc;
-    lp->warps_used = (lp->work_ctas == 1) ? std::max<uint32_t>(1, std::min<uint32_t>(wpc, std::min<uint32_t>(inflight, std::max<uint32_t>(nv, 1)))) : wpc;
+    lp->warps_used = (cpg == 1) ? std::max<uint32_t>(1, std::min<uint32_t>(wpc, std::min<uint32_t>(inflight, std::max<uint32_t>(nv, 1)))) : wpc;
     // slices only exist for staged counts shared by several CTAs; global counts are live for everybody.
     // A whole number of vertices per warp keeps the CTAs' shares equal.
-    if (lp->smem && lp->work_ctas > 1) {
-        const uint32_t wk = lp->work_ctas;
-        lp->slice = std::max<uint32_t>(wk * wpc, std::min<uint32_t>(inflight, nv));
-        lp->slice = std::max<uint32_t>(wk * wpc, lp->slice / (wk * wpc) * (wk * wpc));
+    if (lp->smem && cpg > 1) {
+        lp->slice = std::max<uint32_t>(cpg * wpc, std::min<uint32_t>(inflight, nv));
+        lp->slice = std::max<uint32_t>(cpg * wpc, lp->slice / (cpg * wpc) * (cpg * wpc));
     }
     else lp->slice = std::max<uint32_t>(nv, 1);
     if (kern_is_s2(kernel))
-        lp->smem_bytes = sweep2_layout(h->KA, h->KB, type, wpc, kern_is_f32(kernel) ? 4u : 8u, kern_is_s2_staged(kernel), lp->rows_per_cta).total;
+        lp->smem_bytes = sweep2_layout(h->KA, h->KB, type, wpc, kern_is_f32(kernel) ? 4u : 8u, lp->smem).total;
     else
-        lp->smem_bytes = sweep_smem_bytes(lp->smem, h->KA, h->KB, type, wpc, hb);
+        lp->smem_bytes = sweep_smem_bytes(h->KA, h->KB, type, wpc, hb);
     return BISBM_OK;
 }
 
-template <bool SMEM, typename HistT, int NT>
+template <typename HistT, int NT>
 int launch_sweep_t(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp) {
-    int rc = ensure_smem_attr(h, (const void*)sweep_kernel<SMEM, HistT, NT>, 220 * 1024);
+    int rc = ensure_smem_attr(h, (const void*)sweep_kernel<HistT, NT>, 220 * 1024);
     if (rc) return rc;
     const unsigned grid = P.n_groups * lp.ctas_per_group;
-    sweep_kernel<SMEM, HistT, NT><<<grid, NT, lp.smem_bytes, h->stream>>>(P);
+    sweep_kernel<HistT, NT><<<grid, NT, lp.smem_bytes, h->stream>>>(P);
     {
         const cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess)
@@ -718,17 +684,16 @@ int launch_sweep_t(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp) 
     return BISBM_OK;
 }
 
-template <bool SMEM, typename HistT>
+template <typename HistT>
 int launch_sweep_nt(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp) {
-    if (lp.wpc == 32) return launch_sweep_t<SMEM, HistT, 1024>(h, P, lp);
-    return launch_sweep_t<SMEM, HistT, 512>(h, P, lp);
+    if (lp.wpc == 32) return launch_sweep_t<HistT, 1024>(h, P, lp);
+    return launch_sweep_t<HistT, 512>(h, P, lp);
 }
 
-template <bool SMEM>
 int launch_sweep_h(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp) {
-    if (lp.hist_bytes == 1) return launch_sweep_nt<SMEM, uint8_t>(h, P, lp);
-    if (lp.hist_bytes == 2) return launch_sweep_nt<SMEM, uint16_t>(h, P, lp);
-    return launch_sweep_nt<SMEM, uint32_t>(h, P, lp);
+    if (lp.hist_bytes == 1) return launch_sweep_nt<uint8_t>(h, P, lp);
+    if (lp.hist_bytes == 2) return launch_sweep_nt<uint16_t>(h, P, lp);
+    return launch_sweep_nt<uint32_t>(h, P, lp);
 }
 
 template <typename R, int KF, int TYPE, bool STAGED = true, int NT = 512>
@@ -747,25 +712,8 @@ int launch_sweep2_t(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp,
 }
 
 template <typename R>
-int launch_sweep2_cluster(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp, unsigned grid) {
-    auto fn = sweep2_kernel<R, 0, 0, true, 512, true>;
-    int rc = ensure_smem_attr(h, (const void*)fn, (int)kSmemMax);
-    if (rc) return rc;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid); cfg.blockDim = dim3(lp.wpc * 32); cfg.dynamicSmemBytes = lp.smem_bytes; cfg.stream = h->stream;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = lp.cluster; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    CU(cudaLaunchKernelEx(&cfg, fn, P));
-    wrote_labels8(h);
-    return BISBM_OK;
-}
-
-template <typename R>
 int launch_sweep2(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp, unsigned grid) {
     if (!kern_is_s2(lp.kernel) || lp.wpc > 24) return fail(BISBM_ERR_STATE, "internal: sweep2 launcher with the plan of kernel %d (%u warps)", lp.kernel, lp.wpc);
-    if (lp.cluster) return launch_sweep2_cluster<R>(h, P, lp, grid);
     if (!lp.smem) return launch_sweep2_t<R, 0, 0, false>(h, P, lp, grid);
     // compile-time strides for the common Ka = Kb = 32 pool (BASELINE configs[2])
     if (h->KA == 32 && h->KB == 32 && !h->opt_generic) {
@@ -782,11 +730,10 @@ int launch_sweep2(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp, u
 // per kernel family by the optimiser, and a build of it was seen taking the sweep2 launcher with a round-1 plan.
 __attribute__((noinline)) int dispatch_sweep(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp, unsigned grid) {
     switch (lp.kernel) {
-        case KERN_S2_F64: case KERN_S2L_F64: case KERN_S2C_F64: return launch_sweep2<double>(h, P, lp, grid);
-        case KERN_S2_F32: case KERN_S2L_F32: case KERN_S2C_F32: return launch_sweep2<float>(h, P, lp, grid);
-        case KERN_STAGED_OLD: return launch_sweep_h<true>(h, P, lp);     // (the staged round-1 kernel writes both label arrays)
+        case KERN_S2_F64: case KERN_S2L_F64: return launch_sweep2<double>(h, P, lp, grid);
+        case KERN_S2_F32: case KERN_S2L_F32: return launch_sweep2<float>(h, P, lp, grid);
         case KERN_L2: {
-            const int rc = launch_sweep_h<false>(h, P, lp);
+            const int rc = launch_sweep_h(h, P, lp);
             wrote_labels32(h);
             return rc;
         }
@@ -815,13 +762,13 @@ SweepParams base_params(bisbm_handle* h, uint32_t type) {
 // beta_chain (device, [C], may be null): per-chain 1/T of parallel tempering, which replaces the schedule
 int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_t sweep_in_call, uint32_t max_inflight,
                       const double* beta_chain = nullptr) {
-    uint32_t wpc = 32, cluster = 0;
-    const int kernel = plan_kernel(h, &wpc, &cluster);
-    if (!kern_is_s2(kernel)) {   // the round-1 kernels read the canonical labels (counts in L2) or the shadow (staged) and write the canonical ones
+    uint32_t wpc = 32;
+    const int kernel = plan_kernel(h, &wpc);
+    if (!kern_is_s2(kernel)) {   // the round-1 kernel reads and writes the canonical labels
         int rc = sync_labels32(h);
         if (rc) return rc;
     }
-    {
+    {   // the sweep2 kernels read and write the u8 shadow (refreshed for the round-1 kernel too, which does not read it)
         int rc = sync_labels8(h);
         if (rc) return rc;
     }
@@ -829,50 +776,45 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
         const uint32_t nv = type ? h->nb : h->na;
         if (nv == 0) continue;
         LaunchPlan lp;
-        int rc = plan_sweep(h, type, max_inflight, kernel, wpc, &lp, cluster);
+        int rc = plan_sweep(h, type, max_inflight, kernel, wpc, &lp);
         if (rc) return rc;
         const uint32_t kmax = type ? h->KB : h->KA;
         const uint32_t tot = h->n_chains * kmax;
         logq_refresh_kernel<<<(tot * 16 + 127) / 128, 128, 0, h->stream>>>(sview(h), tview(h, false), h->d_lq, h->n_chains, type);
         h->last_launches += 1;
         const uint32_t n_m = h->C * h->KA * h->KB, n_e = h->C * (h->KA + h->KB);
-        const bool sliced = lp.smem && lp.work_ctas > 1;
-        const bool s2 = kern_is_s2(kernel);
+        const bool sliced = lp.smem && lp.ctas_per_group > 1;   // (only the staged sweep2 kernels are sliced)
         h->last_wpc = lp.wpc; h->last_cpg = lp.ctas_per_group; h->last_slice = lp.slice;
         h->last_kernel = kernel;
         // spare SMs: when the groups' CTAs do not fill the GPU (8 groups x 18 CTAs on 148 SMs), the rest are handed to the groups
         // in turn, one more CTA (and one more CTA's worth of positions) for `extras` groups per launch
         uint32_t extras = 0;
         const uint32_t G = h->C / 32;
-        if (sliced && s2 && !lp.cluster && h->opt_spare_sms && max_inflight == 0 && (uint32_t)h->sm_count > G * lp.ctas_per_group)   // (an explicit in-flight bound is kept to the letter)
+        if (sliced && h->opt_spare_sms && max_inflight == 0 && (uint32_t)h->sm_count > G * lp.ctas_per_group)   // (an explicit in-flight bound is kept to the letter)
             extras = std::min<uint32_t>((uint32_t)h->sm_count - G * lp.ctas_per_group, G - 1);
         const uint32_t per_cta = lp.slice / std::max<uint32_t>(1, lp.ctas_per_group);
         for (uint32_t l = 0;; ++l) {
             // the group that has been handed the fewest extra slots (the last one) decides when the half sweep is over
             const uint64_t pos = extras ? ((uint64_t)l * lp.ctas_per_group + ((uint64_t)l * extras) / G) * per_cta : (uint64_t)l * lp.slice;
             if (pos >= nv) break;
-            if (sliced && s2 && l != 0 && l % h->opt_logq_every == 0) {
+            if (sliced && l != 0 && l % h->opt_logq_every == 0) {
                 // the blocks whose (e_r, n_r) have left the inner part of their log q expansion's range are expanded again
                 logq_refresh_kernel<<<(tot * 16 + 127) / 128, 128, 0, h->stream>>>(sview(h), tview(h, false), h->d_lq, h->n_chains, type, 1u);
                 h->last_launches += 1;
             }
-            if (sliced && s2) {
+            if (sliced) {
                 // next := -(publishers - 1) * base: every CTA adds its whole staged copy (sweep2.cuh)
                 // and the moving type's eta into the snapshot the launch reads (its commits go to d_eta)
                 const uint32_t nmax = std::max(std::max(n_m, n_e), G * kmax * h->W * 32u);
                 sweep2_preinit_kernel<<<(nmax + 255) / 256, 256, 0, h->stream>>>(h->d_m, h->d_e, h->d_nr, h->d_m2, h->d_e2, h->d_nr2,
                                                                                  h->d_nr_live, n_m, n_e, h->KA, h->KB, type, lp.ctas_per_group - 1,
-                                                                                 lp.cluster ? lp.ctas_per_group / lp.cluster - 1 : lp.ctas_per_group - 1,
                                                                                  G, extras, l, h->d_eta, h->d_eta_snap, h->W);
                 h->last_launches += 1;
-            } else if (sliced) {  // next := base; the launch adds each CTA's (staged - base) into next
-                CU(cudaMemcpyAsync(h->d_m2, h->d_m, (size_t)n_m * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
-                CU(cudaMemcpyAsync(h->d_e2, h->d_e, (size_t)n_e * sizeof(int32_t), cudaMemcpyDeviceToDevice, h->stream));
             }
             SweepParams P = base_params(h, type);
             // sliced staged launches read eta as it was before the launch: what other CTAs commit meanwhile is not seen,
-            // so the result does not depend on their timing (the cluster form's counts are shared live anyway)
-            if (sliced && s2 && !lp.cluster) P.eta_read = h->d_eta_snap;
+            // so the result does not depend on their timing
+            if (sliced) P.eta_read = h->d_eta_snap;
             P.ctas_per_group = lp.ctas_per_group; P.warps_used = lp.warps_used;
             P.pos_begin = (uint32_t)pos; P.pos_end = (uint32_t)std::min<uint64_t>(nv, pos + lp.slice);
             P.exclusive = sliced ? 0 : 1;
@@ -887,7 +829,6 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
                 else if (!((float)lo < p0)) { P.schedule = BISBM_CONSTANT; P.p0 = 0.0f; P.beta0 = -1.0; }
             }
             P.beta_chain = beta_chain;
-            P.cluster_size = lp.cluster; P.rows_per_cta = lp.rows_per_cta; P.work_ctas = lp.work_ctas;
             P.extras = extras; P.launch_idx = l; P.per_cta = per_cta;
             const unsigned grid = P.n_groups * lp.ctas_per_group + extras;
             rc = dispatch_sweep(h, P, lp, grid);
@@ -895,8 +836,7 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
             h->last_launches += 1;
             h->last_sweep_launches += 1;
             if (sliced) {
-                std::swap(h->d_m, h->d_m2); std::swap(h->d_e, h->d_e2);
-                if (s2) std::swap(h->d_nr, h->d_nr2);
+                std::swap(h->d_m, h->d_m2); std::swap(h->d_e, h->d_e2); std::swap(h->d_nr, h->d_nr2);
             }
         }
     }
@@ -906,7 +846,7 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
 }
 
 // refresh the u8 label shadow from the canonical i32 labels (replay moves, 32-bit set_chains, randomize and the round-1
-// kernels only write the canonical array); no-op while the shadow is current
+// kernel only write the canonical array); no-op while the shadow is current
 int sync_labels8(bisbm_handle* h) {
     if (!h->lab8_stale) return BISBM_OK;
     const uint64_t total = (uint64_t)h->n * h->C;
@@ -2241,8 +2181,8 @@ int bisbm_set_option(bisbm_handle* h, const char* name, int64_t value) {
     if (!h || !name) return fail(BISBM_ERR_ARG, "null argument");
     const std::string k(name);
     if (k == "kernel") {
-        if (value != -1 && value != KERN_L2 && value != KERN_STAGED_OLD && value != KERN_S2L_F64 && value != KERN_S2C_F64)
-            return fail(BISBM_ERR_ARG, "kernel: -1 (automatic), 0 (round-1 kernel, counts in L2), 1 (round-1 staged double kernel), 5 (sweep2, counts in L2) or 7 (sweep2, counts distributed over a cluster)");
+        if (value != -1 && value != KERN_L2 && value != KERN_S2L_F64)
+            return fail(BISBM_ERR_ARG, "kernel: -1 (automatic), 0 (round-1 kernel, counts in L2) or 5 (sweep2, counts in L2)");
         h->opt_kernel = (int)value;
     } else if (k == "inflight_div") {
         if (value < 1 || value > (1 << 30)) return fail(BISBM_ERR_ARG, "inflight_div must be >= 1");
@@ -2292,8 +2232,8 @@ int bisbm_parallel_transition(bisbm_handle* h, uint32_t chain, uint32_t v, uint3
         if (log_accu) *log_accu = NAN;
         return BISBM_OK;
     }
-    uint32_t wpc = 32, cluster = 0;
-    const int kernel = plan_kernel(h, &wpc, &cluster);
+    uint32_t wpc = 32;
+    const int kernel = plan_kernel(h, &wpc);
     if (!kern_is_s2(kernel))
         return fail(BISBM_ERR_STATE, "bisbm_parallel_transition needs the sweep2 kernel (degrees > 255 or K > 256 per type take the round-1 kernel)");
     const uint32_t type = va ? 0 : 1;
@@ -2306,21 +2246,14 @@ int bisbm_parallel_transition(bisbm_handle* h, uint32_t chain, uint32_t v, uint3
     LaunchPlan lp;
     memset(&lp, 0, sizeof lp);
     lp.kernel = kernel; lp.smem = kern_is_s2_staged(kernel); lp.hist_bytes = 1; lp.wpc = wpc; lp.warps_used = 1; lp.ctas_per_group = 1; lp.slice = 1;
-    lp.cluster = kern_is_cluster(kernel) ? cluster : 0;
-    lp.rows_per_cta = lp.cluster ? ((type ? h->KB : h->KA) + cluster - 1) / cluster : 0;
-    if (lp.cluster) lp.ctas_per_group = lp.cluster;
-    lp.smem_bytes = sweep2_layout(h->KA, h->KB, type, wpc, kern_is_f32(kernel) ? 4u : 8u, lp.smem, lp.rows_per_cta).total;
+    lp.smem_bytes = sweep2_layout(h->KA, h->KB, type, wpc, kern_is_f32(kernel) ? 4u : 8u, lp.smem).total;
     SweepParams P = base_params(h, type);
     P.n_groups = 1; P.group_offset = chain / 32;
     P.ctas_per_group = 1; P.warps_used = 1; P.pos_begin = 0; P.pos_end = 1; P.exclusive = 1;
     P.schedule = BISBM_CONSTANT; P.p0 = 1.0f; P.p1 = 0.0f; P.beta0 = 1.0;
     P.kat_mode = 1; P.kat_chain = chain; P.kat_v = v; P.kat_s = va ? s : s - ka;
-    P.cluster_size = lp.cluster; P.rows_per_cta = lp.rows_per_cta;
-    if (lp.cluster) P.ctas_per_group = lp.cluster;
-    P.work_ctas = 1;
-    const unsigned kat_grid = lp.cluster ? lp.cluster : 1;
     const bool stale = h->lab32_stale;
-    rc = kern_is_f32(kernel) ? launch_sweep2<float>(h, P, lp, kat_grid) : launch_sweep2<double>(h, P, lp, kat_grid);
+    rc = kern_is_f32(kernel) ? launch_sweep2<float>(h, P, lp, 1) : launch_sweep2<double>(h, P, lp, 1);
     h->lab32_stale = stale;   // nothing was written
     if (rc) return rc;
     double out[2];

@@ -8,17 +8,11 @@
 // deltas keep the counts exactly consistent with the labels; concurrent moves of one chain
 // couple only through slightly stale count READS.
 //
-// Two variants of one kernel (template<bool SMEM>):
-//   SMEM = true   each CTA stages its chain group's m_rs (+ e_r, 1/(e_t + eps K)) in shared
-//                 memory, laid out [entry][lane] so every access is bank-conflict free; moves
-//                 read and commit there (shared atomics).  When several CTAs share a chain group
-//                 the half sweep is cut into slices (one launch each): a CTA's counts are exact
-//                 for its own moves and one slice stale for the others'; at the end of the launch
-//                 it adds (staged - base) into the next base with global reductions.
-//   SMEM = false  counts stay in HBM/L2 (K too large for shared memory): L2 loads (ld.global.cg)
-//                 and global atomics per move.
-// n_r and eta always live in global memory: the "would empty block r" veto of
-// apply_mcmc_moves needs an exact atomic decrement-and-check.
+// The round-1 kernel here keeps every count (m_rs, e_r, n_r, eta) in HBM/L2: L2 loads
+// (ld.global.cg) and global atomics per move, so every CTA sees every committed move at once
+// and the "would empty block r" veto of apply_mcmc_moves is an exact atomic
+// decrement-and-check.  It serves the graphs and K the staged kernel of sweep2.cuh cannot
+// take (hubs of degree > 255, K > 256 per type).
 //
 // Per move this is the arithmetic of the reference's step():
 //   proposal   single_vertex_change      reference src/blockmodel.cc:613-637
@@ -53,8 +47,8 @@ struct SweepParams {
     GraphView g;
     StateView s;                     // s.m / s.e = BASE counts of this launch
     Tables tb;
-    uint8_t* lab8;                   // SMEM variant: u8 shadow of the labels (chain-minor), 4x less gather traffic
-    int32_t* m_next;                 // SMEM variant with shared groups: where deltas are added
+    uint8_t* lab8;                   // sweep2_kernel: u8 shadow of the labels (chain-minor), 4x less gather traffic
+    int32_t* m_next;                 // staged sweep2_kernel, sliced launches: where the staged m_rs / e_r are added
     int32_t* e_next;
     const uint64_t* seeds;           // [C]
     const uint8_t* active;           // [C]
@@ -83,9 +77,6 @@ struct SweepParams {
     uint32_t kat_chain, kat_v, kat_s;   //    {dS, log accu_r} to kat_out instead of accepting / committing (bisbm_parallel_transition)
     double* kat_out;
     double beta0;                    // 1 / p0, computed once on the host (constant schedule: 1/T of every step)
-    uint32_t cluster_size;           // sweep2_kernel<.., CLUSTER>: CTAs per cluster (m_rs of the group distributed over their shared memories)
-    uint32_t rows_per_cta;           //   own-type blocks whose m rows one CTA of the cluster holds (ceil(kown_max / cluster_size))
-    uint32_t work_ctas;              //   CTAs per group that take vertices (<= ctas_per_group; the rest only hold their rows of m)
     // spare SMs (sliced staged launches whose groups x CTAs do not fill the GPU): `extras` more CTAs per launch, handed to the
     // groups in turn (extra slot number s of the half sweep goes to group s mod n_groups; launch l hands out slots
     // [l extras, (l+1) extras)); a group's positions then advance by (ctas_per_group + its extra) x per_cta per launch
@@ -181,12 +172,6 @@ BISBM_HD void acc_guard(MoveAcc& A) {  // keep the running products inside doubl
 // counts in global memory are updated with L2 atomics by every SM; L1 is not coherent, so every
 // count READ from global goes to L2 (ld.global.cg).
 __device__ __forceinline__ int ldc(const int32_t* p) { return __ldcg(p); }
-
-template <bool SMEM>
-__device__ __forceinline__ int cnt_ld(const int32_t* p) {
-    if (SMEM) return *p;
-    return __ldcg(p);
-}
 
 #endif  // __CUDACC__ (reopened below)
 
@@ -286,23 +271,13 @@ __global__ void logq_refresh_kernel(StateView s, Tables tb, LogqExp* lq, uint32_
     if (sub == 0) lq[off] = logq_from_stencil(e, n, f);
 }
 
-// shared memory of the SMEM variant, in this order:
-//   int32  sM  [KA*KB*32]      m_rs of the group, [a][b][lane]
-//   int32  sEo [kown_max*32]   e_r of the moving type's blocks
-//   int32  sEp [kopp_max*32]   e_t of the frozen type's blocks
-//   double sInv[kopp_max*32]   1 / (e_t + eps K)
-//   HistT  hist[warps][kopp_max*32]
-// the non-SMEM variant only has hist.
-__host__ __device__ inline size_t sweep_smem_bytes(bool smem, uint32_t KA, uint32_t KB, uint32_t type, uint32_t warps,
-                                                   uint32_t hist_bytes) {
-    const uint32_t kown = type ? KB : KA, kopp = type ? KA : KB;
-    size_t b = 0;
-    if (smem) b += (size_t)KA * KB * 128 + (size_t)kown * 128 + (size_t)kopp * 128 + (size_t)kopp * 256;
-    b += (size_t)warps * ((kopp * hist_bytes + 3) / 4) * 128;   // lane-major 32-bit words
-    return b;
+// shared memory of sweep_kernel: the warps' neighbour-block histograms, HistT hist[warps][kopp_max*32]
+__host__ __device__ inline size_t sweep_smem_bytes(uint32_t KA, uint32_t KB, uint32_t type, uint32_t warps, uint32_t hist_bytes) {
+    const uint32_t kopp = type ? KA : KB;
+    return (size_t)warps * ((kopp * hist_bytes + 3) / 4) * 128;   // lane-major 32-bit words
 }
 
-// 16-byte staged copy (all staged arrays are multiples of 128 bytes)
+// 16-byte staged copy (all staged arrays are multiples of 128 bytes; sweep2.cuh)
 __device__ __forceinline__ void copy_i4(int32_t* dst, const int32_t* src, uint32_t n_int) {
     const int4* s4 = reinterpret_cast<const int4*>(src);
     int4* d4 = reinterpret_cast<int4*>(dst);
@@ -317,12 +292,11 @@ __device__ __forceinline__ void copy_i4(int32_t* dst, const int32_t* src, uint32
 }
 
 // ---- explicit shared-space accesses on 32-bit shared addresses (ld/st/red.shared): the
-//      staged counts are only ever touched through these, so no generic-address LD/ATOM and no
-//      64-bit index arithmetic is left in the move loop ----
+//      staged counts of sweep2.cuh are only ever touched through these, so no generic-address
+//      LD/ATOM and no 64-bit index arithmetic is left in the move loop ----
 // (count / inverse loads are plain asm so the compiler may schedule them early; a value that is a
 //  few instructions stale is harmless -- other warps update the same entries concurrently anyway)
 __device__ __forceinline__ int sh_ld(uint32_t a) { int v; asm("ld.shared.s32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
-__device__ __forceinline__ double sh_ld_f64(uint32_t a) { double v; asm("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a)); return v; }
 __device__ __forceinline__ void sh_red_add(uint32_t a, int v) { asm volatile("red.shared.add.s32 [%0], %1;" :: "r"(a), "r"(v) : "memory"); }
 template <typename T> struct ShHist;
 template <> struct ShHist<uint8_t> {
@@ -338,22 +312,14 @@ template <> struct ShHist<uint32_t> {
     static __device__ __forceinline__ void st(uint32_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" :: "r"(a), "r"(v) : "memory"); }
 };
 
-// one lane's view of a count array: entry j of this chain is element [j*32] (elements of 4 bytes)
-template <bool SMEM> struct Cnt;
-template <> struct Cnt<true> {   // staged in shared memory
-    uint32_t base;               // shared byte address of entry 0 for this lane
-    __device__ __forceinline__ int ld(uint32_t idx32) const { return sh_ld(base + idx32 * 4u); }
-    __device__ __forceinline__ void add(uint32_t idx32, int v) const { sh_red_add(base + idx32 * 4u, v); }
-};
-template <> struct Cnt<false> {  // in global memory: L2 loads, global reductions
+// one lane's view of a count array in global memory: entry j of this chain is element [j*32]; L2 loads, global reductions
+struct Cnt {
     int32_t* p;
     __device__ __forceinline__ int ld(uint32_t idx32) const { return __ldcg(p + idx32); }
     __device__ __forceinline__ void add(uint32_t idx32, int v) const { atomicAdd(p + idx32, v); }
 };
 
-// KF > 0: specialisation for KA == KB == KF with the moving type TYPE fixed at compile time (all strides
-// and loop bounds become constants); KF == 0: generic, everything from SweepParams.
-template <bool SMEM, typename HistT, int NT, int KF = 0, int TYPE = 0>
+template <typename HistT, int NT>
 __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // lane / warp ids through volatile asm: the compiler must keep them in registers instead of
@@ -364,9 +330,9 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     warp >>= 5;
     const uint32_t wpc = blockDim.x >> 5;
     const GraphView& G = P.g;
-    const uint32_t type = KF ? (uint32_t)TYPE : P.type;
-    const uint32_t C = P.s.C, KB = KF ? (uint32_t)KF : P.s.KB, KA = KF ? (uint32_t)KF : P.s.KA, W = P.s.W, KK = KA + KB;
-    const uint32_t kown_max = type ? KB : KA, kopp_max = KF ? (uint32_t)KF : P.kopp_max;
+    const uint32_t type = P.type;
+    const uint32_t C = P.s.C, KB = P.s.KB, KA = P.s.KA, W = P.s.W, KK = KA + KB;
+    const uint32_t kown_max = type ? KB : KA, kopp_max = P.kopp_max;
     const uint32_t group = blockIdx.x % P.n_groups;
     const uint32_t cta_in_group = blockIdx.x / P.n_groups;
     const uint32_t own_off = type ? KA : 0, opp_off = type ? 0 : KA;
@@ -386,27 +352,7 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     const uint32_t kown = type ? kb : ka;
     const double eps = P.s.eps, epsK = eps * (double)K;
 
-    // ---- stage the group's counts ----
-    int32_t* sM = nullptr; int32_t* sEo = nullptr; int32_t* sEp; double* sInv; HistT* hist_all;
-    if (SMEM) {
-        sM = reinterpret_cast<int32_t*>(smem_raw);
-        sEo = sM + KA * KB * 32;
-        sEp = sEo + kown_max * 32;
-        sInv = reinterpret_cast<double*>(sEp + kopp_max * 32);
-        hist_all = reinterpret_cast<HistT*>(sInv + kopp_max * 32);
-        copy_i4(sM, gM, KA * KB * 32);
-        copy_i4(sEo, gE + own_off * 32, kown_max * 32);
-        for (uint32_t i = threadIdx.x; i < kopp_max * 32; i += blockDim.x) {
-            const int e = gE[opp_off * 32 + i];
-            const uint32_t ci = group * 32 + (i & 31);
-            const double Kc = (double)(P.s.ka[ci] + P.s.kb[ci]);
-            sEp[i] = e;
-            sInv[i] = 1.0 / ((double)e + eps * Kc);
-        }
-    } else {
-        sEp = nullptr; sInv = nullptr;
-        hist_all = reinterpret_cast<HistT*>(smem_raw);
-    }
+    HistT* const hist_all = reinterpret_cast<HistT*>(smem_raw);
     {
         uint32_t* hw = reinterpret_cast<uint32_t*>(hist_all);
         const uint32_t words = wpc * (((kopp_max * (uint32_t)sizeof(HistT) + 3u) / 4u)) * 32u;
@@ -415,16 +361,8 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     __syncthreads();
 
     // lane-private accessors (entry j of this chain at element j*32)
-    Cnt<SMEM> M, Eo, Ep;
-    uint32_t inv_base = 0;
-    if constexpr (SMEM) {
-        M.base = (uint32_t)__cvta_generic_to_shared(sM) + lane * 4u;
-        Eo.base = (uint32_t)__cvta_generic_to_shared(sEo) + lane * 4u;
-        Ep.base = (uint32_t)__cvta_generic_to_shared(sEp) + lane * 4u;
-        inv_base = (uint32_t)__cvta_generic_to_shared(sInv) + lane * 8u;
-    } else {
-        M.p = gM + lane; Eo.p = gE + own_off * 32 + lane; Ep.p = gE + opp_off * 32 + lane;
-    }
+    Cnt M, Eo, Ep;
+    M.p = gM + lane; Eo.p = gE + own_off * 32 + lane; Ep.p = gE + opp_off * 32 + lane;
     // histogram bins are packed BPW per 32-bit word and the words are LANE-MAJOR ([t / BPW][lane]), so
     // lane l only ever touches bank l: bin t of this lane is at hist_base + (t / BPW) * 128 + (t % BPW) * sizeof(HistT)
     constexpr uint32_t BPW = 4u / (uint32_t)sizeof(HistT);
@@ -437,11 +375,7 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     // m(x_own, t_opp) = M[x*sx + t*st]   (element indices, already multiplied by the 32-chain interleave)
     const uint32_t sx = (type ? 1u : KB) * 32u, st = (type ? KB : 1u) * 32u;
     int32_t* const LAB = P.s.labels;
-    uint8_t* const LAB8 = P.lab8;
-    auto label_of = [&](uint32_t vtx) -> uint32_t {
-        if constexpr (SMEM) return (uint32_t)LAB8[(size_t)vtx * C + cc];
-        else return (uint32_t)LAB[(size_t)vtx * C + cc];
-    };
+    auto label_of = [&](uint32_t vtx) -> uint32_t { return (uint32_t)LAB[(size_t)vtx * C + cc]; };
     const uint64_t seed = P.seeds[cc];
     const uint32_t key0 = (uint32_t)seed, key1 = (uint32_t)(seed >> 32);
     const uint32_t nv = type ? G.nb : G.na, v0 = type ? G.na : 0;
@@ -562,9 +496,7 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
                 ShHist<HistT>::st(ha, (uint32_t)(cnt + 1));
                 const uint32_t it = t * st;
                 const int m_r = M.ld(ir + it), m_s = M.ld(is + it);
-                double inv;
-                if constexpr (SMEM) inv = sh_ld_f64(inv_base + t * 256u);
-                else inv = 1.0 / ((double)Ep.ld(t * 32u) + epsK);
+                const double inv = 1.0 / ((double)Ep.ld(t * 32u) + epsK);
                 acc_edge(A, m_r, m_s, cnt, inv, eps);
             };
             uint32_t base = 0;
@@ -648,7 +580,6 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
                     atomicSub(&gETA[(r * W + didx) * 32 + lane], 1);
                     atomicAdd(&gETA[(s * W + didx) * 32 + lane], 1);
                     LAB[(size_t)v * C + cc] = (int32_t)s;
-                    if constexpr (SMEM) LAB8[(size_t)v * C + cc] = (uint8_t)s;
                     ++n_acc;
                     ds_sum += dS;
                 }
@@ -657,33 +588,6 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
         if (live) {
             if (n_acc) atomicAdd(&P.accepted[c], n_acc);
             if (ds_sum != 0.0) atomicAdd(&P.dS_accum[c], ds_sum);
-        }
-    }
-
-    // ---- publish the staged counts ----
-    if (SMEM) {
-        __syncthreads();
-        if (P.exclusive) {
-            copy_i4(gM, sM, KA * KB * 32);
-            copy_i4(gE + own_off * 32, sEo, kown_max * 32);
-        } else {
-            int32_t* const nM = P.m_next + (size_t)group * KA * KB * GROUP;
-            int32_t* const nE = P.e_next + (size_t)group * KK * GROUP + own_off * 32;
-            // two neighbouring int32 deltas per 64-bit reduction (d0 + d1 * 2^32 in two's complement: exact in any
-            // order since every final count is >= 0; see sweep_fast.cuh) -- half the L2 atomics of the burst
-            const int4* const s4 = reinterpret_cast<const int4*>(sM);
-            const int4* const g4 = reinterpret_cast<const int4*>(gM);
-            unsigned long long* const n8 = reinterpret_cast<unsigned long long*>(nM);
-            for (uint32_t i = threadIdx.x; i < KA * KB * 8; i += blockDim.x) {
-                const int4 a = g4[i], b = s4[i];
-                const int d0 = b.x - a.x, d1 = b.y - a.y, d2 = b.z - a.z, d3 = b.w - a.w;
-                if (d0 | d1) atomicAdd(&n8[2 * i], (unsigned long long)((long long)d0 + ((long long)d1 << 32)));
-                if (d2 | d3) atomicAdd(&n8[2 * i + 1], (unsigned long long)((long long)d2 + ((long long)d3 << 32)));
-            }
-            for (uint32_t i = threadIdx.x; i < kown_max * 32; i += blockDim.x) {
-                const int dlt = sEo[i] - gE[own_off * 32 + i];
-                if (dlt) atomicAdd(&nE[i], dlt);
-            }
         }
     }
 }

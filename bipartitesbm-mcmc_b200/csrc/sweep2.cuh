@@ -310,12 +310,11 @@ inline
 #ifdef __CUDACC__
 __host__ __device__
 #endif
-Sweep2Layout sweep2_layout(uint32_t KA, uint32_t KB, uint32_t type, uint32_t warps, uint32_t rsize, bool staged = true,
-                           uint32_t rows_per_cta = 0) {   // rows_per_cta > 0: cluster form, this CTA holds that many own-type rows of m
+Sweep2Layout sweep2_layout(uint32_t KA, uint32_t KB, uint32_t type, uint32_t warps, uint32_t rsize, bool staged = true) {
     const uint32_t kown = type ? KB : KA, kopp = type ? KA : KB;
     Sweep2Layout L;
     uint32_t o = 0;
-    L.oM = o; o += staged ? (rows_per_cta ? rows_per_cta * kopp : KA * KB) * 128u : 0u;        // counts in L2 (staged = false): only the read-only tables,
+    L.oM = o; o += staged ? KA * KB * 128u : 0u;        // counts in L2 (staged = false): only the read-only tables,
     L.oEo = o; o += staged ? kown * 128u : 0u;          // the vertex batch, the histograms and the label tiles
     L.oNo = o; o += staged ? kown * 128u : 0u;
     L.oEp = o; o += kopp * 128u;
@@ -381,17 +380,6 @@ __device__ __forceinline__ void bulk_red_add_s32(void* dst, uint32_t src, uint32
 __device__ __forceinline__ void bulk_commit_wait_all() {
     asm volatile("cp.async.bulk.commit_group;" ::: "memory");
     asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-}
-
-// thread-block cluster: rank, address of a shared-memory location in another CTA of the cluster, accesses through it, barrier
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t cluster_map(uint32_t saddr, uint32_t rank) {
-    uint32_t a; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(saddr), "r"(rank)); return a;
-}
-__device__ __forceinline__ int cl_ld(uint32_t a) { int v; asm volatile("ld.shared::cluster.s32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
-__device__ __forceinline__ void cl_red(uint32_t a, int v) { asm volatile("red.shared::cluster.add.s32 [%0], %1;" :: "r"(a), "r"(v) : "memory"); }
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
 }
 
 // counts kept in L2 (STAGED = false): every read goes to L2 (ld.global.cg: other SMs update them with reductions)
@@ -466,7 +454,7 @@ __device__ __noinline__ static double slow2_beta(int schedule, float p0, float p
 __global__ void sweep2_preinit_kernel(const int32_t* __restrict__ m, const int32_t* __restrict__ e, const int32_t* __restrict__ nr,
                                       int32_t* __restrict__ m2, int32_t* __restrict__ e2, int32_t* __restrict__ nr2,
                                       int32_t* __restrict__ nr_live, uint32_t n_m, uint32_t n_e, uint32_t KA, uint32_t KB,
-                                      uint32_t type, uint32_t mult, uint32_t mult_m,    // mult_m: publishers of m per group - 1 (clusters, or CTAs)
+                                      uint32_t type, uint32_t mult,                     // mult: publishers per group - 1
                                       uint32_t n_groups, uint32_t extras, uint32_t launch_idx,   // spare-SM CTAs: one more publisher in the groups that have one
                                       const int32_t* __restrict__ eta, int32_t* __restrict__ eta_snap, uint32_t W) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -483,7 +471,7 @@ __global__ void sweep2_preinit_kernel(const int32_t* __restrict__ m, const int32
         const uint32_t slot0 = (uint32_t)(((uint64_t)launch_idx * extras) % n_groups);
         return ((grp + n_groups - slot0) % n_groups < extras) ? 1u : 0u;
     };
-    if (i < n_m) m2[i] = (int32_t)(0u - (mult_m + extra_of(i / (KA * KB * 32u))) * (uint32_t)m[i]);
+    if (i < n_m) m2[i] = (int32_t)(0u - (mult + extra_of(i / (KA * KB * 32u))) * (uint32_t)m[i]);
     if (i < n_e) {
         const uint32_t slot = (i >> 5) % (KA + KB);
         const bool own = type ? (slot >= KA) : (slot < KA);
@@ -499,22 +487,16 @@ __global__ void sweep2_preinit_kernel(const int32_t* __restrict__ m, const int32
 // 512 threads (16 warps x 128 registers), one CTA per SM.  Preconditions (plan_sweep): max degree <= 255 (u8
 // histogram bins), K per type <= 256 (u8 labels).
 // STAGED = false: K too large for shared memory -- m_rs / e_r / n_r stay in L2 (loads .cg, commits by global reductions,
-// every CTA sees every committed move at once: no slices, no staging, no publish); the rest of the kernel is the same.
-// CLUSTER = true (K too large for one CTA's shared memory, up to ~64 + 64): the group's m_rs is DISTRIBUTED over the shared
-// memories of a thread-block cluster -- CTA k of the cluster holds the rows of own-type blocks [k RPC, (k+1) RPC) -- and every
-// CTA reads / reduces all of it through distributed shared memory (ld / red.shared::cluster).  The row of the source block r
-// and of the target s are fixed per vertex, so the pass and the commit address m(r,t), m(s,t) exactly as in the one-CTA form
-// (one multiply-add per edge on a per-vertex base); only the categorical scan walks all CTAs.  The cluster's copy is exact for
-// all its CTAs (no staleness inside a cluster); several clusters per group publish like several CTAs do.
-template <typename R, int KF, int TYPE, bool STAGED = true, int NT = 512, bool CLUSTER = false>
+// every CTA sees every committed move at once: no slices, no staging, no publish, warps take vertices from a shared counter);
+// the rest of the kernel is the same.
+template <typename R, int KF, int TYPE, bool STAGED = true, int NT = 512>
 __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ SweepParams P) {
     typedef Ar<R> AR;
-    // staged counts: the warps of a CTA take the vertices of a batch in fixed rounds (warp w: w, w + warps_used, ..), every
-    // warp of a round evaluates its move against the counts left by the rounds before, then all commit: the counts a move
+    // staged counts always run in fixed rounds: the warps of a CTA take the vertices of a batch in turn (warp w: w,
+    // w + warps_used, ..), every warp of a round evaluates its move against the counts left by the rounds before, then all commit: the counts a move
     // sees do not depend on timing, so a call's result is a function of its inputs -- except where a block of a chain is
     // small enough to empty within the launch: the "would empty block r" veto below is an atomic decrement-and-check whose
     // order among the moves out of r (other warps' in the commit phase, other CTAs' on nr_live) is not fixed
-    constexpr bool LOCKSTEP = STAGED && !CLUSTER;
     extern __shared__ __align__(128) unsigned char s2_smem[];
     unsigned char* const smem_raw = s2_smem;
     constexpr uint32_t FULL = 0xffffffffu;
@@ -527,17 +509,14 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     const uint32_t type = KF ? (uint32_t)TYPE : P.type;
     const uint32_t C = P.s.C, KB = KF ? (uint32_t)KF : P.s.KB, KA = KF ? (uint32_t)KF : P.s.KA, W = P.s.W, KK = KA + KB;
     const uint32_t kown_max = type ? KB : KA, kopp_max = type ? KA : KB;
-    static_assert(!CLUSTER || (STAGED && KF == 0), "the cluster form is a staged, generic-stride instantiation");
-    uint32_t crank = 0, csz = 1;
-    if constexpr (CLUSTER) { crank = cluster_ctarank(); csz = P.cluster_size; }
-    const uint32_t unit = CLUSTER ? blockIdx.x / csz : blockIdx.x;       // cluster (or CTA) index: consecutive units -> consecutive groups
-    // spare-SM CTAs come after the regular ones: extra CTA j of launch l takes slot l extras + j, i.e. group (slot mod n_groups)
-    const bool extra_cta = !CLUSTER && P.extras != 0u && unit >= P.n_groups * P.ctas_per_group;
+    // consecutive CTAs -> consecutive groups; spare-SM CTAs come after the regular ones: extra CTA j of launch l takes slot
+    // l extras + j, i.e. group (slot mod n_groups)
+    const uint32_t cta = blockIdx.x;
+    const bool extra_cta = P.extras != 0u && cta >= P.n_groups * P.ctas_per_group;
     const uint32_t slot0 = (uint32_t)(((uint64_t)P.launch_idx * P.extras) % P.n_groups);
-    const uint32_t grp0 = extra_cta ? (slot0 + (unit - P.n_groups * P.ctas_per_group)) % P.n_groups : unit % P.n_groups;
+    const uint32_t grp0 = extra_cta ? (slot0 + (cta - P.n_groups * P.ctas_per_group)) % P.n_groups : cta % P.n_groups;
     const uint32_t group = P.group_offset + grp0;
-    const uint32_t cta_in_group = CLUSTER ? (unit / P.n_groups) * csz + crank : (extra_cta ? P.ctas_per_group : unit / P.n_groups);
-    const uint32_t RPC = CLUSTER ? P.rows_per_cta : 0u;
+    const uint32_t cta_in_group = extra_cta ? P.ctas_per_group : cta / P.n_groups;
     const uint32_t own_off = type ? KA : 0, opp_off = type ? 0 : KA;
 
     int32_t* const gM = P.s.m + (size_t)group * KA * KB * GROUP;
@@ -556,7 +535,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     const R eps = (R)P.s.eps;
     const R epsK32 = (R)(P.s.eps * (double)K * 4294967296.0);   // threshold scale of the uniform-vs-categorical test
 
-    const Sweep2Layout L = sweep2_layout(KA, KB, type, wpc, (uint32_t)sizeof(R), STAGED, RPC);
+    const Sweep2Layout L = sweep2_layout(KA, KB, type, wpc, (uint32_t)sizeof(R), STAGED);
     const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(smem_raw);
     int32_t* const sM = reinterpret_cast<int32_t*>(smem_raw + L.oM);
     int32_t* const sEo = reinterpret_cast<int32_t*>(smem_raw + L.oEo);
@@ -577,26 +556,10 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         }
         __syncthreads();
         if (threadIdx.x == 0) {
-            const uint32_t bO = kown_max * 128u, bP = kopp_max * 128u;
-            if constexpr (CLUSTER) {
-                // this CTA's rows of m: own-type blocks [x0, x0 + nx).  Type a owns rows of the [KA][KB] array (contiguous);
-                // type b owns columns (one segment per row a), kept as [a][local b]
-                const uint32_t x0 = crank * RPC, nx = (x0 < kown_max) ? min(RPC, kown_max - x0) : 0u;
-                mbar_expect_tx(mbar, nx * kopp_max * 128u + 2u * bO + bP);
-                if (type == 0) {
-                    const uint32_t bM = nx * KB * 128u;
-                    const char* src = reinterpret_cast<const char*>(gM) + (size_t)x0 * KB * 128u;
-                    for (uint32_t off = 0; off < bM; off += 32768u) bulk_g2s(sbase + L.oM + off, src + off, min(32768u, bM - off), mbar);
-                } else if (nx) {
-                    for (uint32_t a = 0; a < KA; ++a)
-                        bulk_g2s(sbase + L.oM + a * RPC * 128u, reinterpret_cast<const char*>(gM) + ((size_t)a * KB + x0) * 128u, nx * 128u, mbar);
-                }
-            } else {
-            const uint32_t bM = KA * KB * 128u;
+            const uint32_t bM = KA * KB * 128u, bO = kown_max * 128u, bP = kopp_max * 128u;
             mbar_expect_tx(mbar, bM + 2u * bO + bP);
             for (uint32_t off = 0; off < bM; off += 32768u)
                 bulk_g2s(sbase + L.oM + off, reinterpret_cast<const char*>(gM) + off, min(32768u, bM - off), mbar);
-            }
             bulk_g2s(sbase + L.oEo, gE + own_off * 32, bO, mbar);
             bulk_g2s(sbase + L.oNo, gNR + own_off * 32, bO, mbar);
             bulk_g2s(sbase + L.oEp, gE + opp_off * 32, bP, mbar);
@@ -611,9 +574,9 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
 
     // ---- the CTA's share of the slice: positions pos_begin + cta + j * ctas_per_group, j < cnt ----
     const uint32_t nv = type ? G.nb : G.na, v0 = type ? G.na : 0;
-    uint32_t cpg = CLUSTER ? P.work_ctas : P.ctas_per_group;            // CTAs of the group that take vertices
+    uint32_t cpg = P.ctas_per_group;                                     // CTAs of the group that take vertices
     uint32_t pos_begin = P.pos_begin, pos_end = P.pos_end;
-    if (!CLUSTER && P.extras != 0u) {
+    if (P.extras != 0u) {
         // this group's slice: it has advanced by per_cta x (ctas_per_group per launch + one per extra slot it was handed so far)
         const uint64_t s0 = (uint64_t)P.launch_idx * P.extras;
         const uint32_t before = (uint32_t)((s0 + P.n_groups - 1u - grp0) / P.n_groups);
@@ -664,7 +627,6 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         }
     }
     __syncthreads();
-    if constexpr (CLUSTER) cluster_sync_all();      // every CTA's rows of m are in place before anybody reads them
 
     // estimate mode: occupied blocks of this lane's chain, per type (own type tracked through this warp's own moves)
     int occ_own = 0, occ_opp = 0;
@@ -689,30 +651,17 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     const uint32_t tile_st = tile_w + (lane >> 2) * 32u + (lane & 3u) * 8u;        // store base: row lane/4 (+ 8 j), chains 8 (lane%4) ..
     constexpr uint32_t TE = 32u;                                                   // bytes between consecutive edges of one chain
     // m(x_own, t_opp) at byte offset x*SX + t*ST of this lane's view of m_rs
-    const uint32_t SX = (type ? 1u : KB) * 128u, ST = (type ? (CLUSTER ? RPC : KB) : 1u) * 128u;
-    // cluster form: this lane's view of CTA k's rows starts at cbase0 + k * cstride in the shared::cluster window
-    uint32_t cbase0 = 0, cstride = 0;
-    if constexpr (CLUSTER) {
-        cbase0 = cluster_map(M_base, 0);
-        cstride = cluster_map(M_base, 1) - cbase0;
-        for (uint32_t k = 2; k < csz; ++k) if (cluster_map(M_base, k) != cbase0 + k * cstride) asm volatile("trap;");
-    }
-    const uint32_t rpc_rcp = CLUSTER ? (65536u + RPC - 1u) / RPC : 0u;      // x / RPC = (x * rpc_rcp) >> 16 for x < 256
-    // handle of own-type block x's row of m: byte offset (one CTA) or shared::cluster address (cluster)
-    auto m_row = [&](uint32_t x) -> uint32_t {
-        if constexpr (CLUSTER) { const uint32_t o = (x * rpc_rcp) >> 16; return cbase0 + o * cstride + (x - o * RPC) * SX; }
-        else return x * SX;
-    };
+    const uint32_t SX = (type ? 1u : KB) * 128u, ST = (type ? KB : 1u) * 128u;
     // count accessors: shared-memory views (STAGED) or the arrays in L2
     const uint64_t gMl = (uint64_t)__cvta_generic_to_global(gM + lane);
     const uint64_t gEol = (uint64_t)__cvta_generic_to_global(gE + own_off * 32 + lane);
     const uint64_t gNol = (uint64_t)__cvta_generic_to_global(gNR + own_off * 32 + lane);
     const uint32_t live_u = live ? 1u : 0u;
     auto m_ld = [&](uint32_t off) -> int {
-        if constexpr (CLUSTER) return cl_ld(off); else if constexpr (STAGED) return sh_ld(M_base + off); else return gl_ld(gMl, off, live_u);
+        if constexpr (STAGED) return sh_ld(M_base + off); else return gl_ld(gMl, off, live_u);
     };
     auto m_red = [&](uint32_t off, int v) {
-        if constexpr (CLUSTER) cl_red(off, v); else if constexpr (STAGED) sh_red_add(M_base + off, v); else gl_red(gMl, off, v);
+        if constexpr (STAGED) sh_red_add(M_base + off, v); else gl_red(gMl, off, v);
     };
     auto eo_ld = [&](uint32_t blk) -> int { if constexpr (STAGED) return sh_ld(Eo_base + blk * 128u); else return gl_ld(gEol, blk * 128u, live_u); };
     auto eo_red = [&](uint32_t blk, int v) { if constexpr (STAGED) sh_red_add(Eo_base + blk * 128u, v); else gl_red(gEol, blk * 128u, v); };
@@ -773,16 +722,16 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %0, %1, %2;\n\tst.global.u8 [a], %3;\n\t}" :: "r"(vtx), "r"(C), "l"(LAB8 + (uint64_t)lane), "r"(x) : "memory");
     };
     RC_DECL();
-    uint32_t ticket = warp;                               // LOCKSTEP: this warp's next vertex of the batch
+    uint32_t ticket = warp;                               // STAGED: this warp's next vertex of the batch
     auto pop = [&]() -> uint32_t {
-        if constexpr (LOCKSTEP) { const uint32_t i = ticket; ticket += P.warps_used; return i; }
+        if constexpr (STAGED) { const uint32_t i = ticket; ticket += P.warps_used; return i; }
         uint32_t i = 0;
         if (lane == 0) i = atomicAdd(sCtr, 1u);
         return __shfl_sync(FULL, i, 0);
     };
     const uint32_t round_threads = P.warps_used * 32u;
-    auto round_barrier = [&]() {                          // LOCKSTEP: the warps that take vertices
-        if constexpr (LOCKSTEP) asm volatile("bar.sync 1, %0;" :: "r"(round_threads) : "memory");
+    auto round_barrier = [&]() {                          // STAGED: the warps that take vertices
+        if constexpr (STAGED) asm volatile("bar.sync 1, %0;" :: "r"(round_threads) : "memory");
     };
 
     for (uint32_t j0 = 0;;) {
@@ -864,17 +813,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 // categorical over row m[t][.]: s = #{x : cum_x <= z}; wz tracks cum - z - 1 (negative while cum <= z)
                 int wz = -(int)mulhi32(rz, (uint32_t)e_t) - 1;
                 uint32_t cnt_le = 0;
-                if constexpr (CLUSTER) {
-                    for (uint32_t o = 0, x0 = 0; x0 < kown_max; ++o, x0 += RPC) {       // CTA o of the cluster holds blocks x0 ..
-                        uint32_t a = cbase0 + o * cstride + tq * ST;
-                        const uint32_t nx = min(RPC, kown_max - x0);
-#pragma unroll 4
-                        for (uint32_t x = 0; x < nx; ++x, a += SX) {
-                            wz += m_ld(a);
-                            cnt_le += ((uint32_t)wz) >> 31;
-                        }
-                    }
-                } else {
+                {
                     uint32_t a = tq * ST;
 #pragma unroll 8
                     for (uint32_t x = 0; x < kown_max; ++x, a += SX) {   // uniform bound; blocks >= kown hold 0
@@ -902,11 +841,11 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     continue;
                 }
                 // eta of the move is requested before the pass: the pass's shared-memory round trips cover its L2 latency, which
-                // dS would otherwise wait for (+5.6 % on the C3 bench, profiles/r05_eta_early_ab.txt).  The staged one-CTA form
-                // commits only between the round's barriers, so these are the values a read after the pass would see; the
-                // cluster and counts-in-L2 forms read eta live and keep the read after the pass
+                // dS would otherwise wait for (+5.6 % on the C3 bench, profiles/r05_eta_early_ab.txt).  The staged form commits
+                // only between the round's barriers, so these are the values a read after the pass would see; the counts-in-L2
+                // form reads eta live and keeps the read after the pass
                 int eta_r = 0, eta_s = 0;
-                if constexpr (LOCKSTEP) {
+                if constexpr (STAGED) {
                     eta_r = ldc(&gETAr[(r * W + didx) * 32 + lane]);
                     eta_s = ldc(&gETAr[(s * W + didx) * 32 + lane]);
                 }
@@ -914,7 +853,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 // ---- one pass over v's neighbours: dS and the Hastings factor (transition_ratio).  Every lane
                 //      runs it (masked lanes cost the same issue slots); only `eval` lanes may commit. ----
                 MAcc<R> A; macc_init(A);
-                const uint32_t Mr = m_row(r), Ms = m_row(s);
+                const uint32_t Mr = r * SX, Ms = s * SX;
                 // histogram bin of label t: word t / 4, byte t % 4 -- or, with exactly 8 words (the Ka = Kb = 32 instantiation),
                 // word t % 8, byte t / 8: the byte's shift is then t & 0x18, one instruction less per edge
                 auto h_sh = [&](uint32_t t) -> uint32_t { if constexpr (KF == 32) return t & 0x18u; else return (t & 3u) << 3; };
@@ -985,7 +924,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 // what stays in global memory -- the two log q expansions (read only) and, where it was not requested before the
                 // pass, eta (L2, updated by atomics) -- is requested first; the e_r terms below only need shared memory and cover
                 // part of the latency
-                if constexpr (!LOCKSTEP) {
+                if constexpr (!STAGED) {
                     eta_r = ldc(&gETAr[(r * W + didx) * 32 + lane]);
                     eta_s = ldc(&gETAr[(s * W + didx) * 32 + lane]);
                 }
@@ -1120,7 +1059,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                 round_barrier();                             // every warp of the round has committed
                 RC_MARK(4);
             }
-            if constexpr (LOCKSTEP)                          // rounds of the batch in which this warp has no vertex
+            if constexpr (STAGED)                            // rounds of the batch in which this warp has no vertex
                 for (const uint32_t all = (nb + P.warps_used - 1u) / P.warps_used; rounds < all; ++rounds) {
                     RC_ROUND(); round_barrier(); RC_MARK(3); round_barrier(); RC_MARK(4);
                 }
@@ -1131,44 +1070,16 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         nb = prepare(j0);
         __syncthreads();
     }
-    RC_PUBLISH(LOCKSTEP && warp < P.warps_used && lane == 0);
+    RC_PUBLISH(STAGED && warp < P.warps_used && lane == 0);
     if (warp < P.warps_used && live) {
         if (n_acc) atomicAdd(&P.accepted[c], (unsigned long long)n_acc);
         if (ds_sum != 0.0) atomicAdd(&P.dS_accum[c], ds_sum);
     }
 
     // ---- publish the staged counts ----
-    if constexpr (CLUSTER) cluster_sync_all();       // the other CTAs' reductions into this CTA's rows have landed; nobody touches them again
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // shared-memory writes of this thread -> visible to the bulk engine
     __syncthreads();
     if (P.kat_mode || !STAGED) return;
-    if constexpr (CLUSTER) {
-        if (P.exclusive) {     // one working CTA: its e_r / n_r views and the cluster's m are exact -> written back in place
-            const uint32_t x0 = crank * RPC, nx = (x0 < kown_max) ? min(RPC, kown_max - x0) : 0u;
-            if (type == 0) copy_i4(gM + (size_t)x0 * KB * 32, sM, nx * KB * 32);
-            else for (uint32_t a = 0; a < KA; ++a) copy_i4(gM + ((size_t)a * KB + x0) * 32, sM + a * RPC * 32, nx * 32);
-            if (cta_in_group == 0) {
-                copy_i4(gE + own_off * 32, sEo, kown_max * 32);
-                copy_i4(gNR + own_off * 32, sNo, kown_max * 32);
-            }
-            return;
-        }
-        if (threadIdx.x == 0) {
-            const uint32_t x0 = crank * RPC, nx = (x0 < kown_max) ? min(RPC, kown_max - x0) : 0u;
-            char* const nM = reinterpret_cast<char*>(P.m_next + (size_t)group * KA * KB * GROUP);
-            const uint32_t bO = kown_max * 128u;
-            if (type == 0) {
-                const uint32_t bM = nx * KB * 128u;
-                for (uint32_t off = 0; off < bM; off += 32768u) bulk_red_add_s32(nM + (size_t)x0 * KB * 128u + off, sbase + L.oM + off, min(32768u, bM - off));
-            } else if (nx) {
-                for (uint32_t a = 0; a < KA; ++a) bulk_red_add_s32(nM + ((size_t)a * KB + x0) * 128u, sbase + L.oM + a * RPC * 128u, nx * 128u);
-            }
-            bulk_red_add_s32(P.e_next + (size_t)group * KK * GROUP + own_off * 32, sbase + L.oEo, bO);
-            bulk_red_add_s32(P.nr_next + (size_t)group * KK * GROUP + own_off * 32, sbase + L.oNo, bO);
-            bulk_commit_wait_all();
-        }
-        return;
-    }
     if (P.exclusive) {
         copy_i4(gM, sM, KA * KB * 32);
         copy_i4(gE + own_off * 32, sEo, kown_max * 32);

@@ -409,7 +409,7 @@ class ChainPool:
 
     def sweep_info(self):
         """(kernel, warps per CTA, CTAs per chain group, slice) of the last parallel call; kernel 3 = sweep2<double>,
-        2 = sweep2<float>, 1 = round-1 staged double kernel, 0 = counts in L2."""
+        2 = sweep2<float>, 5 / 4 = sweep2<double / float> with counts in L2, 0 = round-1 kernel, counts in L2."""
         k, w, c, sl = C.c_int(), C.c_uint32(), C.c_uint32(), C.c_uint32()
         _check(self.L.bisbm_sweep_info(self.g.h, C.byref(k), C.byref(w), C.byref(c), C.byref(sl)))
         return k.value, w.value, c.value, sl.value

@@ -174,8 +174,8 @@ enum { BISBM_PRECISION_FP32 = 0, BISBM_PRECISION_FP64 = 1 };
 int bisbm_set_precision(bisbm_handle* h, int mode);
 /* Tuning options of the parallel sweep (no environment variables are read):
  *   "inflight_div"  default in-flight bound of bisbm_anneal(max_inflight = 0) = half sweep / value (default 64)
- *   "kernel"        -1 automatic; 0 / 1 force the round-1 kernels (counts in L2 / staged, double); 5 force sweep2 with
- *                   counts in L2; 7 sweep2 with m_rs distributed over a thread-block cluster (A/B runs and tests)
+ *   "kernel"        -1 automatic; 0 force the round-1 kernel (double, counts in L2); 5 force sweep2 with counts in L2
+ *                   (the kernels the automatic choice takes for hubs and for large K); other values are rejected
  *   "generic"       1: never take the Ka = Kb = 32 compile-time specialisation
  *   "spare_sms"     0: do not hand the SMs that n_groups x ctas_per_group leaves idle to the chain groups in turn (default 1;
  *                   only with max_inflight = 0: a group holding a spare CTA evaluates one more CTA's worth of moves per launch)
@@ -187,10 +187,10 @@ int bisbm_set_precision(bisbm_handle* h, int mode);
  *                   bisbm_replay_agg_merge with a negative diff (agg_split) adds to a chain */
 int bisbm_set_option(bisbm_handle* h, const char* name, int64_t value);
 /* which sweep kernel the last parallel call launched and how the half sweep was cut:
- * kernel 0 = round-1 sweep_kernel (double, counts in L2: hubs of degree > 255, K > 256 per type); 1 = round-1 staged
- * double kernel; 2 / 3 = sweep2_kernel<float / double>, counts staged in shared memory (3 is the default);
- * 4 / 5 = sweep2_kernel<float / double>, counts in L2 (K too large for shared memory); 6 / 7 = sweep2_kernel<float /
- * double>, m_rs distributed over a thread-block cluster (on request);
+ * kernel 0 = round-1 sweep_kernel (double, counts in L2: hubs of degree > 255, K > 256 per type);
+ * 2 / 3 = sweep2_kernel<float / double>, counts staged in shared memory (3 is the default);
+ * 4 / 5 = sweep2_kernel<float / double>, counts in L2 (K too large for shared memory);
+ * ids 1, 6 and 7 (the retired round-1 staged kernel and sweep2's thread-block-cluster form) are no longer produced;
  * slice = vertices of the visiting order per launch (the staleness bound between CTAs of one chain group) */
 int bisbm_sweep_info(bisbm_handle* h, int* kernel, uint32_t* warps_per_cta, uint32_t* ctas_per_group, uint32_t* slice);
 /* transition_ratio (src/metropolis_hasting.cc:103-192) for moving v to global block s in chain `chain`, evaluated by the

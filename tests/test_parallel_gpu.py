@@ -175,66 +175,47 @@ def test_large_graph_invariants_and_logq_expansion(host):
         assert abs((f2[c] - f1[c]) - pool2.entropy_accum(c)) <= 1e-6 * abs(f1[c])
 
 
-@pytest.mark.parametrize("kernel", [-1, 7, 0])
+@pytest.mark.parametrize("kernel", [-1, 0, 4])
 def test_large_k_kernels(host, kernel):
     """K too large for one CTA's shared memory (KA*KB*128 B > 220 KB): the counts stay in L2 and commits are global
-    atomics -- sweep2_kernel<.., STAGED = false> (kernel 5) by default, the round-1 kernel (0) on request -- or, on request,
-    m_rs is distributed over the shared memories of a thread-block cluster (sweep2_kernel<.., CLUSTER>, kernel 7).
-    Same invariants; sequential chains are exact."""
+    atomics -- sweep2_kernel<double, .., STAGED = false> (kernel 5) by default, the round-1 kernel (0) on request, and
+    sweep2_kernel<float, .., STAGED = false> (4) as the automatic choice in fp32 precision.  Same invariants; sequential
+    chains are exact.  The retired kernel ids 1 (round-1 staged) and 7 (sweep2 over a thread-block cluster) are
+    rejected."""
     na = nb = 3000
     ka = kb = 48
     edges = planted(na, nb, 8, 8, 60000, 11)
     graph = host.Graph(edges, na, nb)
     C = 33
     lab0 = np.concatenate([np.arange(na) % ka, ka + np.arange(nb) % kb]).astype(np.uint32)
+    option = -1 if kernel == 4 else kernel
+    precision = "fp32" if kernel == 4 else "fp64"
     pool = host.ChainPool(graph, np.tile(lab0, (C, 1)), ka, kb, 1.0)
-    pool.set_option("kernel", kernel)
+    for retired in (1, 7):
+        with pytest.raises(host.BisbmError) as ei:
+            pool.set_option("kernel", retired)
+        assert ei.value.code == 1     # BISBM_ERR_ARG
+    pool.set_option("kernel", option)
+    pool.set_precision(precision)
     seeds = np.arange(C, dtype=np.uint64) + 31
     pool.randomize(seeds)
     e1 = pool.entropy()
     pool.anneal("constant", 1.0, 0.0, 4 * (na + nb), 10 ** 9, seeds)
-    assert pool.sweep_info()[0] == {-1: 5, 7: 7, 0: 0}[kernel]
+    assert pool.sweep_info()[0] == {-1: 5, 0: 0, 4: 4}[kernel]
     check_invariants(pool, edges, na, nb, [0, 31, 32])
     pool.anneal("abrupt_cool", 2.0 * (na + nb), 0.0, 6 * (na + nb), 10 ** 9, seeds, max_inflight=1)
     check_invariants(pool, edges, na, nb, [0, 32])
     e2 = pool.entropy()
     assert (e2 < e1).all()
     pool2 = host.ChainPool(graph, np.tile(lab0, (C, 1)), ka, kb, 1.0)
-    pool2.set_option("kernel", kernel)
+    pool2.set_option("kernel", option)
+    pool2.set_precision(precision)
     pool2.randomize(seeds)
     f1 = pool2.entropy()
     pool2.anneal("constant", 1.0, 0.0, 2 * (na + nb), 10 ** 9, seeds, max_inflight=1)
     f2 = pool2.entropy()
     for c in (0, 32):
         assert abs((f2[c] - f1[c]) - pool2.entropy_accum(c)) <= 1e-6 * abs(f1[c])
-
-
-def test_cluster_kernel_many_clusters_per_group(host):
-    """The cluster form (opt-in, option "kernel" = 7) on a graph large enough for several clusters per chain group (sliced launches: every cluster adds its
-    rows of m, every CTA its e_r / n_r views, into the next base): counts == rebuild from the labels, acceptance and
-    description length agree with the counts-in-L2 form of the same kernel on the same seeds' statistics."""
-    na = nb = 60000
-    ka = kb = 64
-    edges = planted(na, nb, 16, 16, 1200000, 5)
-    graph = host.Graph(edges, na, nb)
-    C = 64
-    lab0 = np.concatenate([np.arange(na) * ka // na, ka + np.arange(nb) * kb // nb]).astype(np.uint32)
-    res = {}
-    for kernel in (7, 5):
-        pool = host.ChainPool(graph, np.tile(lab0, (C, 1)), ka, kb, 1.0)
-        pool.set_option("kernel", kernel)
-        seeds = np.arange(C, dtype=np.uint64) + 3
-        pool.randomize(seeds)
-        acc, sw = pool.anneal("constant", 1.0, 0.0, 6 * (na + nb), 10 ** 9, seeds)
-        kern, wpc, cpg, sl = pool.sweep_info()
-        assert kern == kernel
-        if kernel == 7:
-            assert cpg >= 8 and sl < na          # several clusters per group, sliced
-        check_invariants(pool, edges, na, nb, [0, 31, 32, 63])
-        res[kernel] = (acc.copy(), pool.entropy().copy())
-    from scipy.stats import ks_2samp
-    assert ks_2samp(res[7][0], res[5][0]).pvalue > 0.001
-    assert ks_2samp(res[7][1], res[5][1]).pvalue > 0.001
 
 
 def test_ka_kb_grid_of_chains(host):
@@ -446,7 +427,7 @@ def test_asymmetric_and_borderline_k(host, ka, kb):
     assert (sw == 3).all() and (acc > 0).all()
     check_invariants(pool, edges, na, nb, [0, 31, 39])
     kern = pool.sweep_info()[0]
-    assert kern in (3, 5, 7)   # sweep2_kernel<double>: staged counts (fewer warps when shared memory is short), cluster form, or counts in L2
+    assert kern in (3, 5)   # sweep2_kernel<double>: staged counts (fewer warps when shared memory is short) or counts in L2
     f1 = pool.entropy()
     d0 = np.array([pool.entropy_accum(c) for c in (0, 39)])
     pool.anneal("constant", 1.0, 0.0, 1 * (na + nb), 10 ** 9, seeds + np.uint64(7), max_inflight=1)

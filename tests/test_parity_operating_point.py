@@ -47,7 +47,7 @@ def _kat_check(pool, chain, kv, ks, kd, ka, lab, precision):
     return worst_ds, worst_la, checked
 
 
-@pytest.mark.parametrize("counts", ["staged", "l2", "cluster"])
+@pytest.mark.parametrize("counts", ["staged", "l2", "staged_k32"])
 @pytest.mark.parametrize("precision", ["fp64", "fp32"])
 @pytest.mark.parametrize("name", KAT_GOLDENS)
 def test_parallel_kernel_transition_kats(host, name, precision, counts):
@@ -59,8 +59,12 @@ def test_parallel_kernel_transition_kats(host, name, precision, counts):
     pool.set_precision(precision)
     if counts == "l2":
         pool.set_option("kernel", 5)      # sweep2_kernel<.., STAGED = false>: the large-K form of the same kernel
-    if counts == "cluster":
-        pool.set_option("kernel", 7)      # sweep2_kernel<.., CLUSTER>: m_rs distributed over a thread-block cluster
+    if counts == "staged_k32":
+        # count strides of 32 + 32 (the chains keep their K; the extra blocks stay empty): the Ka = Kb = 32 compile-time
+        # specialisations sweep2_kernel<R, 32, TYPE> that the benchmark runs
+        pool.set_option("reserve_ka", 32)
+        pool.set_option("reserve_kb", 32)
+        pool.set_labels(np.tile(g["init_labels"], (C, 1)))
     w1, w2, n = _kat_check(pool, 33, g["kat_v"], g["kat_s"], g["kat_dS"], g["kat_accu"], g["init_labels"], precision)
     print("%s %s: %d known answers, worst rel dS error %.2e, worst |log accu error| %.2e" % (name, precision, n, w1, w2))
     assert n > 0
