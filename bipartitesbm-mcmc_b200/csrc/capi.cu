@@ -607,7 +607,7 @@ const size_t kSmemMax = 227 * 1024;
 int plan_kernel(const bisbm_handle* h, uint32_t* wpc_out) {
     const uint32_t hb = h->max_degree <= 255u ? 1 : (h->max_degree <= 65535u ? 2 : 4);
     *wpc_out = 32;
-    if (h->opt_kernel == KERN_L2 && !h->opt_vary_k) return KERN_L2;
+    if (h->opt_kernel == KERN_L2) return KERN_L2;
     const bool k8 = h->KA <= 256 && h->KB <= 256;
     if (hb == 1 && k8) {
         const uint32_t rs = h->precision == BISBM_PRECISION_FP32 ? 4u : 8u;

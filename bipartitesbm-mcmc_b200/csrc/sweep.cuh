@@ -12,7 +12,8 @@
 // (ld.global.cg) and global atomics per move, so every CTA sees every committed move at once
 // and the "would empty block r" veto of apply_mcmc_moves is an exact atomic
 // decrement-and-check.  It serves the graphs and K the staged kernel of sweep2.cuh cannot
-// take (hubs of degree > 255, K > 256 per type).
+// take (hubs of degree > 255, K > 256 per type).  In estimate mode (SweepParams::vary_k) the veto
+// is off and dS carries the change of the K-dependent prior terms, as in sweep2_kernel.
 //
 // Per move this is the arithmetic of the reference's step():
 //   proposal   single_vertex_change      reference src/blockmodel.cc:613-637
@@ -319,6 +320,18 @@ struct Cnt {
     __device__ __forceinline__ void add(uint32_t idx32, int v) const { atomicAdd(p + idx32, v); }
 };
 
+// estimate mode: change of the K-dependent terms of entropy() (src/blockmodel.cc:780-782: lbinom(Ka Kb + E - 1, E) +
+// lbinom(na - 1, Ka - 1) + lbinom(nb - 1, Kb - 1)) when the number of occupied blocks of the moving type goes k -> k + dk.
+// Out of line: a move changes the occupied count rarely.  Used by sweep_kernel and sweep2_kernel.
+__device__ __noinline__ static double prior_k_delta(double E, double n_own, double k_own, double k_opp, int dk) {
+    auto lbin = [](double N, double k) -> double {
+        if (N == 0.0 || k == 0.0 || k > N) return 0.0;
+        return lgamma(N + 1.0) - lgamma(k + 1.0) - lgamma(N - k + 1.0);
+    };
+    const double k2 = k_own + (double)dk;
+    return (lbin(k2 * k_opp + E - 1.0, E) + lbin(n_own - 1.0, k2 - 1.0)) - (lbin(k_own * k_opp + E - 1.0, E) + lbin(n_own - 1.0, k_own - 1.0));
+}
+
 template <typename HistT, int NT>
 __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -384,6 +397,14 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
     const bool const_T = (P.schedule == 3) || P.beta_chain;
     double T_const = (double)P.p0, beta_const = 1.0 / (double)P.p0;
     if (P.beta_chain) { beta_const = P.beta_chain[cc]; T_const = 1.0 / beta_const; }   // (a ladder never holds T = 0)
+
+    // estimate mode: occupied blocks of this lane's chain, per type (own type tracked through this warp's own moves)
+    int occ_own = 0, occ_opp = 0;
+    if (P.vary_k) {
+        const int32_t* const gNRopp = P.s.nr + (size_t)group * KK * GROUP + (size_t)opp_off * 32;
+        for (uint32_t b = 0; b < kown_max; ++b) occ_own += (ldc(&gNR[b * 32 + lane]) > 0) ? 1 : 0;
+        for (uint32_t b = 0; b < kopp_max; ++b) occ_opp += (ldc(&gNRopp[b * 32 + lane]) > 0) ? 1 : 0;
+    }
 
     unsigned long long n_acc = 0;
     double ds_sum = 0.0;
@@ -535,12 +556,19 @@ __global__ void __launch_bounds__(NT, 1) sweep_kernel(SweepParams P) {
                 dS += block_degree_delta(e_r, e_s, (int)d);
                 dS += logq_delta(P.tb, gLQ[r * 32 + lane], e_r, n_r, -(int)d, -1);
                 dS += logq_delta(P.tb, gLQ[s * 32 + lane], e_s, n_s, (int)d, 1);
+                // estimate mode: the move empties r and / or opens s, the K-dependent prior terms change with the occupied count
+                const int dk = ((n_s == 0) ? 1 : 0) - ((n_r == 1) ? 1 : 0);
+                if (P.vary_k && eval && dk != 0)
+                    dS += prior_k_delta((double)G.n_edges, (double)nv, (double)occ_own, (double)occ_opp, dk);
                 // ---- accept (step) ----
                 const double beta = const_T ? beta_const : 1.0 / T;
                 const double a = ((d == 0) ? 0.0 : log(A.a1 / A.a0)) - dS * beta;
                 const bool go_hot = (a > 0.0) || (((double)ra.w + 0.5) * (1.0 / 4294967296.0) < exp(a));
                 go = eval && ((T == 0.0) ? (dS < 0.0) : go_hot);
-                if (go) {
+                if (go && P.vary_k) {
+                    atomicSub(&gNR[r * 32 + lane], 1);   // estimate mode: a block may empty
+                    occ_own += dk;
+                } else if (go) {
                     // the exact "would empty block r" veto of apply_mcmc_moves.  n_r was read from L2 a moment
                     // ago; fewer than SAFE_NR moves of this chain can be in flight, so a block that large
                     // cannot empty and a fire-and-forget reduction is enough (no round trip on the critical path)

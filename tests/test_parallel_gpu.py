@@ -581,10 +581,24 @@ def test_estimate_mode_variable_k(host, precision):
     entropy() (which counts occupied blocks in this mode) although blocks come and go; counts always equal a rebuild
     from the labels."""
     g = load_golden("c1_seed1")
-    na, nb, edges = g["na"], g["nb"], g["edges"]
+    _estimate_mode_check(host, g["edges"], g["na"], g["nb"], g["labels0"], precision, 2 if precision == "fp32" else 3)
+
+
+def test_estimate_mode_hub_round1(host):
+    """The same on a graph with a hub (256 parallel edges between the first a-node and the first b-node): degree > 255
+    takes the round-1 kernel (0), which must run estimate mode as well -- blocks empty at T = 2 and, for strictly
+    sequential chains, the accumulated dS equals the change of entropy() counted with the occupied blocks."""
+    g = load_golden("c1_seed1")
+    na, nb = g["na"], g["nb"]
+    hub = np.tile(np.array([[0, na]], dtype=np.uint32), (256, 1))
+    edges = np.concatenate([np.asarray(g["edges"], dtype=np.uint32).reshape(-1, 2), hub])
+    _estimate_mode_check(host, edges, na, nb, g["labels0"], "fp64", 0)
+
+
+def _estimate_mode_check(host, edges, na, nb, labels0, precision, kernel):
     graph = host.Graph(edges, na, nb)
     C = 64
-    pool = host.ChainPool(graph, np.tile(g["labels0"], (C, 1)), 5, 5, 1.0)
+    pool = host.ChainPool(graph, np.tile(labels0, (C, 1)), 5, 5, 1.0)
     pool.set_precision(precision)
     pool.set_option("vary_k", 1)
     seeds = np.arange(C, dtype=np.uint64) + 17
@@ -595,6 +609,7 @@ def test_estimate_mode_variable_k(host, precision):
     emptied = 0
     for rnd in range(6):
         acc, sw = pool.anneal("constant", 2.0, 0.0, 30 * (na + nb), 10 ** 9, seeds + np.uint64(1000 * rnd), max_inflight=1)
+        assert pool.sweep_info()[0] == kernel
         kk = pool.occupied_blocks()
         emptied += int((kk < 5).any())
         for c in (0, 31, 63):
