@@ -30,6 +30,7 @@
 #include "merge.cuh"
 #include "gltable.h"
 #include "sweep_aux.cuh"
+#include "align.cuh"
 #include "sweep2.cuh"
 #include "tempering.cuh"
 
@@ -122,6 +123,10 @@ struct bisbm_handle {
     // marginals
     uint32_t* d_hist = nullptr;
     uint32_t hist_width = 0;
+    // label alignment of the marginal samples (bisbm_marginals_align, align.cuh): a reference is set while al_segments > 0
+    uint32_t al_ka = 0, al_kb = 0, al_segments = 0;
+    uint32_t *d_al_order = nullptr, *d_al_seg = nullptr, *d_al_overlap = nullptr, *d_al_map = nullptr;
+    bool al_sampled = false;                   // d_al_map holds the permutations of an aligned sample
     // timing of the last parallel call
     double last_ms = 0.0;
     uint64_t last_launches = 0, last_moves = 0;
@@ -171,8 +176,15 @@ void free_ladder(bisbm_handle* h) {
     h->tp_round = 0;
 }
 
+void free_align(bisbm_handle* h) {
+    dfree(h->d_al_order); dfree(h->d_al_seg); dfree(h->d_al_overlap); dfree(h->d_al_map);
+    h->al_ka = h->al_kb = h->al_segments = 0;
+    h->al_sampled = false;
+}
+
 void free_chains(bisbm_handle* h) {
     free_ladder(h);
+    free_align(h);
     dfree(h->d_ka); dfree(h->d_kb); dfree(h->d_labels); dfree(h->d_labels_tmp);
     dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_nr_live); dfree(h->d_eta_snap); dfree(h->d_kat_out); dfree(h->d_lab8);
     dfree(h->d_seeds); dfree(h->d_active); dfree(h->d_accepted); dfree(h->d_u); dfree(h->d_sweeps);
@@ -1095,6 +1107,7 @@ static int alloc_chains(bisbm_handle* h, uint32_t n_chains, const uint32_t* ka, 
     if (!(eps > 0.0)) return fail(BISBM_ERR_ARG, "epsilon must be > 0");
     CU(cudaSetDevice(h->device));
     free_ladder(h);      // a new pool has no ladder
+    free_align(h);       // and no alignment reference
     uint32_t KA = 0, KB = 0;
     for (uint32_t c = 0; c < n_chains; ++c) {
         if (ka[c] == 0 || kb[c] == 0) return fail(BISBM_ERR_ARG, "chain %u: ka and kb must be >= 1", c);
@@ -1401,6 +1414,8 @@ MergeCtx mctx(bisbm_handle* h, uint32_t chain, const ReplaySlot& sl, const Merge
 // new block counts of one chain: host copy, device copy, counts rebuilt from the labels (init_bisbm)
 int set_chain_k(bisbm_handle* h, uint32_t chain, uint32_t ka, uint32_t kb) {
     if (ka > h->KA || kb > h->KB) return fail(BISBM_ERR_STATE, "chain %u: (%u, %u) blocks exceed the pool's strides (%u, %u)", chain, ka, kb, h->KA, h->KB);
+    // an alignment reference and its maps are for the (ka, kb) the pool had: a chain with other block counts drops it
+    if (ka != h->h_ka[chain] || kb != h->h_kb[chain]) free_align(h);
     h->h_ka[chain] = ka; h->h_kb[chain] = kb;
     CU(cudaMemcpyAsync(h->d_ka + chain, &h->h_ka[chain], sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(h->d_kb + chain, &h->h_kb[chain], sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
@@ -1742,17 +1757,41 @@ int bisbm_anneal(bisbm_handle* h, int schedule, float p0, float p1, uint64_t dur
 }
 
 // one sample of every chain's current labels into the histogram, straight from the array the sweep kernel keeps
-// current: the u8 shadow (sweep2 kernels) or the i32 labels.  rung (device, may be null): only the chains at rung 0
+// current: the u8 shadow (sweep2 kernels) or the i32 labels.  rung (device, may be null): only the chains at rung 0.
+// With an alignment reference set, every chain's permutations are computed first (align.cuh) and the histogram counts
+// the permuted labels; all of it is queued on the stream, nothing waits for the device.
 static int launch_marginal(bisbm_handle* h, const uint32_t* rung = nullptr) {
     const uint64_t mw = (uint64_t)h->n * (h->C / 32);
     const unsigned mgrid = (unsigned)((mw * 32 + 255) / 256);
+    const uint32_t* map = nullptr;
+    if (h->al_segments) {
+        const uint32_t ka = h->al_ka, kb = h->al_kb;     // == hist_width (bisbm_marginals_align; K changes drop the reference)
+        CU(cudaMemsetAsync(h->d_al_overlap, 0, (size_t)h->C * ((size_t)ka * ka + (size_t)kb * kb) * sizeof(uint32_t), h->stream));
+        const dim3 ogrid(h->al_segments, h->C / 32);
+        const size_t osmem = (size_t)std::max(ka, kb) * 32 * sizeof(uint32_t);
+        const uint32_t *seg_begin = h->d_al_seg, *seg_ref = h->d_al_seg + h->al_segments + 1;
+        if (h->lab32_stale)
+            align_overlap_kernel<uint8_t><<<ogrid, 256, osmem, h->stream>>>(h->d_lab8, h->C, h->n_chains, ka, kb, h->d_al_order,
+                                                                          seg_begin, seg_ref, h->d_al_overlap);
+        else
+            align_overlap_kernel<int32_t><<<ogrid, 256, osmem, h->stream>>>(h->d_labels, h->C, h->n_chains, ka, kb, h->d_al_order,
+                                                                          seg_begin, seg_ref, h->d_al_overlap);
+        align_assign_kernel<<<dim3(h->n_chains, 2), 32, align_assign_smem(std::max(ka, kb)), h->stream>>>(h->d_al_overlap, h->C, ka, kb,
+                                                                                                     h->d_al_map);
+        CU(cudaGetLastError());
+        map = h->d_al_map;
+        h->al_sampled = true;
+    }
     if (h->lab32_stale)
-        marginal_kernel<uint8_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_lab8, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width, rung);
+        marginal_kernel<uint8_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_lab8, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width, rung, map);
     else
-        marginal_kernel<int32_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_labels, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width, rung);
+        marginal_kernel<int32_t><<<mgrid, 256, 0, h->stream>>>(gview(h), h->d_labels, h->C, h->d_ka, h->n_chains, h->d_hist, h->hist_width, rung, map);
     CU(cudaGetLastError());
     return BISBM_OK;
 }
+
+// kernel launches of one marginal sample (the alignment adds the overlap and assignment kernels)
+static uint64_t marginal_launches(const bisbm_handle* h) { return h->al_segments ? 3 : 1; }
 
 int bisbm_marginal_sample(bisbm_handle* h) {
     int rc = need_chains(h);
@@ -1773,6 +1812,72 @@ int bisbm_marginals_clear(bisbm_handle* h) {
     }
     CU(cudaMemsetAsync(h->d_hist, 0, (size_t)h->n * width * sizeof(uint32_t), h->stream));
     CU(cudaStreamSynchronize(h->stream));
+    return BISBM_OK;
+}
+
+int bisbm_marginals_align(bisbm_handle* h, const uint32_t* ref) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!ref) { free_align(h); return BISBM_OK; }
+    const uint32_t ka = h->h_ka[0], kb = h->h_kb[0], n = h->n, na = h->na, C = h->C;
+    for (uint32_t c = 1; c < h->n_chains; ++c)
+        if (h->h_ka[c] != ka || h->h_kb[c] != kb)
+            return fail(BISBM_ERR_ARG, "alignment needs one (ka, kb) for the pool: chain %u has (%u, %u), chain 0 (%u, %u)", c,
+                        h->h_ka[c], h->h_kb[c], ka, kb);
+    for (uint32_t v = 0; v < n; ++v) {
+        const uint32_t g = ref[v];
+        if (v < na ? g >= ka : (g < ka || g >= ka + kb))
+            return fail(BISBM_ERR_ARG, "reference label %u of node %u is not a type-%c block (ka=%u kb=%u)", g, v, v < na ? 'a' : 'b', ka, kb);
+    }
+    const size_t osmem = (size_t)std::max(ka, kb) * 32 * sizeof(uint32_t), asmem = align_assign_smem(std::max(ka, kb));
+    int optin = 0;
+    CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    if (std::max(osmem, asmem) > (size_t)optin)
+        return fail(BISBM_ERR_ARG, "alignment of %u blocks per type needs %zu bytes of shared memory per block (device: %d)",
+                    std::max(ka, kb), std::max(osmem, asmem), optin);
+    // the histogram a sample adds to must be this pool's width (a pool of other K reusing the buffers keeps the old one)
+    if (h->d_hist && h->hist_width != ka + kb)
+        return fail(BISBM_ERR_STATE, "the histogram is %u blocks wide, the pool has %u: call bisbm_marginals_clear first", h->hist_width, ka + kb);
+    // raised to the device's limit once per handle, so that any later reference fits too
+    if (osmem > 48 * 1024) {
+        rc = ensure_smem_attr(h, (const void*)align_overlap_kernel<uint8_t>, optin);
+        if (!rc) rc = ensure_smem_attr(h, (const void*)align_overlap_kernel<int32_t>, optin);
+        if (rc) return rc;
+    }
+    if (asmem > 48 * 1024 && (rc = ensure_smem_attr(h, (const void*)align_assign_kernel, optin))) return rc;
+    // node ids sorted by reference block (counting sort), cut into segments of at most ALIGN_SEG nodes of one block
+    std::vector<uint32_t> start(ka + kb + 1, 0), order(n);
+    for (uint32_t v = 0; v < n; ++v) ++start[ref[v] + 1];
+    for (uint32_t g = 0; g < ka + kb; ++g) start[g + 1] += start[g];
+    {
+        std::vector<uint32_t> pos(start.begin(), start.end() - 1);
+        for (uint32_t v = 0; v < n; ++v) order[pos[ref[v]]++] = v;
+    }
+    std::vector<uint32_t> seg_begin, seg_ref;
+    for (uint32_t g = 0; g < ka + kb; ++g)
+        for (uint32_t b = start[g]; b < start[g + 1]; b += ALIGN_SEG) { seg_begin.push_back(b); seg_ref.push_back(g); }
+    const uint32_t S = (uint32_t)seg_ref.size();
+    seg_begin.push_back(n);
+    seg_begin.insert(seg_begin.end(), seg_ref.begin(), seg_ref.end());    // device layout: begin[S + 1], then ref[S]
+    free_align(h);
+    CU(cudaMalloc(&h->d_al_order, (size_t)n * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_al_seg, seg_begin.size() * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_al_overlap, (size_t)C * ((size_t)ka * ka + (size_t)kb * kb) * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_al_map, (size_t)C * (ka + kb) * sizeof(uint32_t)));
+    CU(cudaMemcpyAsync(h->d_al_order, order.data(), (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_al_seg, seg_begin.data(), seg_begin.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    h->al_ka = ka; h->al_kb = kb; h->al_segments = S;
+    return BISBM_OK;
+}
+
+int bisbm_marginals_alignment(bisbm_handle* h, uint32_t* map) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!map) return fail(BISBM_ERR_ARG, "null argument");
+    if (!h->al_sampled) return fail(BISBM_ERR_STATE, "no aligned marginal sample since the reference was set");
+    CU(cudaStreamSynchronize(h->stream));
+    CU(cudaMemcpy(map, h->d_al_map, (size_t)h->n_chains * (h->al_ka + h->al_kb) * sizeof(uint32_t), cudaMemcpyDeviceToHost));
     return BISBM_OK;
 }
 
@@ -1803,7 +1908,7 @@ int bisbm_marginalize(bisbm_handle* h, uint64_t burn_in, uint64_t sweeps, uint64
             rc = launch_marginal(h);
             if (rc) return rc;
             h->last_marginal_launches += 1;
-            h->last_launches += 1;
+            h->last_launches += marginal_launches(h);
         }
     }
     CU(cudaEventRecord(h->ev1, h->stream));
@@ -1914,7 +2019,7 @@ int bisbm_tempering_run(bisbm_handle* h, uint64_t sweeps, uint64_t swap_every, u
             rc = launch_marginal(h, h->d_tp_rung_of);
             if (rc) return rc;
             h->last_marginal_launches += 1;
-            h->last_launches += 1;
+            h->last_launches += marginal_launches(h);
         }
     }
     if (unattributed) {      // the sweeps after the last round: credited to the rungs the chains hold now

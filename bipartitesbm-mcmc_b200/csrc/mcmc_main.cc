@@ -11,7 +11,9 @@
 //   --marginalize          README "marginalization": -b burn-in sweeps, -t sampling sweeps, one sample
 //                          every -f sweeps over --chains chains; prints the arg-max label per node.  With
 //                          --tempering T0 T1 .. the chains form ladders of those temperatures (parallel tempering,
-//                          swaps every --swap_every sweeps) and only the chains at T0 are sampled
+//                          swaps every --swap_every sweeps) and only the chains at T0 are sampled.  With --align the
+//                          burn-in runs first, the lowest-entropy (cold) chain becomes the reference partition and
+//                          every sample is relabelled to agree with it before it is counted (bisbm_marginals_align)
 //   --estimate             README "estimation" output format for fixed (Ka, Kb): CSV lines
 //                          sweep,Ka,Kb,loglik,labels... of the last 1000 samples
 //   -g / --merge, -u / --nature, or initial labels whose block counts differ from -z: the agglomerative
@@ -59,6 +61,7 @@ const Spec kSpecs[] = {
     // README-only modes and the extensions of this build
     {"maximize", 0, 0}, {"estimate", 0, 0}, {"marginalize", 0, 0}, {"chains", 0, 1}, {"gen_seed", 0, 1},
     {"device", 0, 1}, {"max_inflight", 0, 1}, {"gpus", 0, 1}, {"tempering", 0, 2}, {"swap_every", 0, 1},
+    {"align", 0, 0},
 };
 
 const Spec* find_spec(const std::string& tok) {
@@ -141,7 +144,11 @@ void usage(const char* argv0) {
                  "                                        these temperatures (non-decreasing, T0 the cold one; --chains a\n"
                  "                                        multiple of their count); -b burn-in and -t sampling sweeps, the\n"
                  "                                        marginals sample only the chains at T0\n"
-                 "  --swap_every arg (=1)                 sweeps between two swap rounds of --tempering\n";
+                 "  --swap_every arg (=1)                 sweeps between two swap rounds of --tempering\n"
+                 "  --align                               --marginalize: after the burn-in, take the chain of lowest entropy\n"
+                 "                                        (at T0 under --tempering; over all GPUs with --gpus) as the reference\n"
+                 "                                        and relabel every sample's blocks, within each type, to agree with it\n"
+                 "                                        on as many nodes as possible before counting it (label switching)\n";
 }
 
 // the ladder of block counts between (start_a, start_b) and (end_a, end_b) (reference src/support/util.hh:99-146): the type
@@ -170,6 +177,19 @@ bool check(int rc) {
 void output_vec(const std::vector<uint32_t>& v, std::ostream& os) {  // reference src/output_functions.hh:20-28
     for (uint32_t x : v) os << x << " ";
     os << "\n";
+}
+
+// --align's reference: the chain of lowest entropy() in the pool (under a ladder, among the chains at rung 0)
+int lowest_entropy_chain(bisbm_handle* h, size_t n_chains, bool cold_only, double* S, uint32_t* best) {
+    std::vector<double> ent(n_chains);
+    std::vector<uint32_t> rung(n_chains, 0);
+    int rc = bisbm_entropy_all(h, ent.data());
+    if (rc == BISBM_OK && cold_only) rc = bisbm_tempering_stats(h, rung.data(), nullptr, nullptr, nullptr, nullptr, nullptr);
+    if (rc != BISBM_OK) return rc;
+    bool found = false;
+    for (size_t c = 0; c < n_chains; ++c)
+        if (rung[c] == 0 && (!found || ent[c] < *S)) { *S = ent[c]; *best = (uint32_t)c; found = true; }
+    return BISBM_OK;
 }
 
 }  // namespace
@@ -256,6 +276,8 @@ int main(int argc, char const* argv[]) {
         if (!o.has("marginalize")) { std::cerr << "--tempering needs --marginalize\n"; return 1; }
         if (chains % temps.size()) { std::cerr << "--chains must be a multiple of the number of --tempering temperatures\n"; return 1; }
     }
+    const bool align = o.has("align");
+    if (align && !o.has("marginalize")) { std::cerr << "--align needs --marginalize\n"; return 1; }
     if (gpus > chains) gpus = chains;
     // stdout carries the label line and nothing else: whatever NCCL has to say (its version banner under NCCL_DEBUG)
     // goes to stderr unless the user chose a file
@@ -437,7 +459,9 @@ int main(int argc, char const* argv[]) {
                 std::vector<uint64_t> sw(nc);
                 if (marg) {
                     if (!ok(bisbm_marginals_clear(hs[g]))) return;
-                    if (!ok(bisbm_marginalize(hs[g], burn_in, sampling_steps, std::max<size_t>(sampling_frequency, 1), seeds.data(), (uint32_t)max_inflight))) return;
+                    // --align: the burn-in only; the reference is chosen over all devices before any sample
+                    if (!ok(bisbm_marginalize(hs[g], burn_in, align ? 0 : sampling_steps, std::max<size_t>(sampling_frequency, 1), seeds.data(), (uint32_t)max_inflight))) return;
+                    if (align && !ok(bisbm_entropy_all(hs[g], ent[g].data()))) return;
                 } else {
                     if (sched >= 0 && !ok(bisbm_anneal(hs[g], sched, kw[0], kw[1], sampling_steps, steps_await, seeds.data(), (uint32_t)max_inflight, acc[g].data(), sw.data()))) return;
                     if (!ok(bisbm_entropy_all(hs[g], ent[g].data()))) return;
@@ -447,6 +471,27 @@ int main(int argc, char const* argv[]) {
         for (size_t g = 0; g < gpus; ++g)
             if (!errs[g].empty()) { std::cerr << "libbisbm (device " << device + g << "): " << errs[g] << "\n"; return 1; }
         std::vector<uint32_t> out(N);
+        if (marg && align) {
+            // one reference for every device -- the lowest-entropy chain after the burn-in -- so that the all-reduced
+            // histogram is aligned to one partition; then the sampling sweeps
+            size_t bg = 0, bi = 0;
+            for (size_t g = 0; g < gpus; ++g)
+                for (size_t i = 0; i < ent[g].size(); ++i)
+                    if (ent[g][i] < ent[bg][bi]) { bg = g; bi = i; }
+            if (!check(bisbm_get_labels(hs[bg], (uint32_t)bi, out.data()))) return 1;
+            th.clear();
+            for (size_t g = 0; g < gpus; ++g)
+                th.emplace_back([&, g]() {
+                    auto ok = [&](int rc) { if (rc != BISBM_OK) { errs[g] = bisbm_last_error(); return false; } return true; };
+                    std::vector<uint64_t> seeds;
+                    for (size_t c = g; c < chains; c += gpus) seeds.push_back((uint64_t)seed * 0x9E3779B97F4A7C15ull + c);
+                    if (!ok(bisbm_marginals_align(hs[g], out.data()))) return;
+                    ok(bisbm_marginalize(hs[g], 0, sampling_steps, std::max<size_t>(sampling_frequency, 1), seeds.data(), (uint32_t)max_inflight));
+                });
+            for (auto& t : th) t.join();
+            for (size_t g = 0; g < gpus; ++g)
+                if (!errs[g].empty()) { std::cerr << "libbisbm (device " << device + g << "): " << errs[g] << "\n"; return 1; }
+        }
         if (marg) {
             // stdout carries the label line and nothing else: NCCL prints its version banner on stdout when the environment
             // sets NCCL_DEBUG (whatever NCCL_DEBUG_FILE says), so file descriptor 1 points at stderr while NCCL initialises
@@ -492,12 +537,27 @@ int main(int argc, char const* argv[]) {
             const size_t f = std::max<size_t>(sampling_frequency, 1);
             if (!check(bisbm_marginals_clear(h)) || !check(bisbm_tempering_set(h, (uint32_t)temps.size(), temps.data(), nullptr))) return 1;
             if (burn_in && !check(bisbm_tempering_run(h, burn_in, swap_every, 0, seeds.data(), (uint64_t)seed, (uint32_t)max_inflight, nullptr))) return 1;
+            if (align) {
+                double S = 0.0;
+                uint32_t best = 0;
+                if (!check(lowest_entropy_chain(h, chains, true, &S, &best)) || !check(bisbm_get_labels(h, best, out.data())) ||
+                    !check(bisbm_marginals_align(h, out.data()))) return 1;
+            }
             if (!check(bisbm_tempering_run(h, sampling_steps, swap_every, f, seeds.data(), (uint64_t)seed, (uint32_t)max_inflight, nullptr))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
             output_vec(out, std::cout);
         } else if (o.has("marginalize")) {
+            const size_t f = std::max<size_t>(sampling_frequency, 1);
             if (!check(bisbm_marginals_clear(h))) return 1;
-            if (!check(bisbm_marginalize(h, burn_in, sampling_steps, std::max<size_t>(sampling_frequency, 1), seeds.data(), (uint32_t)max_inflight))) return 1;
+            if (align) {
+                // burn-in, then the lowest-entropy chain is the reference every sample is aligned to
+                double S = 0.0;
+                uint32_t best = 0;
+                if (!check(bisbm_marginalize(h, burn_in, 0, f, seeds.data(), (uint32_t)max_inflight)) ||
+                    !check(lowest_entropy_chain(h, chains, false, &S, &best)) || !check(bisbm_get_labels(h, best, out.data())) ||
+                    !check(bisbm_marginals_align(h, out.data())) ||
+                    !check(bisbm_marginalize(h, 0, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
+            } else if (!check(bisbm_marginalize(h, burn_in, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
             output_vec(out, std::cout);
         } else {

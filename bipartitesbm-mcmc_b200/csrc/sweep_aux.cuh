@@ -326,9 +326,11 @@ __global__ void bookkeep_kernel(uint32_t n_chains, uint8_t* active, const double
 // chains' labels are ONE 128-byte line of the chain-minor i32 labels (or one 32-byte sector of the u8 shadow, LabT =
 // uint8_t); lanes holding the same label elect one of them, which adds their count -- a handful of atomics per warp
 // instead of 32.  rung (may be null = every chain): parallel tempering samples only the chains with rung[c] == 0.
+// map (may be null): label alignment (align.cuh), chain c's block g is counted as map[c * width + g].
 template <typename LabT>
 __global__ void marginal_kernel(GraphView G, const LabT* __restrict__ labels, uint32_t C, const uint32_t* __restrict__ ka,
-                                uint32_t n_chains, uint32_t* hist, uint32_t width, const uint32_t* __restrict__ rung) {
+                                uint32_t n_chains, uint32_t* hist, uint32_t width, const uint32_t* __restrict__ rung,
+                                const uint32_t* __restrict__ map) {
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t n_groups = C / 32;
     const uint64_t w = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -338,6 +340,7 @@ __global__ void marginal_kernel(GraphView G, const LabT* __restrict__ labels, ui
     if (c < n_chains && (!rung || rung[c] == 0)) {
         const uint32_t l = (uint32_t)labels[(size_t)v * C + c];
         g = v < G.na ? l : ka[c] + l;
+        if (map) g = map[(size_t)c * width + g];
     }
     const uint32_t peers = __match_any_sync(0xffffffffu, g);
     if (g != 0xffffffffu && lane == (uint32_t)(__ffs(peers) - 1)) atomicAdd(&hist[(size_t)v * width + g], (uint32_t)__popc(peers));

@@ -77,6 +77,8 @@ SIGNATURES = {
     "bisbm_marginalize": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, _u64p, C.c_uint32]),
     "bisbm_marginals_clear": (C.c_int, [C.c_void_p]),
     "bisbm_marginal_sample": (C.c_int, [C.c_void_p]),
+    "bisbm_marginals_align": (C.c_int, [C.c_void_p, _u32p]),
+    "bisbm_marginals_alignment": (C.c_int, [C.c_void_p, _u32p]),
     "bisbm_tempering_set": (C.c_int, [C.c_void_p, C.c_uint32, _dp, _u32p]),
     "bisbm_tempering_run": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, _u64p, C.c_uint64, C.c_uint32, _dp]),
     "bisbm_tempering_stats": (C.c_int, [C.c_void_p, _u32p, _u64p, _u64p, _u64p, _u64p, _u64p]),
@@ -429,6 +431,28 @@ class ChainPool:
 
     def marginal_sample(self):
         _check(self.L.bisbm_marginal_sample(self.g.h))
+
+    def marginals_align(self, labels):
+        """Align every later marginal sample to the partition `labels` [n] (global block ids, e.g. labels(c) or
+        marginal_argmax()): each chain's blocks are permuted within each type to agree with it on as many nodes as
+        possible before they are counted.  None clears the reference.  Needs one (ka, kb) for the whole pool."""
+        if labels is None:
+            _check(self.L.bisbm_marginals_align(self.g.h, None))
+            return
+        ref = np.ascontiguousarray(labels, dtype=np.uint32)
+        if ref.shape != (self.g.n,):
+            raise ValueError("the reference needs one label per node")
+        _check(self.L.bisbm_marginals_align(self.g.h, _p(ref, C.c_uint32)))
+
+    def marginals_alignment(self):
+        """[n_chains][ka + kb]: the global id each chain's block was counted as in the last aligned sample."""
+        # sized from the library, not from self.ka / self.kb: while maps exist, the histogram is exactly ka + kb wide (without
+        # a histogram there is no aligned sample, and the call fails without writing)
+        ptr, ne, w = C.c_void_p(), C.c_uint64(), C.c_uint32()
+        width = w.value if self.L.bisbm_marginals_device(self.g.h, C.byref(ptr), C.byref(ne), C.byref(w)) == 0 else 0
+        out = np.zeros((self.n_chains, width), dtype=np.uint32)
+        _check(self.L.bisbm_marginals_alignment(self.g.h, _p(out, C.c_uint32)))
+        return out
 
     def stream(self):
         """cudaStream_t (as int) the handle launches on."""

@@ -140,6 +140,29 @@ int bisbm_marginalize(bisbm_handle* h, uint64_t burn_in, uint64_t sweeps, uint64
 int bisbm_marginals_clear(bisbm_handle* h);
 /* adds ONE sample of every chain's current labels to the histogram (asynchronous on the handle's stream) */
 int bisbm_marginal_sample(bisbm_handle* h);
+/* Label alignment of the marginals (SURVEY H9; no counterpart in the reference).  Block ids mean nothing across chains: a
+ * chain started from a randomised partition, or one that exchanged two blocks on its way, calls a group "block 3" that
+ * its neighbours call "block 1", and the summed histogram mixes unrelated groups.  ref_labels[n]: a partition in the
+ * pool's global numbering (type-a ids < ka, type-b ids in [ka, ka + kb)), e.g. what bisbm_get_labels or
+ * bisbm_marginal_argmax return.  While a reference is set, every marginal sample (bisbm_marginal_sample,
+ * bisbm_marginalize, bisbm_tempering_run's rung-0 samples) first relabels each chain, within each type, by the
+ * permutation of its blocks that maximises the number of nodes whose block agrees with the reference.  Among maximal
+ * permutations it takes the one with the most fixed points, so a chain equal to the reference keeps its labels (and, in
+ * estimate mode, "vary_k", empty blocks stay where they are); any remaining tie is broken deterministically (the same
+ * overlaps always give the same permutation), so an aligned run is as reproducible as an unaligned one.  The chains themselves are not touched.  NULL clears the reference.
+ * The reference's node order is sorted and uploaded here; a sample queues its kernels on the handle's stream with no host
+ * synchronisation.  bisbm_set_chains* clears the reference, and so does a replay merge / split that changes a chain's
+ * (ka, kb); bisbm_randomize and bisbm_marginals_clear keep it, so a caller
+ * can marginalise, set the reference to the arg-max, clear and marginalise again.  Multi-GPU: set the same reference on
+ * every handle (or rank) before sampling, and the all-reduced histogram is aligned to that one partition.
+ * Errors: BISBM_ERR_ARG for a null handle, a pool whose chains differ in (ka, kb), a reference label outside its node's
+ * type range, or more blocks per type than the device's shared memory per block holds (about 1700); BISBM_ERR_STATE for a
+ * histogram of another width than ka + kb (left from a pool of other K: bisbm_marginals_clear first). */
+int bisbm_marginals_align(bisbm_handle* h, const uint32_t* ref_labels);
+/* the permutations the last aligned sample used: map[c * (ka + kb) + g] = the global id chain c's block g was counted as
+ * ([n_chains][ka + kb], computed for every chain, also those a tempering sample skips).  BISBM_ERR_STATE before any aligned
+ * sample under the current reference. */
+int bisbm_marginals_alignment(bisbm_handle* h, uint32_t* map);
 /* ---- parallel tempering (replica exchange; no counterpart in the reference) ----------------------------------------
  * Ladder: n_rungs = R temperatures temps[0..R-1], each finite and > 0, non-decreasing; rung 0 is the cold one.  n_chains
  * must be a multiple of R: chains l R .. l R + R - 1 form ladder l, and chain l R + i starts at rung i unless rung_of_chain
