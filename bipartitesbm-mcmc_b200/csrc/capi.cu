@@ -105,9 +105,13 @@ struct bisbm_handle {
     uint32_t *d_ka = nullptr, *d_kb = nullptr;
     int32_t *d_labels = nullptr, *d_labels_tmp = nullptr, *d_m = nullptr, *d_e = nullptr, *d_nr = nullptr,
             *d_eta = nullptr;
-    int32_t *d_m2 = nullptr, *d_e2 = nullptr, *d_nr2 = nullptr;  // "next" count buffers of the sliced shared-memory sweep
-    int32_t* d_nr_live = nullptr;              // exact n_r counters of the blocks that could empty within one sliced launch
-    int32_t* d_eta_snap = nullptr;             // eta as a sliced shared-memory launch reads it (taken before the launch)
+    // sliced staged sweep (launch_full_sweep): the base counts rotate through three buffer sets.  A launch reads d_m / d_e / d_nr,
+    // publishes into the *2 set, which is zero whenever no sliced launch is running, and zeroes the *3 set for the launch after it
+    int32_t *d_m2 = nullptr, *d_e2 = nullptr, *d_nr2 = nullptr, *d_m3 = nullptr, *d_e3 = nullptr, *d_nr3 = nullptr;
+    int32_t* d_nr_live[2] = {nullptr, nullptr};   // per-block decrements of n_r within one sliced launch (the exact veto);
+    uint64_t nr_live_pos = 0;                     // d_nr_live[nr_live_pos & 1], zero between launches, is the next launch's
+    // eta of the sliced launches: three buffers of C x KK x W, all zero between half sweeps (launch_full_sweep)
+    int32_t* d_eta_ring = nullptr;
     double* d_kat_out = nullptr;               // {dS, log accu_r} of bisbm_parallel_transition
     ncclComm_t comm = nullptr;                 // bisbm_nccl_init: communicator of the marginal-histogram all-reduce
     uint8_t* d_lab8 = nullptr;                 // u8 shadow of the labels for the shared-memory sweep
@@ -186,7 +190,8 @@ void free_chains(bisbm_handle* h) {
     free_ladder(h);
     free_align(h);
     dfree(h->d_ka); dfree(h->d_kb); dfree(h->d_labels); dfree(h->d_labels_tmp);
-    dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_nr_live); dfree(h->d_eta_snap); dfree(h->d_kat_out); dfree(h->d_lab8);
+    dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_m3); dfree(h->d_e3); dfree(h->d_nr3);
+    dfree(h->d_nr_live[0]); dfree(h->d_nr_live[1]); dfree(h->d_eta_ring); dfree(h->d_kat_out); dfree(h->d_lab8);
     dfree(h->d_seeds); dfree(h->d_active); dfree(h->d_accepted); dfree(h->d_u); dfree(h->d_sweeps);
     dfree(h->d_dS); dfree(h->d_entmin); dfree(h->d_ent_out); dfree(h->d_nactive); dfree(h->d_hist);
     for (auto& kv : h->replay) { dfree(kv.second.d_rs); dfree(kv.second.d_vlist); dfree(kv.second.d_kh); }
@@ -712,9 +717,22 @@ template <typename R, int KF, int TYPE, bool STAGED = true, int NT = 512>
 int launch_sweep2_t(bisbm_handle* h, const SweepParams& P, const LaunchPlan& lp, unsigned grid) {
     int rc = ensure_smem_attr(h, (const void*)sweep2_kernel<R, KF, TYPE, STAGED, NT>, (int)kSmemMax);
     if (rc) return rc;
-    sweep2_kernel<R, KF, TYPE, STAGED, NT><<<grid, lp.wpc * 32, lp.smem_bytes, h->stream>>>(P);
+    cudaError_t launched = cudaSuccess;
+    if (STAGED && !P.exclusive) {
+        // sliced: programmatic dependent launch, so the launch's blocks start (up to griddepcontrol.wait) while the one before
+        // finishes
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        at[0].val.programmaticStreamSerializationAllowed = 1;
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3(grid); cfg.blockDim = dim3(lp.wpc * 32); cfg.dynamicSmemBytes = lp.smem_bytes; cfg.stream = h->stream;
+        cfg.attrs = at; cfg.numAttrs = 1;
+        launched = cudaLaunchKernelEx(&cfg, sweep2_kernel<R, KF, TYPE, STAGED, NT>, P);
+    } else {
+        sweep2_kernel<R, KF, TYPE, STAGED, NT><<<grid, lp.wpc * 32, lp.smem_bytes, h->stream>>>(P);
+    }
     {
-        const cudaError_t e = cudaGetLastError();
+        const cudaError_t le = cudaGetLastError(), e = launched != cudaSuccess ? launched : le;
         if (e != cudaSuccess)
             return fail(BISBM_ERR_CUDA, "sweep2_kernel launch failed: %s (kernel %d, grid %u, %u warps, %zu bytes of shared memory)",
                         cudaGetErrorString(e), lp.kernel, grid, lp.wpc, lp.smem_bytes);
@@ -757,8 +775,8 @@ SweepParams base_params(bisbm_handle* h, uint32_t type) {
     SweepParams P;
     memset(&P, 0, sizeof P);
     P.g = gview(h); P.s = sview(h); P.tb = tview(h, false);
-    P.lab8 = h->d_lab8; P.m_next = h->d_m2; P.e_next = h->d_e2; P.nr_next = h->d_nr2; P.nr_live = h->d_nr_live;
-    P.eta_read = h->d_eta;
+    P.lab8 = h->d_lab8;
+    P.eta_read = h->d_eta; P.eta_commit = h->d_eta;
     P.seeds = h->d_seeds; P.active = h->d_active; P.accepted = h->d_accepted; P.dS_accum = h->d_dS;
     P.lq = h->d_lq;
     P.n_chains = h->n_chains; P.type = type; P.n_groups = h->C / 32;
@@ -794,7 +812,6 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
         const uint32_t tot = h->n_chains * kmax;
         logq_refresh_kernel<<<(tot * 16 + 127) / 128, 128, 0, h->stream>>>(sview(h), tview(h, false), h->d_lq, h->n_chains, type);
         h->last_launches += 1;
-        const uint32_t n_m = h->C * h->KA * h->KB, n_e = h->C * (h->KA + h->KB);
         const bool sliced = lp.smem && lp.ctas_per_group > 1;   // (only the staged sweep2 kernels are sliced)
         h->last_wpc = lp.wpc; h->last_cpg = lp.ctas_per_group; h->last_slice = lp.slice;
         h->last_kernel = kernel;
@@ -805,6 +822,9 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
         if (sliced && h->opt_spare_sms && max_inflight == 0 && (uint32_t)h->sm_count > G * lp.ctas_per_group)   // (an explicit in-flight bound is kept to the letter)
             extras = std::min<uint32_t>((uint32_t)h->sm_count - G * lp.ctas_per_group, G - 1);
         const uint32_t per_cta = lp.slice / std::max<uint32_t>(1, lp.ctas_per_group);
+        const size_t n_eta = (size_t)h->C * (h->KA + h->KB) * h->W;
+        int32_t* const eta_S[3] = {h->d_eta_ring, h->d_eta_ring + n_eta, h->d_eta_ring + 2 * n_eta};
+        int32_t *last_read = nullptr, *last_commit = nullptr;
         for (uint32_t l = 0;; ++l) {
             // the group that has been handed the fewest extra slots (the last one) decides when the half sweep is over
             const uint64_t pos = extras ? ((uint64_t)l * lp.ctas_per_group + ((uint64_t)l * extras) / G) * per_cta : (uint64_t)l * lp.slice;
@@ -814,19 +834,22 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
                 logq_refresh_kernel<<<(tot * 16 + 127) / 128, 128, 0, h->stream>>>(sview(h), tview(h, false), h->d_lq, h->n_chains, type, 1u);
                 h->last_launches += 1;
             }
-            if (sliced) {
-                // next := -(publishers - 1) * base: every CTA adds its whole staged copy (sweep2.cuh)
-                // and the moving type's eta into the snapshot the launch reads (its commits go to d_eta)
-                const uint32_t nmax = std::max(std::max(n_m, n_e), G * kmax * h->W * 32u);
-                sweep2_preinit_kernel<<<(nmax + 255) / 256, 256, 0, h->stream>>>(h->d_m, h->d_e, h->d_nr, h->d_m2, h->d_e2, h->d_nr2,
-                                                                                 h->d_nr_live, n_m, n_e, h->KA, h->KB, type, lp.ctas_per_group - 1,
-                                                                                 G, extras, l, h->d_eta, h->d_eta_snap, h->W);
-                h->last_launches += 1;
-            }
             SweepParams P = base_params(h, type);
-            // sliced staged launches read eta as it was before the launch: what other CTAs commit meanwhile is not seen,
-            // so the result does not depend on their timing
-            if (sliced) P.eta_read = h->d_eta_snap;
+            if (sliced) {
+                // launch l reads eta as it was at its start, S_l, which no launch writes meanwhile: what other CTAs commit is not
+                // seen, so the result does not depend on their timing.  It commits into S_{l+1} (zero at its start) and adds S_l
+                // there too, so S_{l+1} ends as eta at the start of launch l + 1; it zeroes S_{l+2}.  S_0 is eta itself, then
+                // the three ring buffers take turns.
+                P.eta_read = (l == 0) ? h->d_eta : eta_S[(l - 1) % 3];
+                P.eta_commit = eta_S[l % 3];
+                P.eta_zero = eta_S[(l + 1) % 3];
+                // counts: read d_m (base), publish into d_m2 (zero), zero d_m3 (the previous base)
+                P.m_next = h->d_m2; P.e_next = h->d_e2; P.nr_next = h->d_nr2;
+                P.m_zero = h->d_m3; P.e_zero = h->d_e3; P.nr_zero = h->d_nr3;
+                P.nr_live = h->d_nr_live[h->nr_live_pos & 1]; P.nr_live_zero = h->d_nr_live[(h->nr_live_pos + 1) & 1];
+                last_read = (l == 0) ? nullptr : eta_S[(l - 1) % 3];
+                last_commit = P.eta_commit;
+            }
             P.ctas_per_group = lp.ctas_per_group; P.warps_used = lp.warps_used;
             P.pos_begin = (uint32_t)pos; P.pos_end = (uint32_t)std::min<uint64_t>(nv, pos + lp.slice);
             P.exclusive = sliced ? 0 : 1;
@@ -848,8 +871,18 @@ int launch_full_sweep(bisbm_handle* h, int schedule, float p0, float p1, uint64_
             h->last_launches += 1;
             h->last_sweep_launches += 1;
             if (sliced) {
-                std::swap(h->d_m, h->d_m2); std::swap(h->d_e, h->d_e2); std::swap(h->d_nr, h->d_nr2);
+                int32_t* t = h->d_m; h->d_m = h->d_m2; h->d_m2 = h->d_m3; h->d_m3 = t;
+                t = h->d_e; h->d_e = h->d_e2; h->d_e2 = h->d_e3; h->d_e3 = t;
+                t = h->d_nr; h->d_nr = h->d_nr2; h->d_nr2 = h->d_nr3; h->d_nr3 = t;
+                h->nr_live_pos += 1;
             }
+        }
+        if (last_commit) {
+            // the live eta (read by the other kernels and the host) := the buffer the last launch committed into
+            const uint32_t kown = type ? h->KB : h->KA, tot_eta = G * kown * h->W * 32u;
+            eta_publish_kernel<<<(tot_eta + 255) / 256, 256, 0, h->stream>>>(h->d_eta, last_commit, last_read, G, h->KA + h->KB,
+                                                                            type ? h->KA : 0u, kown, h->W);
+            h->last_launches += 1;
         }
     }
     h->sweep_epoch++;
@@ -1130,15 +1163,18 @@ static int alloc_chains(bisbm_handle* h, uint32_t n_chains, const uint32_t* ka, 
         CU(cudaMalloc(&h->d_labels_tmp, (size_t)n * C * sizeof(int32_t)));
         CU(cudaMalloc(&h->d_m, (size_t)C * KA * KB * sizeof(int32_t)));
         CU(cudaMalloc(&h->d_e, (size_t)C * KK * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_m2, (size_t)C * KA * KB * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_e2, (size_t)C * KK * sizeof(int32_t)));
         CU(cudaMalloc(&h->d_lab8, (size_t)n * C));
         CU(cudaMalloc(&h->d_nr, (size_t)C * KK * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_nr2, (size_t)C * KK * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_nr_live, (size_t)C * KK * sizeof(int32_t)));
+        for (int32_t** p : {&h->d_m2, &h->d_m3}) CU(cudaMalloc(p, (size_t)C * KA * KB * sizeof(int32_t)));
+        for (int32_t** p : {&h->d_e2, &h->d_e3, &h->d_nr2, &h->d_nr3, &h->d_nr_live[0], &h->d_nr_live[1]})
+            CU(cudaMalloc(p, (size_t)C * KK * sizeof(int32_t)));
         CU(cudaMalloc(&h->d_kat_out, 2 * sizeof(double)));
         CU(cudaMalloc(&h->d_eta, (size_t)C * KK * h->W * sizeof(int32_t)));
-        CU(cudaMalloc(&h->d_eta_snap, (size_t)C * KK * h->W * sizeof(int32_t)));
+        CU(cudaMalloc(&h->d_eta_ring, 3 * (size_t)C * KK * h->W * sizeof(int32_t)));
+        // what must be zero when no sliced launch is running
+        CU(cudaMemsetAsync(h->d_m2, 0, (size_t)C * KA * KB * sizeof(int32_t), h->stream));
+        for (int32_t* p : {h->d_e2, h->d_nr2, h->d_nr_live[0], h->d_nr_live[1]}) CU(cudaMemsetAsync(p, 0, (size_t)C * KK * sizeof(int32_t), h->stream));
+        CU(cudaMemsetAsync(h->d_eta_ring, 0, 3 * (size_t)C * KK * h->W * sizeof(int32_t), h->stream));
         CU(cudaMalloc(&h->d_lq, (size_t)C * KK * sizeof(LogqExp)));
         CU(cudaMalloc(&h->d_seeds, C * sizeof(uint64_t)));
         CU(cudaMalloc(&h->d_active, C));
@@ -2314,12 +2350,12 @@ int bisbm_set_option(bisbm_handle* h, const char* name, int64_t value) {
 }
 
 #ifdef BISBM_ROUND_CLOCKS
-// instrumented builds only (scripts/round_clocks.py): copy the 8 counters of sweep2.cuh's g_round_clocks to `out`, then zero them
+// instrumented builds only (scripts/round_clocks.py): copy the 11 counters of sweep2.cuh's g_round_clocks to `out`, then zero them
 int bisbm_round_clocks(unsigned long long* out) {
     if (!out) return fail(BISBM_ERR_ARG, "null argument");
     CU(cudaDeviceSynchronize());
-    CU(cudaMemcpyFromSymbol(out, g_round_clocks, sizeof(unsigned long long) * 8));
-    const unsigned long long zero[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+    CU(cudaMemcpyFromSymbol(out, g_round_clocks, sizeof(unsigned long long) * 11));
+    const unsigned long long zero[11] = {};
     CU(cudaMemcpyToSymbol(g_round_clocks, zero, sizeof zero));
     return BISBM_OK;
 }

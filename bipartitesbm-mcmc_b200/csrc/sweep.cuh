@@ -71,8 +71,18 @@ struct SweepParams {
     float p0, p1;
     // sweep2_kernel (sweep2.cuh)
     int32_t* nr_next;                // sliced launches: where the n_r view is added
-    int32_t* nr_live;                // exact n_r counters for blocks small enough to empty within a launch
-    const int32_t* eta_read;         // sweep2: where eta is READ (a snapshot taken before a sliced launch; commits go to s.eta)
+    int32_t* nr_live;                // sliced launches: decrements of n_r within the launch (zero at its start), the exact "would
+                                     // empty" counters of blocks small enough to empty within a launch
+    // sweep2: where eta is READ and where its commits go.  Sliced staged launches read eta as it was at their start (a buffer no
+    // launch writes meanwhile) and commit into the next launch's buffer; otherwise both are s.eta
+    const int32_t* eta_read;
+    int32_t* eta_commit;
+    // sliced staged launches: after griddepcontrol.wait the CTAs of a group share the buffer work for the launches around this one
+    // (launch_full_sweep): eta_commit += eta_read (moving type; with the launch's commits it becomes the next launch's eta_read),
+    // eta_zero := 0 (the moving type's eta_commit of the next launch), m_zero / e_zero / nr_zero := 0 (the base of the previous
+    // launch, where the next launch publishes), nr_live_zero := 0 (the nr_live of the next launch)
+    int32_t* eta_zero;
+    int32_t *m_zero, *e_zero, *nr_zero, *nr_live_zero;
     uint32_t group_offset;           // first chain group of this launch (0 except for single-group launches)
     uint32_t kat_mode;               // 1: evaluate ONE forced proposal (kat_v -> own-type block kat_s of chain kat_chain) and write
     uint32_t kat_chain, kat_v, kat_s;   //    {dS, log accu_r} to kat_out instead of accepting / committing (bisbm_parallel_transition)

@@ -25,8 +25,8 @@
 //     handed out to warps dynamically (no warp waits for the slowest one's static share);
 //   * staging is one thread issuing bulk-async copies (cp.async.bulk + mbarrier); publishing is one
 //     thread issuing bulk-async REDUCTIONS of the staged arrays themselves (cp.reduce.async.bulk
-//     .add.s32): the host pre-loads the next base with -(ctas_per_group - 1) * base, so the sum of all
-//     CTAs' staged copies is base + sum of their deltas -- no base re-read, no per-entry atomics.
+//     .add.s32): the CTAs of the group have added -(ctas_per_group - 1) * base into the next base at the start of the
+//     launch, so the sum of all CTAs' staged copies is base + sum of their deltas -- no base re-read, no per-entry atomics.
 //
 // Per move this is still the arithmetic of the reference's step():
 //   proposal   single_vertex_change      reference src/blockmodel.cc:613-637
@@ -402,8 +402,9 @@ __device__ __forceinline__ int gl_atom(uint64_t base, uint32_t off, int v) {
 #ifdef BISBM_ROUND_CLOCKS
 // instrumented builds (scripts/round_clocks.py): clock64 cycles of the staged sweep's warps, summed over all launches --
 // [0] proposal + pass, [1] dS / accept, [2] commit, [3] waiting at the barrier after the round's reads, [4] waiting at the
-// barrier after its commits, [5] vertices, [6] the longest proposal + pass of one vertex, [7] warp-rounds
-__device__ unsigned long long g_round_clocks[8];
+// barrier after its commits, [5] vertices, [6] the longest proposal + pass of one vertex, [7] warp-rounds; and per CTA (its
+// thread 0): [8] kernel start -> first round (the prologue), [9] last round -> publish done (the epilogue), [10] CTAs
+__device__ unsigned long long g_round_clocks[11];
 #define RC_DECL() long long rc[5] = {0, 0, 0, 0, 0}, rc_t = 0, rc_v0 = 0, rc_pass_max = 0; unsigned long long rc_n = 0, rc_rounds = 0
 #define RC_START() (rc_t = clock64())
 #define RC_MARK(ph) do { const long long t_ = clock64(); rc[ph] += t_ - rc_t; rc_t = t_; } while (0)
@@ -414,6 +415,11 @@ __device__ unsigned long long g_round_clocks[8];
         for (int k_ = 0; k_ < 5; ++k_) atomicAdd(&g_round_clocks[k_], (unsigned long long)rc[k_]);                    \
         atomicAdd(&g_round_clocks[5], rc_n); atomicMax(&g_round_clocks[6], (unsigned long long)rc_pass_max);          \
         atomicAdd(&g_round_clocks[7], rc_rounds); } } while (0)
+#define RC_CTA_DECL() long long rck_ = clock64()
+#define RC_CTA_MARK(slot) do { const long long t_ = clock64();                                                        \
+        if (threadIdx.x == 0) atomicAdd(&g_round_clocks[slot], (unsigned long long)(t_ - rck_)); rck_ = t_; } while (0)
+#define RC_CTA_RESET() (rck_ = clock64())
+#define RC_CTA_END() do { RC_CTA_MARK(9); if (threadIdx.x == 0) atomicAdd(&g_round_clocks[10], 1ull); } while (0)
 #else
 #define RC_DECL() do {} while (0)
 #define RC_START() ((void)0)
@@ -422,6 +428,10 @@ __device__ unsigned long long g_round_clocks[8];
 #define RC_PASS() ((void)0)
 #define RC_ROUND() ((void)0)
 #define RC_PUBLISH(on) ((void)0)
+#define RC_CTA_DECL() do {} while (0)
+#define RC_CTA_MARK(slot) ((void)0)
+#define RC_CTA_RESET() ((void)0)
+#define RC_CTA_END() ((void)0)
 #endif
 
 // the rare double-precision completions, out of line (arguments by value)
@@ -438,38 +448,53 @@ __device__ __noinline__ static double slow2_beta(int schedule, float p0, float p
     return (T == 0.0) ? -1.0 : 1.0 / T;
 }
 
-// next base of a sliced launch: every CTA of a group adds its whole staged copy (base + its deltas) into
-// `next`, so next starts at -(ctas_per_group - 1) * base for the arrays the CTAs publish (m_rs, and e_r / n_r of
-// the moving type) and at base for the frozen type's e_r / n_r.  nr_live := n_r (exact veto counters).  eta_snap := eta of the moving type.
-__global__ void sweep2_preinit_kernel(const int32_t* __restrict__ m, const int32_t* __restrict__ e, const int32_t* __restrict__ nr,
-                                      int32_t* __restrict__ m2, int32_t* __restrict__ e2, int32_t* __restrict__ nr2,
-                                      int32_t* __restrict__ nr_live, uint32_t n_m, uint32_t n_e, uint32_t KA, uint32_t KB,
-                                      uint32_t type, uint32_t mult,                     // mult: publishers per group - 1
-                                      uint32_t n_groups, uint32_t extras, uint32_t launch_idx,   // spare-SM CTAs: one more publisher in the groups that have one
-                                      const int32_t* __restrict__ eta, int32_t* __restrict__ eta_snap, uint32_t W) {
+// end of a sliced half sweep: eta of the moving type := S, the buffer its last launch committed into.  S and `prev` (the buffer
+// that launch read; null when it read eta itself) are zeroed, so all of the ring is zero between half sweeps (the third buffer
+// was zeroed by the last launch).
+__global__ void eta_publish_kernel(int32_t* __restrict__ eta, int32_t* __restrict__ S, int32_t* __restrict__ prev, uint32_t n_groups,
+                                   uint32_t KK, uint32_t own_off, uint32_t kown, uint32_t W) {
+    const uint32_t per = kown * W * 32u;
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    {   // eta_snap := eta for the moving type's blocks: the launch reads the snapshot and commits into eta
-        const uint32_t kown = type ? KB : KA, per = kown * W * 32u;
-        if (i < n_groups * per) {
-            const uint32_t g = i / per;
-            const size_t j = ((size_t)g * (KA + KB) + (type ? KA : 0u)) * W * 32u + (i - g * per);
-            eta_snap[j] = eta[j];
-        }
+    if (i >= n_groups * per) return;
+    const uint32_t g = i / per;
+    const size_t j = ((size_t)g * KK + own_off) * W * 32u + (i - g * per);
+    eta[j] = S[j];
+    S[j] = 0;
+    if (prev) prev[j] = 0;
+}
+
+// sliced staged launches, after griddepcontrol.wait: this CTA's 1/cpg share (cpg = the group's publishers) of its group's buffer
+// work for the launches around this one.  Every publisher adds its whole staged copy into the next base, so the next base gets
+// -(cpg - 1) x base where they publish (m_rs, and e_r / n_r of the moving type) and base elsewhere; it was zeroed by the launch
+// before.  Out of line: the rounds' register allocation does not see it.
+__device__ __noinline__ static void sliced_buffer_work(const SweepParams& P, uint32_t group, uint32_t cta_in_group, uint32_t cpg,
+                                                       uint32_t type, uint32_t KA, uint32_t KB, uint32_t kown, uint32_t W) {
+    const uint32_t KK = KA + KB;
+    const uint32_t t0 = cta_in_group * blockDim.x + threadIdx.x, stride = cpg * blockDim.x;
+    const uint32_t nM = KA * KB * 32u, nE = KK * 32u;
+    const size_t offM = (size_t)group * KA * KB * GROUP, offE = (size_t)group * KK * GROUP;
+    for (uint32_t i = t0; i < nM + 2u * nE; i += stride) {
+        const bool in_m = i < nM, in_e = !in_m && i < nM + nE;
+        const uint32_t j = in_m ? i : (in_e ? i - nM : i - nM - nE);
+        const size_t o = (in_m ? offM : offE) + j;
+        const int32_t* const src = in_m ? P.s.m : (in_e ? P.s.e : P.s.nr);
+        int32_t* const dst = in_m ? P.m_next : (in_e ? P.e_next : P.nr_next);
+        int32_t* const zero = in_m ? P.m_zero : (in_e ? P.e_zero : P.nr_zero);
+        const uint32_t slot = j >> 5;
+        const bool own = in_m || (type ? slot >= KA : slot < KA);
+        const uint32_t a = (uint32_t)__ldcg(src + o);
+        const int32_t add = (int32_t)(own ? 0u - (cpg - 1u) * a : a);
+        if (add != 0) atomicAdd(dst + o, add);
+        zero[o] = 0;
     }
-    auto extra_of = [&](uint32_t grp) -> uint32_t {
-        if (extras == 0u) return 0u;
-        const uint32_t slot0 = (uint32_t)(((uint64_t)launch_idx * extras) % n_groups);
-        return ((grp + n_groups - slot0) % n_groups < extras) ? 1u : 0u;
-    };
-    if (i < n_m) m2[i] = (int32_t)(0u - (mult + extra_of(i / (KA * KB * 32u))) * (uint32_t)m[i]);
-    if (i < n_e) {
-        const uint32_t slot = (i >> 5) % (KA + KB);
-        const bool own = type ? (slot >= KA) : (slot < KA);
-        const uint32_t ev = (uint32_t)e[i], nv = (uint32_t)nr[i];
-        const uint32_t mg = mult + extra_of(i / ((KA + KB) * 32u));
-        e2[i] = (int32_t)(own ? 0u - mg * ev : ev);
-        nr2[i] = (int32_t)(own ? 0u - mg * nv : nv);
-        nr_live[i] = (int32_t)nv;
+    for (uint32_t i = t0; i < nE; i += stride) P.nr_live_zero[offE + i] = 0;
+    // eta of the moving type: the buffer this launch commits into (zeroed by the launch before) also gets what it reads, so it
+    // ends as the next launch's eta; the launch after next commits into eta_zero
+    const size_t eta_off = (size_t)group * KK * W * GROUP + (size_t)(type ? KA : 0u) * W * 32;
+    for (uint32_t i = t0; i < kown * W * 32u; i += stride) {
+        const int32_t x = __ldcg(P.eta_read + eta_off + i);
+        if (x != 0) atomicAdd(P.eta_commit + eta_off + i, x);
+        P.eta_zero[eta_off + i] = 0;
     }
 }
 
@@ -487,6 +512,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     // sees do not depend on timing, so a call's result is a function of its inputs -- except where a block of a chain is
     // small enough to empty within the launch: the "would empty block r" veto below is an atomic decrement-and-check whose
     // order among the moves out of r (other warps' in the commit phase, other CTAs' on nr_live) is not fixed
+    RC_CTA_DECL();
     extern __shared__ __align__(128) unsigned char s2_smem[];
     unsigned char* const smem_raw = s2_smem;
     constexpr uint32_t FULL = 0xffffffffu;
@@ -513,8 +539,9 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     int32_t* const gE = P.s.e + (size_t)group * KK * GROUP;
     int32_t* const gNR = P.s.nr + (size_t)group * KK * GROUP;
     int32_t* const gLIVE = P.nr_live + (size_t)group * KK * GROUP + (size_t)own_off * 32;
-    int32_t* const gETA = P.s.eta + (size_t)group * KK * W * GROUP + (size_t)own_off * W * 32;
-    const int32_t* const gETAr = P.eta_read + (size_t)group * KK * W * GROUP + (size_t)own_off * W * 32;
+    const size_t eta_off = (size_t)group * KK * W * GROUP + (size_t)own_off * W * 32;
+    int32_t* const gETA = P.eta_commit + eta_off;
+    const int32_t* const gETAr = P.eta_read + eta_off;
     const LogqExp* const gLQ = P.lq + ((size_t)group * KK + own_off) * GROUP;
 
     const uint32_t c = group * 32 + lane;
@@ -538,26 +565,14 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     const uint32_t mbar = sbase + L.oCtl;
     const uint32_t hist_words = (kopp_max + 3u) / 4u;
 
-    // ---- stage the group's counts: one thread, bulk-async copies ----
-    if (STAGED) {
-        if (threadIdx.x == 0) {
-            mbar_init(mbar, 1);
-            asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            const uint32_t bM = KA * KB * 128u, bO = kown_max * 128u, bP = kopp_max * 128u;
-            mbar_expect_tx(mbar, bM + 2u * bO + bP);
-            for (uint32_t off = 0; off < bM; off += 32768u)
-                bulk_g2s(sbase + L.oM + off, reinterpret_cast<const char*>(gM) + off, min(32768u, bM - off), mbar);
-            bulk_g2s(sbase + L.oEo, gE + own_off * 32, bO, mbar);
-            bulk_g2s(sbase + L.oNo, gNR + own_off * 32, bO, mbar);
-            bulk_g2s(sbase + L.oEp, gE + opp_off * 32, bP, mbar);
-        }
-    } else {
-        for (uint32_t i = threadIdx.x; i < kopp_max * 32u; i += blockDim.x) sEp[i] = __ldcg(gE + opp_off * 32 + i);
+    // Sliced staged launches run under programmatic dependent launch: until griddepcontrol.wait (a no-op in any other launch)
+    // the launch before may still be running, so only what depends on no earlier launch goes first -- the mbarrier, the
+    // histograms and the first vertex batch (Feistel map and graph only).
+    if (STAGED && threadIdx.x == 0) {
+        mbar_init(mbar, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    {   // meanwhile: clear the histograms
+    {
         uint32_t* const hw = reinterpret_cast<uint32_t*>(smem_raw + L.oHist);
         for (uint32_t i = threadIdx.x; i < wpc * hist_words * 32u; i += blockDim.x) hw[i] = 0u;
     }
@@ -595,6 +610,24 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         return nb;
     };
     uint32_t nb = prepare(0);
+    asm volatile("griddepcontrol.wait;" ::: "memory");
+    __syncthreads();
+    // ---- stage the group's counts: one thread, bulk-async copies ----
+    if (STAGED) {
+        if (threadIdx.x == 0) {
+            const uint32_t bM = KA * KB * 128u, bO = kown_max * 128u, bP = kopp_max * 128u;
+            mbar_expect_tx(mbar, bM + 2u * bO + bP);
+            for (uint32_t off = 0; off < bM; off += 32768u)
+                bulk_g2s(sbase + L.oM + off, reinterpret_cast<const char*>(gM) + off, min(32768u, bM - off), mbar);
+            bulk_g2s(sbase + L.oEo, gE + own_off * 32, bO, mbar);
+            bulk_g2s(sbase + L.oNo, gNR + own_off * 32, bO, mbar);
+            bulk_g2s(sbase + L.oEp, gE + opp_off * 32, bP, mbar);
+        }
+    } else {
+        for (uint32_t i = threadIdx.x; i < kopp_max * 32u; i += blockDim.x) sEp[i] = __ldcg(gE + opp_off * 32 + i);
+    }
+    if (STAGED && !P.exclusive && !P.kat_mode) sliced_buffer_work(P, group, cta_in_group, cpg, type, KA, KB, kown_max, W);
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     if (STAGED) mbar_wait(mbar, 0);
     __syncthreads();
     // tables derived from the staged counts
@@ -712,6 +745,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         asm volatile("{\n\t.reg .u64 a;\n\tmad.wide.u32 a, %0, %1, %2;\n\tst.global.u8 [a], %3;\n\t}" :: "r"(vtx), "r"(C), "l"(LAB8 + (uint64_t)lane), "r"(x) : "memory");
     };
     RC_DECL();
+    RC_CTA_MARK(8);
     uint32_t ticket = warp;                               // STAGED: this warp's next vertex of the batch
     auto pop = [&]() -> uint32_t {
         if constexpr (STAGED) { const uint32_t i = ticket; ticket += P.warps_used; return i; }
@@ -975,7 +1009,10 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                                     const int old = sh_atom_add_s32(No_base + r * 128u, -1);
                                     if (old <= 1) { sh_red_add(No_base + r * 128u, 1); go = false; }
                                 } else {
-                                    const int old = atomicSub(&gLIVE[r * 32 + lane], 1);
+                                    // n_r at the start of the launch + the decrements before this one (the base is read-only
+                                    // during the launch)
+                                    const int old = atomicSub(&gLIVE[r * 32 + lane], 1) +
+                                                    ldc(P.s.nr + ((size_t)group * KK + own_off + r) * GROUP + lane);
                                     if (old <= 1) { atomicAdd(&gLIVE[r * 32 + lane], 1); go = false; }
                                     else sh_red_add(No_base + r * 128u, -1);
                                 }
@@ -1061,6 +1098,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         __syncthreads();
     }
     RC_PUBLISH(STAGED && warp < P.warps_used && lane == 0);
+    RC_CTA_RESET();
     if (warp < P.warps_used && live) {
         if (n_acc) atomicAdd(&P.accepted[c], (unsigned long long)n_acc);
         if (ds_sum != 0.0) atomicAdd(&P.dS_accum[c], ds_sum);
@@ -1082,6 +1120,7 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
         bulk_red_add_s32(P.nr_next + (size_t)group * KK * GROUP + own_off * 32, sbase + L.oNo, bO);
         bulk_commit_wait_all();
     }
+    RC_CTA_END();
 }
 
 #endif  // __CUDACC__

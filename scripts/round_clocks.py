@@ -6,13 +6,17 @@ Needs a library built with the round clocks compiled in:
 
 Every warp that takes vertices sums clock64 cycles over five phases: proposal + pass, dS / accept, commit, the wait for the
 round's reads and the wait for its commits, at the two named barriers of a round (sweep2.cuh, BISBM_ROUND_CLOCKS).  Printed: each phase's share of warp time,
-and the mean and max cycles of one vertex's proposal + pass.  One JSON line on stdout.
+and the mean and max cycles of one vertex's proposal + pass.  Per CTA (thread 0) the build also sums the prologue (kernel
+start -> first round: staging, tables, the first vertex batch, and under programmatic dependent launch the wait for the
+launch before) and the epilogue (last round -> publish done), printed as mean cycles per CTA and, at the SM clock
+nvidia-smi reports, microseconds.  One JSON line on stdout.
 """
 import argparse
 import ctypes
 import importlib
 import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -53,7 +57,7 @@ def main():
     pool.set_precision(args.precision)
     seeds = pkg.dist.chain_seeds(0, np.arange(args.chains))
     pool.randomize(seeds)
-    out = (ctypes.c_ulonglong * 8)()
+    out = (ctypes.c_ulonglong * 11)()
     pool.anneal("constant", 1.0, 0.0, args.sweeps * n, 10 ** 18, seeds)       # warm-up: the chains leave their random start
     if L.bisbm_round_clocks(out) != 0:
         raise SystemExit(L.bisbm_last_error().decode())
@@ -69,6 +73,16 @@ def main():
             "share": shares, "wait_share": shares["wait_reads"] + shares["wait_commits"],
             "pass_cycles_mean": c[0] / max(1, c[5]), "pass_cycles_max": c[6], "vertices": c[5], "warp_rounds": c[7],
             "cycles_per_warp_round": total / max(1, c[7])}
+    try:
+        mhz = float(subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=clocks.sm", "--format=csv,noheader,nounits"],
+                                   capture_output=True, text=True, timeout=20).stdout.split()[0])
+    except Exception:
+        mhz = None
+    ctas = max(1, c[10])
+    line["per_cta"] = {"ctas": c[10], "prologue_cycles": c[8] / ctas, "epilogue_cycles": c[9] / ctas, "sm_mhz": mhz,
+                       "prologue_us": c[8] / ctas / mhz if mhz else None, "epilogue_us": c[9] / ctas / mhz if mhz else None,
+                       "sweep_launches": pool.sweep_launches()}
+    print("per CTA: prologue %.0f cycles, epilogue %.0f cycles" % (c[8] / ctas, c[9] / ctas), file=sys.stderr)
     for p in PHASES:
         print("%-14s %6.2f %%" % (p, 100 * shares[p]), file=sys.stderr)
     print("proposal+pass per vertex: mean %.0f cycles, max %d" % (line["pass_cycles_mean"], c[6]), file=sys.stderr)
