@@ -442,6 +442,15 @@ __device__ __noinline__ static double slow2_logq_delta(const Tables tb, int e, i
     return log_q_tab(tb, e + de, n + dn) - log_q_tab(tb, e, n);
 }
 
+// estimate mode: occupied blocks of the moving type in this lane's view of n_r (the shared view, or the counts in L2).  Out of
+// line, like prior_k_delta: only a move that empties or opens a block needs it.
+template <bool STAGED>
+__device__ __noinline__ static int s2_occupied(uint32_t no_base, uint64_t gnol, uint32_t kown, uint32_t on) {
+    int occ = 0;
+    for (uint32_t b = 0; b < kown; ++b) occ += ((STAGED ? sh_ld(no_base + b * 128u) : gl_ld(gnol, b * 128u, on)) > 0) ? 1 : 0;
+    return occ;
+}
+
 // 1/T of global step t; T == 0 is returned as a negative value
 __device__ __noinline__ static double slow2_beta(int schedule, float p0, float p1, uint64_t t) {
     const double T = par_temperature(schedule, p0, p1, t);
@@ -651,12 +660,11 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
     }
     __syncthreads();
 
-    // estimate mode: occupied blocks of this lane's chain, per type (own type tracked through this warp's own moves)
-    int occ_own = 0, occ_opp = 0;
-    if (P.vary_k) {
-        for (uint32_t b = 0; b < kown_max; ++b) occ_own += (__ldcg(gNR + (own_off + b) * 32 + lane) > 0) ? 1 : 0;
+    // estimate mode: occupied blocks of the frozen type of this lane's chain (the moving type's are counted where a move
+    // needs them, from the same view as its n_r)
+    int occ_opp = 0;
+    if (P.vary_k)
         for (uint32_t b = 0; b < kopp_max; ++b) occ_opp += (__ldcg(gNR + (opp_off + b) * 32 + lane) > 0) ? 1 : 0;
-    }
 
     // lane-private shared byte addresses (entry j of this chain at +j*128)
     const uint32_t lane4 = lane * 4u;
@@ -977,11 +985,14 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     }
                     dS = AR::unit() * lgm + ((d == 0u) ? (R)0 : bdd) + lqr + lqs;
                     if (P.vary_k) {
-                        // the move empties r and / or opens s: the K-dependent prior terms change with the occupied count
+                        // the move empties r and / or opens s: the K-dependent prior terms change with the occupied count, read
+                        // from the view n_r came from (every round's commits of this CTA, not only this warp's)
                         const int dk = ((n_s == 0) ? 1 : 0) - ((n_r == 1) ? 1 : 0);
                         if (__any_sync(FULL, eval && dk != 0)) {
-                            if (eval && dk != 0)
+                            if (eval && dk != 0) {
+                                const int occ_own = s2_occupied<STAGED>(No_base, gNol, kown, live_u);
                                 dS += (R)prior_k_delta((double)G.n_edges, (double)nv, (double)occ_own, (double)occ_opp, dk);
+                            }
                             __syncwarp();
                         }
                     }
@@ -999,7 +1010,6 @@ __global__ void __launch_bounds__(NT, 1) sweep2_kernel(const __grid_constant__ S
                     RC_MARK(3);
                     if (go && P.vary_k) {
                         no_red(r, -1);                       // estimate mode: a block may empty
-                        occ_own += ((n_s == 0) ? 1 : 0) - ((n_r == 1) ? 1 : 0);
                     } else if (go) {
                         // the "would empty block r" veto of apply_mcmc_moves: exact where it can matter
                         if constexpr (STAGED) {
