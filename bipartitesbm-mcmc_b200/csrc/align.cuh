@@ -55,33 +55,22 @@ __global__ void __launch_bounds__(256) align_overlap_kernel(const LabT* __restri
     }
 }
 
-// shared memory of one align_assign_kernel warp for K blocks: u, v, minv (int64), p, way (int32), used (u8), each K + 1
+// shared memory of one warp_min_assign warp for K blocks: u, v, minv (int64), p, way (int32), used (u8), each K + 1
 __host__ __device__ inline size_t align_assign_smem(uint32_t K) { return (size_t)(K + 1) * (3 * 8 + 2 * 4 + 1); }
 
-// grid = (n_chains, 2 types), one warp per CTA, dynamic shared memory = align_assign_smem(max(ka, kb)).
-// Maximises sum_r w(r, pi(r)) with w(r, r') = O[r][r'] (K+1) + [r == r']: the overlap decides and the fixed-point bonus
-// (at most K < K+1) only breaks ties, so among the permutations of maximal overlap the one with the most fixed points
-// wins -- a chain equal to the reference keeps its labels, and empty blocks (zero rows and columns) stay in place.
-// Shortest augmenting paths with potentials (Hungarian / Jonker-Volgenant, minimising -w) in exact int64 arithmetic:
-// rows i = chain blocks, columns j = reference blocks, both 1-based (0 is the virtual start column).  The column loops
-// are lane-parallel; the argmin takes the lowest column among equals, so the result is deterministic.
-// map[c * (ka + kb) + g] = the global id chain c's block g is counted as.
-__global__ void __launch_bounds__(32) align_assign_kernel(const uint32_t* __restrict__ overlap, uint32_t C, uint32_t ka, uint32_t kb,
-                                                          uint32_t* __restrict__ map) {
-    extern __shared__ __align__(8) unsigned char s_hu[];
-    const uint32_t c = blockIdx.x, tb = blockIdx.y, lane = threadIdx.x;
-    const uint32_t K = tb ? kb : ka;
-    int64_t* const u = reinterpret_cast<int64_t*>(s_hu);
+// Minimum-cost assignment of a K x K integer cost (rows i to columns j, both 1-based), run by one warp in the
+// align_assign_smem(K) bytes at smem.  Shortest augmenting paths with potentials (Hungarian / Jonker-Volgenant) in exact
+// int64 arithmetic: 0 is the virtual start column.  The column loops are lane-parallel; the argmin takes the lowest column
+// among equals, so the result is deterministic.  Returns p: p[j] (j = 1..K) is the row assigned to column j, valid for
+// every lane after the call.  Used by align_assign_kernel and agree_final_kernel (agree.cuh).
+template <typename Cost>
+__device__ __forceinline__ const int32_t* warp_min_assign(uint32_t K, Cost cost, unsigned char* smem, uint32_t lane) {
+    int64_t* const u = reinterpret_cast<int64_t*>(smem);
     int64_t* const v = u + (K + 1);
     int64_t* const minv = v + (K + 1);
     int32_t* const p = reinterpret_cast<int32_t*>(minv + (K + 1));
     int32_t* const way = p + (K + 1);
     uint8_t* const used = reinterpret_cast<uint8_t*>(way + (K + 1));
-    const uint32_t* O = overlap + ((size_t)(c / 32) * ((size_t)ka * ka + (size_t)kb * kb) + (tb ? (size_t)ka * ka : 0)) * 32 + (c % 32);
-    const int64_t W1 = (int64_t)K + 1;
-    auto cost = [&](uint32_t i, uint32_t j) -> int64_t {       // -w of chain block i-1 against reference block j-1
-        return -((int64_t)O[((size_t)(i - 1) * K + (j - 1)) * 32] * W1 + (i == j ? 1 : 0));
-    };
     const int64_t INF = INT64_MAX / 4;
     for (uint32_t j = lane; j <= K; j += 32) { u[j] = 0; v[j] = 0; p[j] = 0; way[j] = 0; }
     __syncwarp();
@@ -122,6 +111,26 @@ __global__ void __launch_bounds__(32) align_assign_kernel(const uint32_t* __rest
         }
         __syncwarp();
     }
+    return p;
+}
+
+// grid = (n_chains, 2 types), one warp per CTA, dynamic shared memory = align_assign_smem(max(ka, kb)).
+// Maximises sum_r w(r, pi(r)) with w(r, r') = O[r][r'] (K+1) + [r == r']: the overlap decides and the fixed-point bonus
+// (at most K < K+1) only breaks ties, so among the permutations of maximal overlap the one with the most fixed points
+// wins -- a chain equal to the reference keeps its labels, and empty blocks (zero rows and columns) stay in place.
+// warp_min_assign minimises -w: rows i = chain blocks, columns j = reference blocks.
+// map[c * (ka + kb) + g] = the global id chain c's block g is counted as.
+__global__ void __launch_bounds__(32) align_assign_kernel(const uint32_t* __restrict__ overlap, uint32_t C, uint32_t ka, uint32_t kb,
+                                                          uint32_t* __restrict__ map) {
+    extern __shared__ __align__(8) unsigned char s_hu[];
+    const uint32_t c = blockIdx.x, tb = blockIdx.y, lane = threadIdx.x;
+    const uint32_t K = tb ? kb : ka;
+    const uint32_t* O = overlap + ((size_t)(c / 32) * ((size_t)ka * ka + (size_t)kb * kb) + (tb ? (size_t)ka * ka : 0)) * 32 + (c % 32);
+    const int64_t W1 = (int64_t)K + 1;
+    auto cost = [&](uint32_t i, uint32_t j) -> int64_t {       // -w of chain block i-1 against reference block j-1
+        return -((int64_t)O[((size_t)(i - 1) * K + (j - 1)) * 32] * W1 + (i == j ? 1 : 0));
+    };
+    const int32_t* p = warp_min_assign(K, cost, s_hu, lane);
     const uint32_t base = tb ? ka : 0;
     uint32_t* const m = map + (size_t)c * (ka + kb) + base;
     for (uint32_t j = 1 + lane; j <= K; j += 32) m[p[j] - 1] = base + j - 1;

@@ -17,6 +17,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <map>
 #include <set>
 #include <memory>
@@ -32,6 +33,7 @@
 #include "sweep_aux.cuh"
 #include "align.cuh"
 #include "coassign.cuh"
+#include "agree.cuh"
 #include "sweep2.cuh"
 #include "tempering.cuh"
 
@@ -2018,6 +2020,151 @@ int bisbm_coassign_get(bisbm_handle* h, uint32_t* counts, uint64_t* n_counted) {
         }
     }
     if (n_counted) *n_counted = h->co_counted;
+    return BISBM_OK;
+}
+
+int bisbm_chain_agreement(bisbm_handle* h, const uint32_t* ref_labels, int with_overlap, double* out) {
+    if (!h) return fail(BISBM_ERR_ARG, "null handle");
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!out) return fail(BISBM_ERR_ARG, "null argument");
+    const uint32_t N = h->n_chains, C = h->C, G = C / 32, n = h->n, na = h->na, nb = h->n - h->na;
+    // the table side of a type: the pool's largest block count of it (smaller chains leave zero rows and columns)
+    uint32_t KA = 0, KB = 0;
+    for (uint32_t c = 0; c < N; ++c) { KA = std::max(KA, h->h_ka[c]); KB = std::max(KB, h->h_kb[c]); }
+    std::vector<uint32_t> ref;
+    if (ref_labels) {
+        ref.resize(n);
+        for (uint32_t v = 0; v < n; ++v) {
+            const uint32_t g = ref_labels[v];
+            if (v < na ? g >= KA : (g < KA || g >= KA + KB))
+                return fail(BISBM_ERR_ARG, "reference label %u of node %u is not a type-%c block (pool: ka <= %u, kb <= %u)", g, v,
+                            v < na ? 'a' : 'b', KA, KB);
+            ref[v] = v < na ? g : g - KA;
+        }
+    }
+    int optin = 0;
+    CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    const uint32_t Ks[2] = {KA, KB};
+    uint32_t rpp[2], passes[2];
+    for (int t = 0; t < 2; ++t) {
+        rpp[t] = std::min<uint32_t>(Ks[t], (uint32_t)((size_t)optin / ((size_t)Ks[t] * 32 * sizeof(uint32_t))));
+        if (rpp[t] == 0)
+            return fail(BISBM_ERR_ARG, "%u blocks per type: one row of the contingency table does not fit in %d bytes of shared memory", Ks[t], optin);
+        passes[t] = (Ks[t] + rpp[t] - 1) / rpp[t];
+    }
+    const size_t asmem = with_overlap ? align_assign_smem(std::max(KA, KB)) : 0;
+    if (asmem > (size_t)optin)
+        return fail(BISBM_ERR_ARG, "matching %u blocks needs %zu bytes of shared memory per block (device: %d)", std::max(KA, KB), asmem, optin);
+    // the tables of one row chain against every column group; a chunk holds up to AGREE_CHUNK rows within a quarter of free memory
+    const size_t cells_a = (size_t)G * KA * KA * 32, cells_b = (size_t)G * KB * KB * 32;
+    const size_t per_row = (cells_a + cells_b) * sizeof(uint32_t);
+    const uint32_t n_rows = ref_labels ? 1 : N;
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    if (per_row > free_b / 4)
+        return fail(BISBM_ERR_ARG, "one chain's contingency tables take %zu bytes: more than a quarter of the %zu bytes free", per_row, free_b);
+    const uint32_t chunk = (uint32_t)std::min<size_t>({(size_t)AGREE_CHUNK, (size_t)n_rows, free_b / 4 / per_row});
+    const size_t n_stats = (size_t)n_rows * N * 2;
+    struct DevBuf {            // freed on every return path
+        void* p = nullptr;
+        ~DevBuf() { if (p) cudaFree(p); }
+    } d_tab, d_stats, d_ref;
+    CU(cudaMalloc(&d_tab.p, chunk * per_row));
+    CU(cudaMalloc(&d_stats.p, n_stats * sizeof(AgreeStats)));
+    if (ref_labels) {
+        CU(cudaMalloc(&d_ref.p, (size_t)n * sizeof(uint32_t)));
+        CU(cudaMemcpyAsync(d_ref.p, ref.data(), (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    }
+    const bool from8 = h->lab32_stale;      // the array the sweep keeps current, as launch_marginal reads
+    for (int t = 0; t < 2; ++t) {
+        const size_t smem = (size_t)rpp[t] * Ks[t] * 32 * sizeof(uint32_t);
+        if (smem > 48 * 1024) {
+            rc = from8 ? ensure_smem_attr(h, (const void*)agree_table_kernel<uint8_t>, optin)
+                       : ensure_smem_attr(h, (const void*)agree_table_kernel<int32_t>, optin);
+            if (rc) return rc;
+        }
+    }
+    if (asmem > 48 * 1024 && (rc = ensure_smem_attr(h, (const void*)agree_final_kernel, optin))) return rc;
+    uint32_t* tab_a = static_cast<uint32_t*>(d_tab.p);
+    AgreeStats* stats = static_cast<AgreeStats*>(d_stats.p);
+    const uint32_t* d_refp = static_cast<const uint32_t*>(d_ref.p);
+    for (uint32_t row0 = 0; row0 < n_rows; row0 += chunk) {
+        const uint32_t rows = std::min(chunk, n_rows - row0);
+        uint32_t* tab_b = tab_a + (size_t)rows * cells_a;
+        CU(cudaMemsetAsync(tab_a, 0, rows * per_row, h->stream));
+        for (int t = 0; t < 2; ++t) {
+            const uint32_t nt = t ? nb : na, v0 = t ? na : 0;
+            if (nt == 0) continue;
+            // split the nodes when (row, group, pass) alone gives fewer than two CTAs per SM; at least 1024 nodes per split
+            const uint64_t base = (uint64_t)rows * (ref_labels ? G : (G + 1) / 2) * passes[t];
+            const uint32_t splits = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>((2ull * h->sm_count + base - 1) / base, (nt + 1023) / 1024));
+            const dim3 grid(rows, G, passes[t] * splits);
+            const size_t smem = (size_t)rpp[t] * Ks[t] * 32 * sizeof(uint32_t);
+            const uint32_t* krow = t ? h->d_kb : h->d_ka;
+            const uint32_t* rp = d_refp ? d_refp + v0 : nullptr;
+            uint32_t* tb = t ? tab_b : tab_a;
+            if (from8)
+                agree_table_kernel<uint8_t><<<grid, AGREE_THREADS, smem, h->stream>>>(h->d_lab8 + (size_t)v0 * C, C, N, nt, Ks[t], krow, rp,
+                                                                                    row0, rpp[t], splits, tb);
+            else
+                agree_table_kernel<int32_t><<<grid, AGREE_THREADS, smem, h->stream>>>(h->d_labels + (size_t)v0 * C, C, N, nt, Ks[t], krow, rp,
+                                                                                    row0, rpp[t], splits, tb);
+            CU(cudaGetLastError());
+        }
+        agree_final_kernel<<<dim3(N, rows, 2), 32, asmem, h->stream>>>(tab_a, tab_b, KA, KB, C, N, row0, ref_labels ? 0 : 1,
+                                                                        with_overlap ? 1 : 0, stats);
+        CU(cudaGetLastError());
+    }
+    std::vector<AgreeStats> st(n_stats);
+    CU(cudaMemcpyAsync(st.data(), stats, n_stats * sizeof(AgreeStats), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    // the metrics of each slot: type a, type b, and the whole partition (the joint table is block-diagonal across the
+    // types, so its statistics are the sums over both)
+    const uint32_t n_cols = ref_labels ? 1 : N;
+    const size_t plane = (size_t)N * n_cols;
+    const double nan = std::numeric_limits<double>::quiet_NaN();
+    auto put = [&](int metric, int slot, uint32_t c, uint32_t col, double x) { out[((size_t)metric * 3 + slot) * plane + (size_t)c * n_cols + col] = x; };
+    for (uint32_t c = 0; c < N; ++c)
+        for (uint32_t col = 0; col < n_cols; ++col) {
+            if (!ref_labels && col < c) {      // mirrored from (col, c): bitwise symmetric
+                for (int metric = 0; metric < 4; ++metric)
+                    for (int slot = 0; slot < 3; ++slot)
+                        out[((size_t)metric * 3 + slot) * plane + (size_t)c * n_cols + col] = out[((size_t)metric * 3 + slot) * plane + (size_t)col * n_cols + c];
+                continue;
+            }
+            // stats rows: the row chain (or the reference) x the column chain
+            const AgreeStats* s = ref_labels ? &st[(size_t)c * 2] : &st[((size_t)c * N + col) * 2];
+            for (int slot = 0; slot < 3; ++slot) {
+                AgreeStats z{};
+                for (int t = 0; t < 2; ++t) {
+                    if (slot != 2 && slot != t) continue;
+                    z.s_xy += s[t].s_xy; z.s_x += s[t].s_x; z.s_y += s[t].s_y;
+                    z.p_xy += s[t].p_xy; z.p_x += s[t].p_x; z.p_y += s[t].p_y; z.m += s[t].m;
+                }
+                const uint64_t nn = slot == 0 ? na : slot == 1 ? nb : n;
+                if (!ref_labels && col == c) {
+                    put(BISBM_AGREE_VI, slot, c, col, 0.0); put(BISBM_AGREE_NMI, slot, c, col, 1.0); put(BISBM_AGREE_ARI, slot, c, col, 1.0);
+                    put(BISBM_AGREE_OVERLAP, slot, c, col, with_overlap ? 1.0 : nan);
+                    continue;
+                }
+                const double dn = (double)nn, ln = nn ? std::log(dn) : 0.0;
+                const uint64_t pairs = nn * (nn - (nn > 0)) / 2;
+                // a partition with all nodes in one block has H = 0 exactly, and shares no information
+                const bool one_x = z.p_x == pairs, one_y = z.p_y == pairs;
+                const double hx = one_x ? 0.0 : ln - z.s_x / dn, hy = one_y ? 0.0 : ln - z.s_y / dn;
+                const double mi = one_x || one_y ? 0.0 : ln + (z.s_xy - z.s_x - z.s_y) / dn;
+                const double vi = nn ? (z.s_x + z.s_y - 2.0 * z.s_xy) / dn : 0.0;
+                const double nmi = hx + hy == 0.0 ? 1.0 : 2.0 * mi / (hx + hy);
+                const double expected = pairs ? (double)z.p_x * (double)z.p_y / (double)pairs : 0.0;
+                const double denom = 0.5 * ((double)z.p_x + (double)z.p_y) - expected;
+                const double ari = denom == 0.0 ? 1.0 : ((double)z.p_xy - expected) / denom;
+                put(BISBM_AGREE_VI, slot, c, col, vi);
+                put(BISBM_AGREE_NMI, slot, c, col, nmi);
+                put(BISBM_AGREE_ARI, slot, c, col, ari);
+                put(BISBM_AGREE_OVERLAP, slot, c, col, with_overlap ? (nn ? (double)z.m / dn : 1.0) : nan);
+            }
+        }
     return BISBM_OK;
 }
 

@@ -17,12 +17,16 @@
 //                          With --coassign FILE --coassign_out OUT every sample also counts, for each pair of the query
 //                          nodes in FILE, the chains in which the two share a block (bisbm_coassign_set); OUT gets the
 //                          matrix, summed over the GPUs of --gpus
+//   --agreement_out FILE   (one GPU: --chains N >= 2, --marginalize, --estimate) compares the final states of the chains
+//                          pairwise (bisbm_chain_agreement): FILE gets NMI / VI / ARI / matched overlap per pair, stderr
+//                          a one-line summary with the modes at overlap >= 0.95
 //   --estimate             README "estimation" output format for fixed (Ka, Kb): CSV lines
 //                          sweep,Ka,Kb,loglik,labels... of the last 1000 samples
 //   -g / --merge, -u / --nature, or initial labels whose block counts differ from -z: the agglomerative
 //                          merge / split initialiser (src/mcmc_main.cc:350-451) over bisbm_replay_agg_merge -- the
 //                          geospace ladder, one greedy sweep between rungs, then the abrupt_cool anneal; one replay
 //                          chain, the label line of the reference for the merge paths
+#include <algorithm>
 #include <chrono>
 #include <cmath>
 #include <cstdint>
@@ -64,7 +68,7 @@ const Spec kSpecs[] = {
     // README-only modes and the extensions of this build
     {"maximize", 0, 0}, {"estimate", 0, 0}, {"marginalize", 0, 0}, {"chains", 0, 1}, {"gen_seed", 0, 1},
     {"device", 0, 1}, {"max_inflight", 0, 1}, {"gpus", 0, 1}, {"tempering", 0, 2}, {"swap_every", 0, 1},
-    {"align", 0, 0}, {"coassign", 0, 1}, {"coassign_out", 0, 1},
+    {"align", 0, 0}, {"coassign", 0, 1}, {"coassign_out", 0, 1}, {"agreement_out", 0, 1},
 };
 
 const Spec* find_spec(const std::string& tok) {
@@ -156,7 +160,11 @@ void usage(const char* argv0) {
                  "                                        counts, per pair of query nodes of one type, the chains in which the\n"
                  "                                        two share a block (posterior co-assignment, label-switching free)\n"
                  "  --coassign_out arg                    file the counts go to: a line \"Q n_counted\", then Q lines of Q\n"
-                 "                                        counts in query order (summed over the GPUs of --gpus)\n";
+                 "                                        counts in query order (summed over the GPUs of --gpus)\n"
+                 "  --agreement_out arg                   one GPU, --chains >= 2 (plain, --marginalize, --estimate): compare\n"
+                 "                                        the chains' final states pairwise; the file gets a line n_chains,\n"
+                 "                                        then per pair c1 < c2: c1 c2 nmi vi ari overlap, then the same four\n"
+                 "                                        for type a and for type b (label-switching free)\n";
 }
 
 // the ladder of block counts between (start_a, start_b) and (end_a, end_b) (reference src/support/util.hh:99-146): the type
@@ -235,6 +243,54 @@ int add_coassign(bisbm_handle* h, size_t q, std::vector<uint64_t>& sum, uint64_t
     for (size_t i = 0; i < q * q; ++i) sum[i] += c[i];
     n_counted += nc;
     return BISBM_OK;
+}
+
+// --agreement_out: every pair of the pool's chains compared on their current labels (bisbm_chain_agreement).  The file gets
+// "n_chains", then per pair c1 < c2 the whole partition's nmi vi ari overlap, then type a's, then type b's; stderr one
+// summary line: the whole partition's NMI over the pairs and the modes, the connected components of overlap >= 0.95
+bool write_agreement(bisbm_handle* h, size_t nc, const std::string& path) {
+    std::vector<double> a(4 * 3 * nc * nc);
+    if (!check(bisbm_chain_agreement(h, nullptr, 1, a.data()))) return false;
+    auto at = [&](int metric, int slot, size_t i, size_t j) { return a[(((size_t)metric * 3 + slot) * nc + i) * nc + j]; };
+    std::ofstream f(path.c_str());
+    if (!f.is_open()) { std::cerr << "cannot write the --agreement_out file " << path << "\n"; return false; }
+    f.precision(17);
+    f << nc << "\n";
+    const int metrics[4] = {BISBM_AGREE_NMI, BISBM_AGREE_VI, BISBM_AGREE_ARI, BISBM_AGREE_OVERLAP};
+    std::vector<double> nmi;
+    for (size_t i = 0; i < nc; ++i)
+        for (size_t j = i + 1; j < nc; ++j) {
+            f << i << " " << j;
+            for (int slot : {2, 0, 1})
+                for (int metric : metrics) f << " " << at(metric, slot, i, j);
+            f << "\n";
+            nmi.push_back(at(BISBM_AGREE_NMI, 2, i, j));
+        }
+    f.close();
+    if (f.fail()) { std::cerr << "cannot write the --agreement_out file " << path << "\n"; return false; }
+    std::sort(nmi.begin(), nmi.end());
+    const size_t np = nmi.size();
+    const double median = np % 2 ? nmi[np / 2] : 0.5 * (nmi[np / 2 - 1] + nmi[np / 2]);
+    // modes: components of the overlap graph, numbered by their first chain
+    std::vector<size_t> mode(nc, nc), sizes;
+    for (size_t c = 0; c < nc; ++c) {
+        if (mode[c] < nc) continue;
+        const size_t k = sizes.size();
+        sizes.push_back(0);
+        std::vector<size_t> stack{c};
+        mode[c] = k;
+        while (!stack.empty()) {
+            const size_t x = stack.back();
+            stack.pop_back();
+            ++sizes[k];
+            for (size_t y = 0; y < nc; ++y)
+                if (mode[y] == nc && at(BISBM_AGREE_OVERLAP, 2, x, y) >= 0.95) { mode[y] = k; stack.push_back(y); }
+        }
+    }
+    std::clog << "chain agreement: NMI median " << median << " min " << nmi[0] << ", modes at overlap >= 0.95: " << sizes.size() << " (sizes";
+    for (size_t z : sizes) std::clog << " " << z;
+    std::clog << ")\n";
+    return true;
 }
 
 // --align's reference: the chain of lowest entropy() in the pool (under a ladder, among the chains at rung 0)
@@ -346,6 +402,11 @@ int main(int argc, char const* argv[]) {
     }
     std::vector<uint64_t> co_sum;
     uint64_t co_counted = 0;
+    const bool agreement = o.has("agreement_out");
+    if (agreement) {
+        if (gpus > 1) { std::cerr << "--agreement_out compares the chains of one GPU (no --gpus > 1)\n"; return 1; }
+        if (chains < 2) { std::cerr << "--agreement_out needs --chains >= 2\n"; return 1; }
+    }
     if (gpus > chains) gpus = chains;
     // stdout carries the label line and nothing else: whatever NCCL has to say (its version banner under NCCL_DEBUG)
     // goes to stderr unless the user chose a file
@@ -437,8 +498,8 @@ int main(int argc, char const* argv[]) {
         if (merge) { for (size_t v = 0; v < N; ++v) memberships_init[v] = (unsigned)v; ka = NA; kb = NB; }
         int diff_a = (int)ka - (int)KA, diff_b = (int)kb - (int)KB;
         if (merge || diff_a != 0 || diff_b != 0) {
-            if (chains != 1 || o.has("marginalize") || o.has("estimate")) {
-                std::cerr << "the agglomerative paths run one chain (no --chains / --marginalize / --estimate)\n";
+            if (chains != 1 || o.has("marginalize") || o.has("estimate") || agreement) {
+                std::cerr << "the agglomerative paths run one chain (no --chains / --marginalize / --estimate / --agreement_out)\n";
                 return 1;
             }
             if ((double)ka * (double)kb * 128.0 > 16e9) { std::cerr << "too many initial blocks for the K x K block matrix\n"; return 1; }
@@ -620,6 +681,7 @@ int main(int argc, char const* argv[]) {
             }
             if (!check(bisbm_tempering_run(h, sampling_steps, swap_every, f, seeds.data(), (uint64_t)seed, (uint32_t)max_inflight, nullptr))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
+            if (agreement && !write_agreement(h, chains, o.vals["agreement_out"][0])) return 1;
             if (coassign && (!check(add_coassign(h, query.size(), co_sum, co_counted)) ||
                              !write_coassign(o.vals["coassign_out"][0], query.size(), co_sum, co_counted))) return 1;
             output_vec(out, std::cout);
@@ -637,6 +699,7 @@ int main(int argc, char const* argv[]) {
                     !check(bisbm_marginalize(h, 0, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
             } else if (!check(bisbm_marginalize(h, burn_in, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
+            if (agreement && !write_agreement(h, chains, o.vals["agreement_out"][0])) return 1;
             if (coassign && (!check(add_coassign(h, query.size(), co_sum, co_counted)) ||
                              !write_coassign(o.vals["coassign_out"][0], query.size(), co_sum, co_counted))) return 1;
             output_vec(out, std::cout);
@@ -665,6 +728,7 @@ int main(int argc, char const* argv[]) {
                 for (uint32_t x : out) std::cout << "," << x;
                 std::cout << "\n";
             }
+            if (agreement && !write_agreement(h, chains, o.vals["agreement_out"][0])) return 1;
         }
         bisbm_destroy(h);
         return 0;
@@ -690,6 +754,7 @@ int main(int argc, char const* argv[]) {
         for (size_t c = 1; c < chains; ++c) if (ent[c] < ent[best]) best = c;
         rate = acc[best]; S = ent[best];
         if (!check(bisbm_get_labels(h, (uint32_t)best, out.data()))) return 1;
+        if (agreement && !write_agreement(h, chains, o.vals["agreement_out"][0])) return 1;
     }
     std::clog << "acceptance ratio " << rate << "\n";
     std::clog << "(Ka, Kb) = (" << KA << ", " << KB << ") \n";  // blockmodel_t::summary, reference src/blockmodel.cc:748-751

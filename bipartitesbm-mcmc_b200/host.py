@@ -81,6 +81,7 @@ SIGNATURES = {
     "bisbm_marginals_alignment": (C.c_int, [C.c_void_p, _u32p]),
     "bisbm_coassign_set": (C.c_int, [C.c_void_p, C.c_uint32, _u32p]),
     "bisbm_coassign_get": (C.c_int, [C.c_void_p, _u32p, _u64p]),
+    "bisbm_chain_agreement": (C.c_int, [C.c_void_p, _u32p, C.c_int, _dp]),
     "bisbm_tempering_set": (C.c_int, [C.c_void_p, C.c_uint32, _dp, _u32p]),
     "bisbm_tempering_run": (C.c_int, [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, _u64p, C.c_uint64, C.c_uint32, _dp]),
     "bisbm_tempering_stats": (C.c_int, [C.c_void_p, _u32p, _u64p, _u64p, _u64p, _u64p, _u64p]),
@@ -298,6 +299,31 @@ def geometric_ladder(t_min, t_max, n):
     return np.maximum.accumulate(out)
 
 
+def chain_modes(overlap_whole, threshold=0.95):
+    """Mode id per chain from a pairwise overlap matrix (ChainPool.chain_agreement()["overlap"][2]): the connected
+    components of "overlap >= threshold", numbered 0, 1, .. in order of each component's first chain."""
+    o = np.asarray(overlap_whole, dtype=np.float64)
+    if o.ndim != 2 or o.shape[0] != o.shape[1]:
+        raise ValueError("the overlap matrix must be square")
+    n = o.shape[0]
+    adj = o >= threshold
+    mode = np.full(n, -1, dtype=np.int64)
+    k = 0
+    for c in range(n):
+        if mode[c] >= 0:
+            continue
+        mode[c] = k
+        stack = [c]
+        while stack:
+            x = stack.pop()
+            for y in np.flatnonzero(adj[x] | adj[:, x]):
+                if mode[y] < 0:
+                    mode[y] = k
+                    stack.append(y)
+        k += 1
+    return mode
+
+
 def edge_to_adj(edge_list, N, na=None, nb=None, device=0):
     """reference src/graph_utilities.cc:36-49.  The bipartition (na, nb) must be given since
     the device graph validates it; N = na + nb."""
@@ -479,6 +505,26 @@ class ChainPool:
         n = C.c_uint64()
         _check(self.L.bisbm_coassign_get(self.g.h, _p(out, C.c_uint32), C.byref(n)))
         return out, n.value
+
+    def chain_agreement(self, ref=None, overlap=True):
+        """Partition agreement of the chains' current labels (bisbm_chain_agreement), free of label switching: a dict
+        {"vi", "nmi", "ari", "overlap"} of float64 arrays [3][C][C] (slot 0 type a, 1 type b, 2 the whole partition;
+        every pair of chains), or [3][C] against the partition ref (global ids, type b from the pool's largest ka on).
+        overlap=False skips the matching (the "overlap" entries are then NaN)."""
+        C_ = self.n_chains
+        cols = C_ if ref is None else 1
+        out = np.zeros((4, 3, C_, cols), dtype=np.float64)
+        r = None
+        if ref is not None:
+            r = np.asarray(ref)
+            if r.shape != (self.g.n,) or (r.size and (r.min() < 0 or r.max() > 0xffffffff)):
+                raise ValueError("the reference is one block id per node")
+            r = np.ascontiguousarray(r, dtype=np.uint32)
+        _check(self.L.bisbm_chain_agreement(self.g.h, _p(r, C.c_uint32) if r is not None else None, 1 if overlap else 0,
+                                            _p(out, C.c_double)))
+        if ref is not None:
+            out = out[..., 0]
+        return {"vi": out[0], "nmi": out[1], "ari": out[2], "overlap": out[3]}
 
     def stream(self):
         """cudaStream_t (as int) the handle launches on."""

@@ -181,6 +181,31 @@ int bisbm_coassign_set(bisbm_handle* h, uint32_t q, const uint32_t* nodes);
  * of counted (chain, sample) pairs (the counts wrap past 2^32 - 1).  n_counted (may be NULL): the same number as uint64.
  * Waits for the handle's stream.  BISBM_ERR_STATE without a query set.  Multi-GPU: read each handle and sum. */
 int bisbm_coassign_get(bisbm_handle* h, uint32_t* counts, uint64_t* n_counted);
+/* Partition agreement between chains (label-switching free; no counterpart in the reference): do the chains of a pool
+ * sit in one mode?  For chains x, y and a node type with n_t nodes, n_ij = #nodes in block i of x and block j of y, with
+ * row sums a_i and column sums b_j; S_xy = sum n_ij log n_ij, S_x = sum a_i log a_i, S_y = sum b_j log b_j, P_xy =
+ * sum C(n_ij, 2), P_x, P_y alike, M = max over bijections pi of sum_i n_{i,pi(i)} (the nodes that agree after matching):
+ *   VI = (S_x + S_y - 2 S_xy) / n (nats); NMI = 2 I / (H_x + H_y), with H_x = log n - S_x / n, I = log n + (S_xy - S_x -
+ *   S_y) / n, and 1 when H_x + H_y = 0; ARI (Hubert-Arabie) = (P_xy - P_x P_y / C(n,2)) / ((P_x + P_y) / 2 - P_x P_y /
+ *   C(n,2)), 1 when the denominator is 0; overlap = M / n.
+ * The whole bipartite partition sums the statistics of both types (its table is block-diagonal), with n = na + nb.  A
+ * permutation of a chain's block ids changes none of them, so pools of mixed (ka, kb), estimate mode (empty blocks are
+ * zero rows) and tempering pools (every chain, whatever its rung) are compared as they are.
+ * out[4][3][n_chains][n_cols]: metric (BISBM_AGREE_*), slot (0 type a, 1 type b, 2 whole partition), chain, column.
+ *   ref_labels == NULL: every pair of chains, n_cols = n_chains; symmetric bit for bit, diagonal VI = 0, NMI = ARI =
+ *   overlap = 1.  ref_labels[n]: each chain against that one partition, n_cols = 1; global ids in the pool's numbering
+ *   (type a in [0, KA), type b in [KA, KA + KB), KA and KB the largest ka and kb of the pool).
+ *   with_overlap == 0 skips the matching; the overlap entries are then NaN.
+ * Reads the chains' current labels (the u8 shadow or the i32 labels, whichever the sweep keeps current) and changes no
+ * state any other call sees: labels, counts, eta, histogram, co-assignment counts, alignment and tempering counters are
+ * as they were, and bisbm_last_timing and the launch counters are not updated.  The kernels (contingency tables per chunk
+ * of at most 64 row chains, then one warp per pair and type for the statistics) are queued on the handle's stream; the
+ * call synchronises once, to copy the statistics out, and composes the metrics in double on the host.  Two calls give
+ * bit-identical results.  Errors: BISBM_ERR_ARG for a null handle or output, a reference label outside its node's type
+ * range, or one chain's tables (C / 32 * 32 * (KA^2 + KB^2) uint32) larger than a quarter of the free device memory;
+ * BISBM_ERR_STATE without a pool. */
+enum { BISBM_AGREE_VI = 0, BISBM_AGREE_NMI = 1, BISBM_AGREE_ARI = 2, BISBM_AGREE_OVERLAP = 3 };
+int bisbm_chain_agreement(bisbm_handle* h, const uint32_t* ref_labels, int with_overlap, double* out);
 /* ---- parallel tempering (replica exchange; no counterpart in the reference) ----------------------------------------
  * Ladder: n_rungs = R temperatures temps[0..R-1], each finite and > 0, non-decreasing; rung 0 is the cold one.  n_chains
  * must be a multiple of R: chains l R .. l R + R - 1 form ladder l, and chain l R + i starts at rung i unless rung_of_chain
