@@ -33,6 +33,7 @@
 #include "sweep_aux.cuh"
 #include "align.cuh"
 #include "coassign.cuh"
+#include "modes.cuh"
 #include "agree.cuh"
 #include "sweep2.cuh"
 #include "tempering.cuh"
@@ -140,6 +141,15 @@ struct bisbm_handle {
     std::vector<uint32_t> co_pos;              // caller's query index -> position in the type-sorted order
     uint32_t *d_co_nodes = nullptr, *d_co_tiles = nullptr, *d_co_counts = nullptr;
     uint64_t co_counted = 0;                   // (chain, sample) pairs counted since bisbm_coassign_set
+    // marginals by mode (bisbm_marginal_modes_set, modes.cuh): a set of md_M reference partitions is in place while md_M > 0.
+    // Per mode m: its reference-sorted node order at d_md_order + m n, its segments at d_md_seg + md_seg_off[m] (the layout
+    // of d_al_seg), its overlap tables and maps in slices of d_md_overlap and d_md_map
+    uint32_t md_M = 0, md_ka = 0, md_kb = 0;
+    uint64_t md_min_ov = 0;                    // a sample whose best overlap is below this many nodes is left unassigned
+    std::vector<uint32_t> md_segs, md_seg_off;
+    uint32_t *d_md_order = nullptr, *d_md_seg = nullptr, *d_md_overlap = nullptr, *d_md_map = nullptr, *d_md_hist = nullptr;
+    uint32_t *d_md_nearest = nullptr, *d_md_chain = nullptr;
+    unsigned long long* d_md_counted = nullptr;   // [md_M + 1]
     // timing of the last parallel call
     double last_ms = 0.0;
     uint64_t last_launches = 0, last_moves = 0;
@@ -195,6 +205,14 @@ void free_align(bisbm_handle* h) {
     h->al_sampled = false;
 }
 
+void free_modes(bisbm_handle* h) {
+    dfree(h->d_md_order); dfree(h->d_md_seg); dfree(h->d_md_overlap); dfree(h->d_md_map); dfree(h->d_md_hist);
+    dfree(h->d_md_nearest); dfree(h->d_md_chain); dfree(h->d_md_counted);
+    h->md_M = h->md_ka = h->md_kb = 0;
+    h->md_min_ov = 0;
+    h->md_segs.clear(); h->md_seg_off.clear();
+}
+
 void free_coassign(bisbm_handle* h) {
     dfree(h->d_co_nodes); dfree(h->d_co_tiles); dfree(h->d_co_counts);
     h->co_q = h->co_qa = h->co_qb = h->co_tiles = 0;
@@ -205,6 +223,7 @@ void free_coassign(bisbm_handle* h) {
 void free_chains(bisbm_handle* h) {
     free_ladder(h);
     free_align(h);
+    free_modes(h);
     dfree(h->d_ka); dfree(h->d_kb); dfree(h->d_labels); dfree(h->d_labels_tmp);
     dfree(h->d_m); dfree(h->d_e); dfree(h->d_nr); dfree(h->d_eta); dfree(h->d_lq); dfree(h->d_m2); dfree(h->d_e2); dfree(h->d_nr2); dfree(h->d_m3); dfree(h->d_e3); dfree(h->d_nr3);
     dfree(h->d_nr_live[0]); dfree(h->d_nr_live[1]); dfree(h->d_eta_ring); dfree(h->d_kat_out); dfree(h->d_lab8);
@@ -1158,6 +1177,7 @@ static int alloc_chains(bisbm_handle* h, uint32_t n_chains, const uint32_t* ka, 
     CU(cudaSetDevice(h->device));
     free_ladder(h);      // a new pool has no ladder
     free_align(h);       // and no alignment reference
+    free_modes(h);       // nor mode set
     uint32_t KA = 0, KB = 0;
     for (uint32_t c = 0; c < n_chains; ++c) {
         if (ka[c] == 0 || kb[c] == 0) return fail(BISBM_ERR_ARG, "chain %u: ka and kb must be >= 1", c);
@@ -1467,8 +1487,8 @@ MergeCtx mctx(bisbm_handle* h, uint32_t chain, const ReplaySlot& sl, const Merge
 // new block counts of one chain: host copy, device copy, counts rebuilt from the labels (init_bisbm)
 int set_chain_k(bisbm_handle* h, uint32_t chain, uint32_t ka, uint32_t kb) {
     if (ka > h->KA || kb > h->KB) return fail(BISBM_ERR_STATE, "chain %u: (%u, %u) blocks exceed the pool's strides (%u, %u)", chain, ka, kb, h->KA, h->KB);
-    // an alignment reference and its maps are for the (ka, kb) the pool had: a chain with other block counts drops it
-    if (ka != h->h_ka[chain] || kb != h->h_kb[chain]) free_align(h);
+    // an alignment reference, a mode set and their maps are for the (ka, kb) the pool had: a chain with other block counts drops them
+    if (ka != h->h_ka[chain] || kb != h->h_kb[chain]) { free_align(h); free_modes(h); }
     h->h_ka[chain] = ka; h->h_kb[chain] = kb;
     CU(cudaMemcpyAsync(h->d_ka + chain, &h->h_ka[chain], sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemcpyAsync(h->d_kb + chain, &h->h_kb[chain], sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
@@ -1851,12 +1871,42 @@ static int launch_marginal(bisbm_handle* h, const uint32_t* rung = nullptr) {
         CU(cudaGetLastError());
         h->co_counted += rung ? h->n_chains / h->tp_rungs : h->n_chains;    // a ladder has exactly one chain at rung 0
     }
+    if (h->md_M) {
+        // marginals by mode: each mode's permutations by the alignment kernels into its own slices, then the nearest mode
+        // per chain, then the histogram of that mode
+        const uint32_t ka = h->md_ka, kb = h->md_kb, M = h->md_M, width = ka + kb;
+        const size_t tab = (size_t)h->C * ((size_t)ka * ka + (size_t)kb * kb);
+        CU(cudaMemsetAsync(h->d_md_overlap, 0, M * tab * sizeof(uint32_t), h->stream));
+        const size_t osmem = (size_t)std::max(ka, kb) * 32 * sizeof(uint32_t), asmem = align_assign_smem(std::max(ka, kb));
+        for (uint32_t m = 0; m < M; ++m) {
+            const uint32_t S = h->md_segs[m], *order = h->d_md_order + (size_t)m * h->n;
+            const uint32_t *seg_begin = h->d_md_seg + h->md_seg_off[m], *seg_ref = seg_begin + S + 1;
+            uint32_t* ov = h->d_md_overlap + m * tab;
+            const dim3 ogrid(S, h->C / 32);
+            if (h->lab32_stale)
+                align_overlap_kernel<uint8_t><<<ogrid, 256, osmem, h->stream>>>(h->d_lab8, h->C, h->n_chains, ka, kb, order, seg_begin, seg_ref, ov);
+            else
+                align_overlap_kernel<int32_t><<<ogrid, 256, osmem, h->stream>>>(h->d_labels, h->C, h->n_chains, ka, kb, order, seg_begin, seg_ref, ov);
+            align_assign_kernel<<<dim3(h->n_chains, 2), 32, asmem, h->stream>>>(ov, h->C, ka, kb, h->d_md_map + (size_t)m * h->C * width);
+        }
+        modes_select_kernel<<<(h->n_chains + 7) / 8, 256, 0, h->stream>>>(h->d_md_overlap, h->d_md_map, h->C, h->n_chains, ka, kb, M,
+                                                                         h->md_min_ov, rung, h->d_md_nearest, h->d_md_chain, h->d_md_counted);
+        if (h->lab32_stale)
+            modes_marginal_kernel<uint8_t><<<mgrid, 256, 0, h->stream>>>(h->d_lab8, h->n, h->na, h->C, h->n_chains, ka, width, M,
+                                                                         h->d_md_chain, h->d_md_map, h->d_md_hist);
+        else
+            modes_marginal_kernel<int32_t><<<mgrid, 256, 0, h->stream>>>(h->d_labels, h->n, h->na, h->C, h->n_chains, ka, width, M,
+                                                                         h->d_md_chain, h->d_md_map, h->d_md_hist);
+        CU(cudaGetLastError());
+    }
     return BISBM_OK;
 }
 
 // kernel launches of one marginal sample (the alignment adds the overlap and assignment kernels, a query set the
-// co-assignment kernel)
-static uint64_t marginal_launches(const bisbm_handle* h) { return (h->al_segments ? 3 : 1) + (h->co_q ? 1 : 0); }
+// co-assignment kernel, a mode set an overlap and an assignment kernel per mode, the selection and its histogram kernel)
+static uint64_t marginal_launches(const bisbm_handle* h) {
+    return (h->al_segments ? 3 : 1) + (h->co_q ? 1 : 0) + (h->md_M ? 2 * (uint64_t)h->md_M + 2 : 0);
+}
 
 int bisbm_marginal_sample(bisbm_handle* h) {
     int rc = need_chains(h);
@@ -1876,6 +1926,10 @@ int bisbm_marginals_clear(bisbm_handle* h) {
         h->hist_width = width;
     }
     CU(cudaMemsetAsync(h->d_hist, 0, (size_t)h->n * width * sizeof(uint32_t), h->stream));
+    if (h->md_M) {     // a mode set keeps its references; its histograms and counters restart
+        CU(cudaMemsetAsync(h->d_md_hist, 0, (size_t)h->md_M * h->n * (h->md_ka + h->md_kb) * sizeof(uint32_t), h->stream));
+        CU(cudaMemsetAsync(h->d_md_counted, 0, (h->md_M + 1) * sizeof(unsigned long long), h->stream));
+    }
     CU(cudaStreamSynchronize(h->stream));
     return BISBM_OK;
 }
@@ -1943,6 +1997,130 @@ int bisbm_marginals_alignment(bisbm_handle* h, uint32_t* map) {
     if (!h->al_sampled) return fail(BISBM_ERR_STATE, "no aligned marginal sample since the reference was set");
     CU(cudaStreamSynchronize(h->stream));
     CU(cudaMemcpy(map, h->d_al_map, (size_t)h->n_chains * (h->al_ka + h->al_kb) * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    return BISBM_OK;
+}
+
+int bisbm_marginal_modes_set(bisbm_handle* h, uint32_t n_modes, const uint32_t* refs, double min_overlap) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (n_modes == 0 || !refs) { free_modes(h); return BISBM_OK; }
+    const uint32_t ka = h->h_ka[0], kb = h->h_kb[0], n = h->n, na = h->na, C = h->C, M = n_modes, width = ka + kb;
+    for (uint32_t c = 1; c < h->n_chains; ++c)
+        if (h->h_ka[c] != ka || h->h_kb[c] != kb)
+            return fail(BISBM_ERR_ARG, "modes need one (ka, kb) for the pool: chain %u has (%u, %u), chain 0 (%u, %u)", c,
+                        h->h_ka[c], h->h_kb[c], ka, kb);
+    if (!(min_overlap >= 0.0 && min_overlap <= 1.0)) return fail(BISBM_ERR_ARG, "min_overlap %g is not in [0, 1]", min_overlap);
+    for (uint32_t m = 0; m < M; ++m)
+        for (uint32_t v = 0; v < n; ++v) {
+            const uint32_t g = refs[(size_t)m * n + v];
+            if (v < na ? g >= ka : (g < ka || g >= ka + kb))
+                return fail(BISBM_ERR_ARG, "mode %u: reference label %u of node %u is not a type-%c block (ka=%u kb=%u)", m, g, v,
+                            v < na ? 'a' : 'b', ka, kb);
+        }
+    const size_t osmem = (size_t)std::max(ka, kb) * 32 * sizeof(uint32_t), asmem = align_assign_smem(std::max(ka, kb));
+    int optin = 0;
+    CU(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+    if (std::max(osmem, asmem) > (size_t)optin)
+        return fail(BISBM_ERR_ARG, "modes of %u blocks per type need %zu bytes of shared memory per block (device: %d)",
+                    std::max(ka, kb), std::max(osmem, asmem), optin);
+    // histograms and overlap tables may take at most a quarter of the free device memory (with the set in place released)
+    const size_t tab = (size_t)C * ((size_t)ka * ka + (size_t)kb * kb);
+    auto set_words = [&](size_t modes) { return modes * (size_t)n * width + modes * tab; };
+    size_t free_b = 0, total_b = 0;
+    CU(cudaMemGetInfo(&free_b, &total_b));
+    const size_t held = h->md_M ? set_words(h->md_M) * sizeof(uint32_t) : 0, bytes = set_words(M) * sizeof(uint32_t);
+    if (bytes > (free_b + held) / 4)
+        return fail(BISBM_ERR_ARG, "%u modes need %zu bytes of histograms and overlap tables: more than a quarter of the %zu bytes free",
+                    M, bytes, free_b + held);
+    if (osmem > 48 * 1024) {
+        rc = ensure_smem_attr(h, (const void*)align_overlap_kernel<uint8_t>, optin);
+        if (!rc) rc = ensure_smem_attr(h, (const void*)align_overlap_kernel<int32_t>, optin);
+        if (rc) return rc;
+    }
+    if (asmem > 48 * 1024 && (rc = ensure_smem_attr(h, (const void*)align_assign_kernel, optin))) return rc;
+    // per mode, what bisbm_marginals_align does once: node ids sorted by reference block, cut into segments of at most
+    // ALIGN_SEG nodes of one block (device layout per mode: begin[S + 1], then ref[S])
+    std::vector<uint32_t> order((size_t)M * n), segs(M), seg_off(M), seg_all;
+    for (uint32_t m = 0; m < M; ++m) {
+        const uint32_t* ref = refs + (size_t)m * n;
+        uint32_t* ord = order.data() + (size_t)m * n;
+        std::vector<uint32_t> start(width + 1, 0);
+        for (uint32_t v = 0; v < n; ++v) ++start[ref[v] + 1];
+        for (uint32_t g = 0; g < width; ++g) start[g + 1] += start[g];
+        std::vector<uint32_t> pos(start.begin(), start.end() - 1);
+        for (uint32_t v = 0; v < n; ++v) ord[pos[ref[v]]++] = v;
+        std::vector<uint32_t> seg_begin, seg_ref;
+        for (uint32_t g = 0; g < width; ++g)
+            for (uint32_t b = start[g]; b < start[g + 1]; b += ALIGN_SEG) { seg_begin.push_back(b); seg_ref.push_back(g); }
+        segs[m] = (uint32_t)seg_ref.size();
+        seg_off[m] = (uint32_t)seg_all.size();
+        seg_begin.push_back(n);
+        seg_all.insert(seg_all.end(), seg_begin.begin(), seg_begin.end());
+        seg_all.insert(seg_all.end(), seg_ref.begin(), seg_ref.end());
+    }
+    free_modes(h);
+    CU(cudaMalloc(&h->d_md_order, order.size() * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_seg, seg_all.size() * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_overlap, M * tab * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_map, (size_t)M * C * width * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_hist, (size_t)M * n * width * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_nearest, C * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_chain, C * sizeof(uint32_t)));
+    CU(cudaMalloc(&h->d_md_counted, (M + 1) * sizeof(unsigned long long)));
+    CU(cudaMemcpyAsync(h->d_md_order, order.data(), order.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemcpyAsync(h->d_md_seg, seg_all.data(), seg_all.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, h->stream));
+    CU(cudaMemsetAsync(h->d_md_hist, 0, (size_t)M * n * width * sizeof(uint32_t), h->stream));
+    CU(cudaMemsetAsync(h->d_md_counted, 0, (M + 1) * sizeof(unsigned long long), h->stream));
+    // before the first sample no chain has been counted: mode 0xffffffff, maps 0xffffffff
+    CU(cudaMemsetAsync(h->d_md_chain, 0xff, C * sizeof(uint32_t), h->stream));
+    CU(cudaMemsetAsync(h->d_md_nearest, 0xff, C * sizeof(uint32_t), h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    h->md_M = M; h->md_ka = ka; h->md_kb = kb;
+    h->md_min_ov = (uint64_t)std::ceil(min_overlap * (double)n);     // ov < min_overlap n  <=>  ov < ceil(min_overlap n)
+    h->md_segs = std::move(segs); h->md_seg_off = std::move(seg_off);
+    return BISBM_OK;
+}
+
+int bisbm_marginal_modes_get(bisbm_handle* h, uint32_t* hist, uint64_t* counted, uint32_t* chain_mode, uint32_t* map) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!h->md_M) return fail(BISBM_ERR_STATE, "no mode set: call bisbm_marginal_modes_set first");
+    const uint32_t M = h->md_M, N = h->n_chains, C = h->C, width = h->md_ka + h->md_kb;
+    CU(cudaStreamSynchronize(h->stream));
+    if (hist) CU(cudaMemcpy(hist, h->d_md_hist, (size_t)M * h->n * width * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    if (counted) {
+        std::vector<unsigned long long> x(M + 1);
+        CU(cudaMemcpy(x.data(), h->d_md_counted, (M + 1) * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+        for (uint32_t m = 0; m <= M; ++m) counted[m] = x[m];
+    }
+    if (chain_mode) CU(cudaMemcpy(chain_mode, h->d_md_chain, N * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    if (map) {
+        // each chain's row from the slice of the mode it was nearest to
+        std::vector<uint32_t> near(N), all((size_t)M * C * width);
+        CU(cudaMemcpy(near.data(), h->d_md_nearest, N * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        CU(cudaMemcpy(all.data(), h->d_md_map, all.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+        for (uint32_t c = 0; c < N; ++c) {
+            uint32_t* row = map + (size_t)c * width;
+            if (near[c] >= M) std::fill(row, row + width, 0xffffffffu);
+            else std::copy_n(all.data() + ((size_t)near[c] * C + c) * width, width, row);
+        }
+    }
+    return BISBM_OK;
+}
+
+int bisbm_marginal_modes_argmax(bisbm_handle* h, uint32_t* out) {
+    int rc = need_chains(h);
+    if (rc) return rc;
+    if (!h->md_M) return fail(BISBM_ERR_STATE, "no mode set: call bisbm_marginal_modes_set first");
+    if (!out) return fail(BISBM_ERR_ARG, "null argument");
+    const size_t rows = (size_t)h->md_M * h->n;
+    uint32_t* d_out = nullptr;
+    CU(cudaMalloc(&d_out, rows * sizeof(uint32_t)));
+    marginal_argmax_kernel<<<(unsigned)((rows + 255) / 256), 256, 0, h->stream>>>((uint32_t)rows, h->d_md_hist, h->md_ka + h->md_kb, d_out);
+    cudaError_t e = cudaStreamSynchronize(h->stream);
+    if (e == cudaSuccess) e = cudaMemcpy(out, d_out, rows * sizeof(uint32_t), cudaMemcpyDeviceToHost);
+    cudaFree(d_out);
+    if (e != cudaSuccess) return fail(BISBM_ERR_CUDA, "marginal_modes_argmax: %s", cudaGetErrorString(e));
     return BISBM_OK;
 }
 

@@ -20,6 +20,10 @@
 //   --agreement_out FILE   (one GPU: --chains N >= 2, --marginalize, --estimate) compares the final states of the chains
 //                          pairwise (bisbm_chain_agreement): FILE gets NMI / VI / ARI / matched overlap per pair, stderr
 //                          a one-line summary with the modes at overlap >= 0.95
+//   --modes_out FILE       (--marginalize, one GPU, --chains N >= 2) after the burn-in, the modes of the chains (of the
+//                          chains at T0 under --tempering) at overlap >= 0.95 become reference partitions, each the labels
+//                          of its lowest-entropy member, and every sample is counted in the histogram of the nearest one
+//                          (bisbm_marginal_modes_set); FILE gets the per-mode counts and arg-max labels
 //   --estimate             README "estimation" output format for fixed (Ka, Kb): CSV lines
 //                          sweep,Ka,Kb,loglik,labels... of the last 1000 samples
 //   -g / --merge, -u / --nature, or initial labels whose block counts differ from -z: the agglomerative
@@ -69,6 +73,7 @@ const Spec kSpecs[] = {
     {"maximize", 0, 0}, {"estimate", 0, 0}, {"marginalize", 0, 0}, {"chains", 0, 1}, {"gen_seed", 0, 1},
     {"device", 0, 1}, {"max_inflight", 0, 1}, {"gpus", 0, 1}, {"tempering", 0, 2}, {"swap_every", 0, 1},
     {"align", 0, 0}, {"coassign", 0, 1}, {"coassign_out", 0, 1}, {"agreement_out", 0, 1},
+    {"modes_out", 0, 1},
 };
 
 const Spec* find_spec(const std::string& tok) {
@@ -164,7 +169,13 @@ void usage(const char* argv0) {
                  "  --agreement_out arg                   one GPU, --chains >= 2 (plain, --marginalize, --estimate): compare\n"
                  "                                        the chains' final states pairwise; the file gets a line n_chains,\n"
                  "                                        then per pair c1 < c2: c1 c2 nmi vi ari overlap, then the same four\n"
-                 "                                        for type a and for type b (label-switching free)\n";
+                 "                                        for type a and for type b (label-switching free)\n"
+                 "  --modes_out arg                       --marginalize, one GPU, --chains >= 2: after the burn-in, the modes of\n"
+                 "                                        the chains (at T0 under --tempering) at overlap >= 0.95, each\n"
+                 "                                        represented by its lowest-entropy chain, and every sample counted in\n"
+                 "                                        the histogram of the nearest mode; the file gets a line \"M counted_0\n"
+                 "                                        .. counted_M\" (the last: samples of no mode), then M lines of per-mode\n"
+                 "                                        arg-max labels\n";
 }
 
 // the ladder of block counts between (start_a, start_b) and (end_a, end_b) (reference src/support/util.hh:99-146): the type
@@ -245,13 +256,40 @@ int add_coassign(bisbm_handle* h, size_t q, std::vector<uint64_t>& sum, uint64_t
     return BISBM_OK;
 }
 
+// index of (metric, slot, chain i, chain j) in bisbm_chain_agreement's output for every pair of nc chains
+size_t agree_at(int metric, int slot, size_t nc, size_t i, size_t j) { return (((size_t)metric * 3 + slot) * nc + i) * nc + j; }
+
+// the modes among the chains cand: the connected components of "whole-partition overlap >= 0.95", numbered in order of each
+// component's first chain in cand.  a: bisbm_chain_agreement over every pair of the pool's nc chains.  Returns the mode of
+// each entry of cand; sizes gets the members per mode.
+std::vector<size_t> overlap_modes(const std::vector<double>& a, size_t nc, const std::vector<size_t>& cand, std::vector<size_t>& sizes) {
+    const size_t k = cand.size();
+    std::vector<size_t> mode(k, k);
+    sizes.clear();
+    for (size_t c = 0; c < k; ++c) {
+        if (mode[c] < k) continue;
+        const size_t id = sizes.size();
+        sizes.push_back(0);
+        std::vector<size_t> stack{c};
+        mode[c] = id;
+        while (!stack.empty()) {
+            const size_t x = stack.back();
+            stack.pop_back();
+            ++sizes[id];
+            for (size_t y = 0; y < k; ++y)
+                if (mode[y] == k && a[agree_at(BISBM_AGREE_OVERLAP, 2, nc, cand[x], cand[y])] >= 0.95) { mode[y] = id; stack.push_back(y); }
+        }
+    }
+    return mode;
+}
+
 // --agreement_out: every pair of the pool's chains compared on their current labels (bisbm_chain_agreement).  The file gets
 // "n_chains", then per pair c1 < c2 the whole partition's nmi vi ari overlap, then type a's, then type b's; stderr one
 // summary line: the whole partition's NMI over the pairs and the modes, the connected components of overlap >= 0.95
 bool write_agreement(bisbm_handle* h, size_t nc, const std::string& path) {
     std::vector<double> a(4 * 3 * nc * nc);
     if (!check(bisbm_chain_agreement(h, nullptr, 1, a.data()))) return false;
-    auto at = [&](int metric, int slot, size_t i, size_t j) { return a[(((size_t)metric * 3 + slot) * nc + i) * nc + j]; };
+    auto at = [&](int metric, int slot, size_t i, size_t j) { return a[agree_at(metric, slot, nc, i, j)]; };
     std::ofstream f(path.c_str());
     if (!f.is_open()) { std::cerr << "cannot write the --agreement_out file " << path << "\n"; return false; }
     f.precision(17);
@@ -271,22 +309,9 @@ bool write_agreement(bisbm_handle* h, size_t nc, const std::string& path) {
     std::sort(nmi.begin(), nmi.end());
     const size_t np = nmi.size();
     const double median = np % 2 ? nmi[np / 2] : 0.5 * (nmi[np / 2 - 1] + nmi[np / 2]);
-    // modes: components of the overlap graph, numbered by their first chain
-    std::vector<size_t> mode(nc, nc), sizes;
-    for (size_t c = 0; c < nc; ++c) {
-        if (mode[c] < nc) continue;
-        const size_t k = sizes.size();
-        sizes.push_back(0);
-        std::vector<size_t> stack{c};
-        mode[c] = k;
-        while (!stack.empty()) {
-            const size_t x = stack.back();
-            stack.pop_back();
-            ++sizes[k];
-            for (size_t y = 0; y < nc; ++y)
-                if (mode[y] == nc && at(BISBM_AGREE_OVERLAP, 2, x, y) >= 0.95) { mode[y] = k; stack.push_back(y); }
-        }
-    }
+    std::vector<size_t> all(nc), sizes;
+    for (size_t c = 0; c < nc; ++c) all[c] = c;
+    overlap_modes(a, nc, all, sizes);
     std::clog << "chain agreement: NMI median " << median << " min " << nmi[0] << ", modes at overlap >= 0.95: " << sizes.size() << " (sizes";
     for (size_t z : sizes) std::clog << " " << z;
     std::clog << ")\n";
@@ -304,6 +329,50 @@ int lowest_entropy_chain(bisbm_handle* h, size_t n_chains, bool cold_only, doubl
     for (size_t c = 0; c < n_chains; ++c)
         if (rung[c] == 0 && (!found || ent[c] < *S)) { *S = ent[c]; *best = (uint32_t)c; found = true; }
     return BISBM_OK;
+}
+
+// --modes_out: the modes of the chains' current labels (under a ladder, of the chains at rung 0) as --agreement_out finds
+// them, each represented by its member of lowest entropy(), become the references of every later sample (min_overlap 0)
+int set_modes(bisbm_handle* h, size_t nc, size_t n, bool cold_only, uint32_t* n_modes) {
+    std::vector<double> a(4 * 3 * nc * nc), ent(nc);
+    std::vector<uint32_t> rung(nc, 0);
+    int rc = bisbm_chain_agreement(h, nullptr, 1, a.data());
+    if (rc == BISBM_OK) rc = bisbm_entropy_all(h, ent.data());
+    if (rc == BISBM_OK && cold_only) rc = bisbm_tempering_stats(h, rung.data(), nullptr, nullptr, nullptr, nullptr, nullptr);
+    if (rc != BISBM_OK) return rc;
+    std::vector<size_t> cand, sizes;
+    for (size_t c = 0; c < nc; ++c) if (rung[c] == 0) cand.push_back(c);
+    const std::vector<size_t> mode = overlap_modes(a, nc, cand, sizes);
+    std::vector<size_t> best(sizes.size(), nc);
+    for (size_t i = 0; i < cand.size(); ++i)
+        if (best[mode[i]] == nc || ent[cand[i]] < ent[best[mode[i]]]) best[mode[i]] = cand[i];
+    std::vector<uint32_t> refs(sizes.size() * n);
+    for (size_t m = 0; m < sizes.size(); ++m)
+        if ((rc = bisbm_get_labels(h, (uint32_t)best[m], refs.data() + m * n)) != BISBM_OK) return rc;
+    *n_modes = (uint32_t)sizes.size();
+    return bisbm_marginal_modes_set(h, *n_modes, refs.data(), 0.0);
+}
+
+// --modes_out: "M counted_0 .. counted_M", then the M arg-max label lines; stderr one line with the mode weights
+bool write_modes(bisbm_handle* h, uint32_t M, size_t n, const std::string& path) {
+    std::vector<uint64_t> counted(M + 1);
+    std::vector<uint32_t> am((size_t)M * n);
+    if (!check(bisbm_marginal_modes_get(h, nullptr, counted.data(), nullptr, nullptr)) || !check(bisbm_marginal_modes_argmax(h, am.data())))
+        return false;
+    std::ofstream f(path.c_str());
+    if (!f.is_open()) { std::cerr << "cannot write the --modes_out file " << path << "\n"; return false; }
+    f << M;
+    for (uint64_t x : counted) f << " " << x;
+    f << "\n";
+    for (uint32_t m = 0; m < M; ++m) output_vec(std::vector<uint32_t>(am.begin() + (size_t)m * n, am.begin() + (size_t)(m + 1) * n), f);
+    f.close();
+    if (f.fail()) { std::cerr << "cannot write the --modes_out file " << path << "\n"; return false; }
+    uint64_t total = 0;
+    for (uint32_t m = 0; m < M; ++m) total += counted[m];
+    std::clog << "marginal modes: " << M << ", weights";
+    for (uint32_t m = 0; m < M; ++m) std::clog << " " << (total ? (double)counted[m] / (double)total : 0.0);
+    std::clog << " (samples " << total << ", unassigned " << counted[M] << ")\n";
+    return true;
 }
 
 }  // namespace
@@ -407,6 +476,13 @@ int main(int argc, char const* argv[]) {
         if (gpus > 1) { std::cerr << "--agreement_out compares the chains of one GPU (no --gpus > 1)\n"; return 1; }
         if (chains < 2) { std::cerr << "--agreement_out needs --chains >= 2\n"; return 1; }
     }
+    const bool modes = o.has("modes_out");
+    if (modes) {
+        if (!o.has("marginalize")) { std::cerr << "--modes_out needs --marginalize\n"; return 1; }
+        if (gpus > 1) { std::cerr << "--modes_out finds the modes of one GPU's chains (no --gpus > 1)\n"; return 1; }
+        if (chains < 2) { std::cerr << "--modes_out needs --chains >= 2\n"; return 1; }
+    }
+    uint32_t n_modes = 0;
     if (gpus > chains) gpus = chains;
     // stdout carries the label line and nothing else: whatever NCCL has to say (its version banner under NCCL_DEBUG)
     // goes to stderr unless the user chose a file
@@ -679,9 +755,11 @@ int main(int argc, char const* argv[]) {
                 if (!check(lowest_entropy_chain(h, chains, true, &S, &best)) || !check(bisbm_get_labels(h, best, out.data())) ||
                     !check(bisbm_marginals_align(h, out.data()))) return 1;
             }
+            if (modes && !check(set_modes(h, chains, N, true, &n_modes))) return 1;
             if (!check(bisbm_tempering_run(h, sampling_steps, swap_every, f, seeds.data(), (uint64_t)seed, (uint32_t)max_inflight, nullptr))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
             if (agreement && !write_agreement(h, chains, o.vals["agreement_out"][0])) return 1;
+            if (modes && !write_modes(h, n_modes, N, o.vals["modes_out"][0])) return 1;
             if (coassign && (!check(add_coassign(h, query.size(), co_sum, co_counted)) ||
                              !write_coassign(o.vals["coassign_out"][0], query.size(), co_sum, co_counted))) return 1;
             output_vec(out, std::cout);
@@ -689,17 +767,22 @@ int main(int argc, char const* argv[]) {
             const size_t f = std::max<size_t>(sampling_frequency, 1);
             if (!check(bisbm_marginals_clear(h))) return 1;
             if (coassign && !check(bisbm_coassign_set(h, (uint32_t)query.size(), query.data()))) return 1;
-            if (align) {
-                // burn-in, then the lowest-entropy chain is the reference every sample is aligned to
-                double S = 0.0;
-                uint32_t best = 0;
-                if (!check(bisbm_marginalize(h, burn_in, 0, f, seeds.data(), (uint32_t)max_inflight)) ||
-                    !check(lowest_entropy_chain(h, chains, false, &S, &best)) || !check(bisbm_get_labels(h, best, out.data())) ||
-                    !check(bisbm_marginals_align(h, out.data())) ||
-                    !check(bisbm_marginalize(h, 0, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
+            if (align || modes) {
+                // burn-in, then the references chosen from the chains: the lowest-entropy chain every sample is aligned to
+                // (--align), the modes every sample is sorted into (--modes_out); then the sampling sweeps
+                if (!check(bisbm_marginalize(h, burn_in, 0, f, seeds.data(), (uint32_t)max_inflight))) return 1;
+                if (align) {
+                    double S = 0.0;
+                    uint32_t best = 0;
+                    if (!check(lowest_entropy_chain(h, chains, false, &S, &best)) || !check(bisbm_get_labels(h, best, out.data())) ||
+                        !check(bisbm_marginals_align(h, out.data()))) return 1;
+                }
+                if (modes && !check(set_modes(h, chains, N, false, &n_modes))) return 1;
+                if (!check(bisbm_marginalize(h, 0, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
             } else if (!check(bisbm_marginalize(h, burn_in, sampling_steps, f, seeds.data(), (uint32_t)max_inflight))) return 1;
             if (!check(bisbm_marginal_argmax(h, out.data()))) return 1;
             if (agreement && !write_agreement(h, chains, o.vals["agreement_out"][0])) return 1;
+            if (modes && !write_modes(h, n_modes, N, o.vals["modes_out"][0])) return 1;
             if (coassign && (!check(add_coassign(h, query.size(), co_sum, co_counted)) ||
                              !write_coassign(o.vals["coassign_out"][0], query.size(), co_sum, co_counted))) return 1;
             output_vec(out, std::cout);

@@ -79,6 +79,9 @@ SIGNATURES = {
     "bisbm_marginal_sample": (C.c_int, [C.c_void_p]),
     "bisbm_marginals_align": (C.c_int, [C.c_void_p, _u32p]),
     "bisbm_marginals_alignment": (C.c_int, [C.c_void_p, _u32p]),
+    "bisbm_marginal_modes_set": (C.c_int, [C.c_void_p, C.c_uint32, _u32p, C.c_double]),
+    "bisbm_marginal_modes_get": (C.c_int, [C.c_void_p, _u32p, _u64p, _u32p, _u32p]),
+    "bisbm_marginal_modes_argmax": (C.c_int, [C.c_void_p, _u32p]),
     "bisbm_coassign_set": (C.c_int, [C.c_void_p, C.c_uint32, _u32p]),
     "bisbm_coassign_get": (C.c_int, [C.c_void_p, _u32p, _u64p]),
     "bisbm_chain_agreement": (C.c_int, [C.c_void_p, _u32p, C.c_int, _dp]),
@@ -324,6 +327,26 @@ def chain_modes(overlap_whole, threshold=0.95):
     return mode
 
 
+def mode_references(pool, threshold=0.95, chains=None):
+    """(refs [M][n] uint32, mode_of_chain [n_chains]) for ChainPool.marginal_modes_set: the modes are chain_modes of the
+    whole-partition overlap of the chains' current labels at `threshold`, and each mode's reference is the labels of its
+    member of lowest entropy (the lowest chain id among equals).  chains (optional): the candidate chains, e.g. the rung-0
+    chains of a ladder; the others get mode -1."""
+    cand = np.arange(pool.n_chains) if chains is None else np.asarray(chains, dtype=np.int64).ravel()
+    if cand.size == 0 or np.unique(cand).size != cand.size or cand.min() < 0 or cand.max() >= pool.n_chains:
+        raise ValueError("chains must be distinct chain ids of the pool")
+    overlap = pool.chain_agreement()["overlap"][2]
+    modes = chain_modes(overlap[np.ix_(cand, cand)], threshold)
+    ent = np.asarray(pool.entropy(), dtype=np.float64)[cand]
+    refs = []
+    for k in range(int(modes.max()) + 1):
+        members = np.flatnonzero(modes == k)
+        refs.append(pool.labels(int(cand[members[np.argmin(ent[members])]])))
+    mode_of_chain = np.full(pool.n_chains, -1, dtype=np.int64)
+    mode_of_chain[cand] = modes
+    return np.stack(refs).astype(np.uint32), mode_of_chain
+
+
 def edge_to_adj(edge_list, N, na=None, nb=None, device=0):
     """reference src/graph_utilities.cc:36-49.  The bipartition (na, nb) must be given since
     the device graph validates it; N = na + nb."""
@@ -480,6 +503,41 @@ class ChainPool:
         width = w.value if self.L.bisbm_marginals_device(self.g.h, C.byref(ptr), C.byref(ne), C.byref(w)) == 0 else 0
         out = np.zeros((self.n_chains, width), dtype=np.uint32)
         _check(self.L.bisbm_marginals_alignment(self.g.h, _p(out, C.c_uint32)))
+        return out
+
+    def marginal_modes_set(self, refs, min_overlap=0.0):
+        """Resolve every later marginal sample by mode: each chain is counted in the histogram of the reference partition
+        (refs [M][n], global block ids, e.g. from mode_references) it agrees with on the most nodes after alignment, or in
+        none if that is fewer than min_overlap * n nodes.  Histograms and counters start at zero; None clears.  Needs one
+        (ka, kb) for the whole pool."""
+        if refs is None:
+            _check(self.L.bisbm_marginal_modes_set(self.g.h, 0, None, 0.0))
+            self._modes = 0
+            return
+        r = np.asarray(refs)
+        if r.ndim == 1:
+            r = r[None, :]
+        if r.ndim != 2 or r.shape[1] != self.g.n or r.shape[0] == 0 or r.min() < 0 or r.max() > 0xffffffff:
+            raise ValueError("refs is [M][n]: one block id per node for each mode")
+        r = np.ascontiguousarray(r, dtype=np.uint32)
+        _check(self.L.bisbm_marginal_modes_set(self.g.h, r.shape[0], _p(r, C.c_uint32), float(min_overlap)))
+        self._modes = r.shape[0]
+
+    def marginal_modes(self):
+        """dict: "hist" [M][n][ka + kb] uint32, "counted" [M + 1] uint64 (the last entry: samples left unassigned), and of the
+        last sample "chain_mode" [n_chains] (M: unassigned, 0xffffffff: not counted) and "map" [n_chains][ka + kb] (the
+        permutation to each chain's nearest mode)."""
+        M, W = getattr(self, "_modes", 0), int(self.ka[0] + self.kb[0])
+        out = {"hist": np.zeros((M, self.g.n, W), dtype=np.uint32), "counted": np.zeros(M + 1, dtype=np.uint64),
+               "chain_mode": np.zeros(self.n_chains, dtype=np.uint32), "map": np.zeros((self.n_chains, W), dtype=np.uint32)}
+        _check(self.L.bisbm_marginal_modes_get(self.g.h, _p(out["hist"], C.c_uint32), _p(out["counted"], C.c_uint64),
+                                               _p(out["chain_mode"], C.c_uint32), _p(out["map"], C.c_uint32)))
+        return out
+
+    def marginal_modes_argmax(self):
+        """[M][n]: the arg-max label of every node in each mode's histogram."""
+        out = np.zeros((getattr(self, "_modes", 0), self.g.n), dtype=np.uint32)
+        _check(self.L.bisbm_marginal_modes_argmax(self.g.h, _p(out, C.c_uint32)))
         return out
 
     def coassign_set(self, nodes):

@@ -163,6 +163,37 @@ int bisbm_marginals_align(bisbm_handle* h, const uint32_t* ref_labels);
  * ([n_chains][ka + kb], computed for every chain, also those a tempering sample skips).  BISBM_ERR_STATE before any aligned
  * sample under the current reference. */
 int bisbm_marginals_alignment(bisbm_handle* h, uint32_t* map);
+/* Marginals resolved by mode (no counterpart in the reference).  A pool whose chains sit in several modes gives, under one
+ * alignment reference, a histogram that mixes them.  refs[n_modes][n]: reference partitions in the pool's global numbering
+ * (as bisbm_marginals_align takes one), e.g. one per mode that bisbm_chain_agreement finds.  While a set is in place,
+ * every marginal sample (bisbm_marginal_sample, bisbm_marginalize, bisbm_tempering_run's rung-0 samples) also does, for
+ * every counted chain c (a real chain; under a ladder, a chain at rung 0 at sample time):
+ *   1. for every mode m, pi_{c,m}: the permutation bisbm_marginals_align(refs[m]) would use (same objective, same
+ *      deterministic tie-break), and ov_{c,m}: the nodes that agree after pi_{c,m}, over both types;
+ *   2. m* = arg-max_m ov_{c,m}, the lowest m among equals (exact integers);
+ *   3. if ov_{c,m*} < min_overlap n the sample is counted in no histogram: counted[n_modes] += 1;
+ *   4. else hist[m*][v][pi_{c,m*}(label of v)] += 1 for every node v, and counted[m*] += 1.
+ * So for every node sum_{m < n_modes} hist[m][v][:] = sum_{m < n_modes} counted[m], and the mode weights are counted[m] /
+ * sum counted.  The set is independent of the ordinary histogram, of an alignment reference and of a co-assignment query
+ * set: with or without it those, the labels and every later trajectory are bit-identical.  A sample queues 2 n_modes + 2
+ * kernels on the handle's stream with no host synchronisation (the launch counters include them).  bisbm_marginals_clear
+ * zeroes the histograms and counters and keeps the references; bisbm_randomize keeps everything; bisbm_set_chains* and a
+ * replay merge / split that changes a chain's (ka, kb) clear the set.  Multi-GPU: set the same references on every handle
+ * and sum what each returns.  n_modes = 0 or refs = NULL clears and frees; the histograms and counters start at zero.
+ * Errors: BISBM_ERR_ARG for a null handle, a pool whose chains differ in (ka, kb), a reference label outside its node's type
+ * range, min_overlap NaN or outside [0, 1], more blocks per type than shared memory per block holds (as for alignment),
+ * or histograms plus overlap tables (n_modes n (ka + kb) + n_modes C (ka^2 + kb^2) uint32, C = chains rounded up to 32)
+ * larger than a quarter of the free device memory, the set in place then being kept; BISBM_ERR_STATE without a pool. */
+int bisbm_marginal_modes_set(bisbm_handle* h, uint32_t n_modes, const uint32_t* refs, double min_overlap);
+/* any pointer may be NULL.  hist[n_modes][n][ka + kb]; counted[n_modes + 1] (the last entry: samples left unassigned);
+ * chain_mode[n_chains] and map[n_chains][ka + kb]: in the LAST sample, the mode each chain was counted in (n_modes if it
+ * was left unassigned, 0xffffffff if it was not counted, e.g. not at rung 0, or before any sample) and the permutation to
+ * its nearest mode (map[c * (ka + kb) + g] = the global id block g was counted as; 0xffffffff before any sample).
+ * Waits for the handle's stream.  BISBM_ERR_STATE without a set. */
+int bisbm_marginal_modes_get(bisbm_handle* h, uint32_t* hist, uint64_t* counted, uint32_t* chain_mode, uint32_t* map);
+/* per-mode arg-max labels of the histograms, out[n_modes][n] (global ids; the lowest id among equal counts).
+ * BISBM_ERR_STATE without a set. */
+int bisbm_marginal_modes_argmax(bisbm_handle* h, uint32_t* out);
 /* Posterior co-assignment of query node pairs (label-switching free; no counterpart in the reference).  The fraction of
  * counted (chain, sample) pairs in which nodes i and j share a block estimates P(b_i = b_j | data); a permutation of a
  * chain's block ids does not change it, so it is defined across modes, across pools of mixed (ka, kb), in estimate mode
